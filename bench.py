@@ -5,7 +5,7 @@ Metric (BASELINE.json): bootstrapped gates/sec, STD128_OPT GINX, on the syntheti
 NAND / AND / XOR gates (config 3: 1 048 576 gates, gate i has type i mod 3; the reference's composite XOR = 3 bootstraps,
 src/gate.cpp:198-202), plus whole-circuit wall times (configs 4-5) with the CPU port's wall time beside them.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--gates G] [--impl reference] [--no-aux]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--gates G] [--impl reference] [--no-aux] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1; torch.distributed is plumbing only: barrier + max-reduce of times).
 A step = one pass of the hot path (bfhe_eval_bingate_batch: blind rotation + key switch) over one batch of G gates
@@ -56,6 +56,8 @@ def parse():
     ap.add_argument("--no-aux", action="store_true", help="skip the circuit wall-time / AP figures")
     ap.add_argument("--cpu-sample", type=int, default=0,
                     help="gates in the CPU baseline sample (0 = 4096 on >= 16 cores, scaled down on fewer; reference arm: 8 per core per step)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's output ciphertexts of the last timed step (a fixed sample of rows) to DIR as .npy files")
     return ap.parse_args()
 
 
@@ -250,6 +252,8 @@ def main():
     # correctness of what was just timed: every output decrypts to the truth table
     out = slab[n_in:].cpu().numpy().view(np.uint32)
     ok = bool(np.array_equal(ctx.decrypt(out), expected_bits(B, gates, bits)))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, ctx.p.ct_words)
 
     # ---------------- end to end through the host-buffer API (e2e) ----------------
     hin, hout = host_in.numpy().view(np.uint32), host_out.numpy().view(np.uint32)
@@ -333,6 +337,20 @@ def main():
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_ROWS = 8192
+
+
+def dump_outputs(d, out, words):
+    """The output ciphertexts of the timed step, for comparing two builds output for output.  The whole set is ~400 MB at the default
+    size, so a fixed seeded sample of at most DUMP_ROWS gates is written (8192 x 503 words x 8 B = 33 MB); float64 holds every 32-bit
+    word exactly.  ciphertext_rows.npy holds the gate index of each sampled row."""
+    n = out.shape[0]
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, size=DUMP_ROWS, replace=False))
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "ciphertext_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(d, "ciphertexts.npy"), out[rows, :words].astype(np.float64))
 
 
 def peak_hbm():

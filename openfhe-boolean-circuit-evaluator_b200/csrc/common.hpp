@@ -17,7 +17,7 @@ using i64 = int64_t;
 struct DevConst {
   u32 Q, Q2;       // ring modulus (2^26 < Q < 2^27) and 2Q
   u32 qinv_neg;    // -Q^-1 mod 2^32 (Montgomery)
-  u32 mu;          // floor(2^32 / Q) (lazy Barrett)
+  u32 unused_mu;   // unused, like reserved_ below
   u32 oneM;        // 2^32 mod Q  (Montgomery form of 1)
   u32 Q8;          // Q/8 + 1
   u32 n, N, q, factor; // LWE dim, ring dim, LWE modulus, 2N/q
@@ -27,8 +27,7 @@ struct DevConst {
   u32 ninv, ninvs; // N^-1 mod Q and its Shoup companion (debug kernels only)
   u32 nM, nMs;     // N^-1 * 2^32 mod Q (+Shoup): coefficient-form key -> device form
   u32 gate_const[9];
-  u32 sol_zero;           // 0, opaque to the compiler (3-input adds stay on the ALU pipe)
-  u32 sol_sh16, sol_sh11; // 16 and 11 for Q = 2^27 - 2^11 + 1: shift amounts of the ALU-pipe form of t*Q (kernels.cu mul_shoup<true>)
+  u32 reserved_[3]; // unused: with unused_mu they keep tw[] / itw[] at their constant-bank offsets, which decide ptxas's vector constant loads
   // psi^bitrev(k), k in [1,32): the twiddles of every NTT stage whose butterflies span >= 32 indices.
   u32 tw[32], tws[32], itw[32], itws[32];
 };
@@ -110,6 +109,5 @@ int launch_dbg_ntt(const DevConst &P, const u32 *d_a, const u32 *d_b, u32 *d_rt,
                    void *stream);
 int launch_microbench(int which, u32 *d_sink, int iters, int *threads_total, int *ops_per_thread_iter, void *stream);
 int blind_rotate_set_attrs();
-bool kernels_built_for_solinas_q();
 
 } // namespace bfhe

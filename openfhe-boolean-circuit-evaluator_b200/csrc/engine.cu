@@ -5,6 +5,7 @@
 // (all one-off or per-I/O-bit work).  Device side: everything per gate.  There is no CPU fallback for
 // EvalBinGate / Bootstrap / EvalNOT: without a CUDA device those calls fail with BFHE_ERR_CUDA.
 #include "engine.hpp"
+#include "device.cuh"
 #include <algorithm>
 #include <cstdio>
 #include <cstring>
@@ -81,8 +82,8 @@ extern "C" bfhe_ctx *bfhe_create(int paramset, int method, int device) {
     set_error("2N/q must be even (the monomial-factor table of the external product holds even exponents only)");
     return nullptr;
   }
-  if (kernels_built_for_solinas_q() && p.Q != (1ull << 27) - (1ull << 11) + 1) {
-    set_error("kernels are specialised for Q = 2^27 - 2^11 + 1; rebuild with -DBFHE_GENERIC_Q for another modulus");
+  if (p.Q != SOLINAS_Q) {
+    set_error("kernels are specialised for Q = 2^27 - 2^11 + 1");
     return nullptr;
   }
   bfhe_ctx *c = new bfhe_ctx();
@@ -99,10 +100,8 @@ extern "C" bfhe_ctx *bfhe_create(int paramset, int method, int device) {
     for (int i = 0; i < 5; i++) inv *= 2 - (u32)Q * inv;
     P.qinv_neg = 0u - inv;
   }
-  P.mu = (u32)((1ull << 32) / Q);
   P.oneM = (u32)((1ull << 32) % Q);
   P.Q8 = (u32)(Q / 8 + 1);
-  P.sol_sh16 = 16; P.sol_sh11 = 11; P.sol_zero = 0;
   P.n = p.n; P.N = N; P.q = p.q; P.factor = 2 * N / p.q;
   P.qKS = (u32)p.qKS; P.baseKS = p.baseKS; P.dKS = p.dKS;
   P.baseR = p.baseR; P.dR = p.dR; P.dG = p.dG; P.logBG = ilog2_ceil(p.baseG);
@@ -173,8 +172,8 @@ extern "C" bfhe_ctx *bfhe_create(int paramset, int method, int device) {
         t2[2 * N + d] = c->hntt.itw[k]; t2[3 * N + d] = shoup32(c->hntt.itw[k], Q);
       }
       const u64 oneM = (1ull << 32) % Q;
-      for (u32 k = 0; k < 2 * N; k++) // (psi^k - 1) in Montgomery form, stored at the 11-bit rotation of k (kernels_v2.cu f_index)
-        F[((k >> 5) & 63u) | ((k & 31u) << 6)] = (u32)((psiM[k] + Q - oneM) % Q);
+      for (u32 k = 0; k < 2 * N; k++) // (psi^k - 1) in Montgomery form
+        F[f_index(k)] = (u32)((psiM[k] + Q - oneM) % Q);
       ok = cudaMalloc(&c->d_tw2, t2.size() * 4) == cudaSuccess && cudaMalloc(&c->d_F, F.size() * 4) == cudaSuccess &&
            cudaMemcpy(c->d_tw2, t2.data(), t2.size() * 4, cudaMemcpyHostToDevice) == cudaSuccess &&
            cudaMemcpy(c->d_F, F.data(), F.size() * 4, cudaMemcpyHostToDevice) == cudaSuccess;

@@ -19,110 +19,18 @@
 //    -> dG forward NTTs, all in registers of the same warp.
 //  * A CTA carries G gates through the n blind-rotation steps in lock step so that every
 //    bootstrapping-key word loaded from L2 is reused G times from registers (GINX).
-#include "common.hpp"
-#include <algorithm>
+#include "device.cuh"
 #include <type_traits>
 #include <cuda_runtime.h>
 #include <cstdlib>
 
 namespace bfhe {
 
-// cudaFuncSetAttribute is per DEVICE: one process may hold contexts on several GPUs, so the "already done" flags of the launch
-// helpers below are kept per device ordinal
-static inline int attr_device_slot() {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  return dev >= 0 && dev < 64 ? dev : 0;
-}
-
-// ------------------------------------------------------------------------------------------
-// modular arithmetic
-// ------------------------------------------------------------------------------------------
-// Both parameter sets of the reference share Q = PreviousPrime(FirstPrime(27, 2N), 2N) = 2^27 - 2^11 + 1.  For that
-// modulus t*Q mod 2^32 = t - ((t - (t << 16)) << 11): three ALU-pipe instructions instead of one IMAD on the FMA-heavy
-// pipe, which is the unit that bounds the kernel (profiles/r1_blind_rotate_ncu_summary.md).  bfhe_create refuses any other
-// modulus when this is compiled in; build with -DBFHE_GENERIC_Q for the plain form.
-#ifndef BFHE_GENERIC_Q
-#define BFHE_SOLINAS_Q 1
-__device__ __forceinline__ u32 mul_q(u32 t, u32) { return t - ((t - (t << 16)) << 11); }
-#else
-#define BFHE_SOLINAS_Q 0
-__device__ __forceinline__ u32 mul_q(u32 t, u32 Q) { return t * Q; }
-#endif
-bool kernels_built_for_solinas_q() { return BFHE_SOLINAS_Q != 0; }
-// SOL selects where the t*Q term runs: true = three ALU-pipe instructions (shift/add), false = one IMAD on the
-// FMA-heavy pipe.  Both pipes issue 16 lanes/cycle per SM sub-partition, so the kernels mix the two forms per butterfly
-// stage to balance them (masks below).
-// BFHE_SOL_RT: the two shift amounts come from the kernel parameters (DevConst::sol_sh16 / sol_sh11) instead of being literals.  With
-// literal shifts ptxas rewrites the sequence into IMAD / IMAD.SHL with small constants -- back onto the FMA-heavy pipe, which made
-// every round-1 mask measure the same as no mask.  A shift by a run-time amount can only be an SHF on the ALU pipe, and the final
-// 3-input add is an IADD3.
-// Measured in round 2 (profiles/r2_sol_variants.md): with run-time shifts the stages really run on the ALU pipe -- and the throughput
-// kernel gets SLOWER with every stage converted (80.6k -> 74.2k with half of the stages, 66.4k with all): the kernel is bound by
-// instruction issue / dependency latency at two warps per scheduler, not by the FMA-heavy pipe, so one IMAD beats three ALU instructions.
-#ifndef BFHE_SOL_RT
-#define BFHE_SOL_RT 0
-#endif
-// BFHE_ADD3: 2-input adds of the butterflies are written as 3-input adds with a zero that comes from the kernel parameters: ptxas turns
-// plain 2-input adds into IMAD.IADD "to balance the pipes" -- onto the FMA-heavy pipe -- while a 3-input add can only be an IADD3 (ALU).
-// (same measurement: forcing the adds onto the ALU pipe costs 2.6 %, 80.6k -> 78.5k gates/s; off)
-#ifndef BFHE_ADD3
-#define BFHE_ADD3 0
-#endif
-struct SolSh { u32 a, b, z; }; // 16, 11, 0 at run time
-__device__ __forceinline__ SolSh sol_shifts(const DevConst &P) {
-#if BFHE_SOL_RT
-  return SolSh{P.sol_sh16, P.sol_sh11, P.sol_zero};
-#else
-  return SolSh{16, 11, 0};
-#endif
-}
-__device__ __forceinline__ u32 add2(u32 a, u32 b, SolSh sh) {
-#if BFHE_ADD3
-  return a + b + sh.z;
-#else
-  return a + b;
-#endif
-}
-__device__ __forceinline__ u32 sol_tail(u32 xw, u32 t, SolSh sh) { // xw - t*Q for Q = 2^27 - 2^11 + 1
-  const u32 s = add2(t, 0u - (t << sh.a), sh);
-  return (xw - t) + (s << sh.b);
-}
-template <bool SOL = false> __device__ __forceinline__ u32 mul_shoup(u32 x, u32 w, u32 ws, u32 Q, SolSh sh = SolSh{16, 11, 0}) { // [0,2Q)
-  const u32 t = __umulhi(x, ws);
-  if constexpr (SOL && BFHE_SOLINAS_Q) {
-    return sol_tail(x * w, t, sh);
-  } else {
-    return x * w - t * Q;
-  }
-}
-// per-pass stage masks (bit i = stage i of the pass uses the ALU form); tuned with tools/perf_g.py / phase_timing.py
-#ifndef BFHE_AP_HOIST
-#define BFHE_AP_HOIST 0
-#endif
-#ifndef BFHE_KEY_HOIST
-#define BFHE_KEY_HOIST 2 // halves of the key tile requested before the last digit transform (measured: 0: 84.95 k, 1: 86.7 k, 2: 88.2 k gates/s)
-#endif
-#ifndef BFHE_SOL_THR_WIDE
-#define BFHE_SOL_THR_WIDE 0x00 // re-measured after the first-stage product table: 0x00/0x00 80.2k, 0x07/0x03 80.3k, 0x17/0x0b 79.7k,
-#define BFHE_SOL_THR_NARROW 0x00 // 0x1f/0x1f 77.1k gates/s -- within noise of each other except all-on; kept off
-#define BFHE_SOL_LAT_WIDE 0x05
-#define BFHE_SOL_LAT_NARROW 0x0a
-#define BFHE_SOL_LAT_INV 0x00
-#endif
-__device__ __forceinline__ u32 redc(u64 s, u32 Q, u32 qinv_neg) { // s * 2^-32 mod Q, lazy
-  u32 m = (u32)s * qinv_neg;
-  return (u32)((s + (u64)m * Q) >> 32);
-}
-__device__ __forceinline__ u32 lazy_reduce(u32 x, u32 Q, u32 mu) { // any x -> [0,2Q)
-#if BFHE_SOLINAS_Q
-  const u32 t = x >> 27; // floor(2^32 / Q) = 32, so the Barrett quotient estimate is a shift
-  return x - t * Q;
-#else
-  return x - __umulhi(x, mu) * Q;
-#endif
-}
-__device__ __forceinline__ u32 csub(u32 x, u32 Q) { return min(x, x - Q); }                            // [0,2Q) -> [0,Q)
+// Masks of the latency kernel's forward transform: bit i = stage i of the pass (wide: span >= 32, narrow: span < 32) computes the t*Q term
+// of its Shoup multiplies on the ALU pipe (mul_shoup<true>), the other stages on the FMA-heavy pipe; tuned with tools/perf_lat.py /
+// phase_timing.py.  Every other transform uses the IMAD form: the throughput kernel is bound by instruction issue under dependency latency
+// at two warps per scheduler, where one IMAD beats three ALU instructions (DESIGN.md 5.4, profiles/r2_sol_variants.md).
+constexpr int SOL_LAT_WIDE = 0x05, SOL_LAT_NARROW = 0x0a;
 
 // ------------------------------------------------------------------------------------------
 // shared-memory polynomial layout: row t' (the E consecutive indices owned by lane t' in the narrow
@@ -162,38 +70,21 @@ template <int E> __device__ __forceinline__ void col_store(u32 *buf, const u32 (
   for (int k = 0; k < E; k++) buf[Lay<E>::elem_off(k, lane)] = x[k];
 }
 
-// per-lane twiddles of the narrow pass: smem table [C][32] of uint4, entry p of lane t' = psi^br(m+i)
-template <int E> __device__ __forceinline__ void load_lane_tw(const u32 *tab, u32 (&w)[E], int lane) {
-#pragma unroll
-  for (int c = 0; c < E / 4; c++) {
-    uint4 v = reinterpret_cast<const uint4 *>(tab)[c * 32 + lane];
-    w[4 * c] = v.x; w[4 * c + 1] = v.y; w[4 * c + 2] = v.z; w[4 * c + 3] = v.w;
-  }
-}
-
 // ------------------------------------------------------------------------------------------
 // in-register passes.  The E-point sub-transform has the same shape in both passes: stage with
 // half-size t has E/(2t) groups, group gi uses twiddle number p = E/(2t) + gi of the pass's table.
 // ------------------------------------------------------------------------------------------
 // Cooley-Tukey (forward).  No range correction: x + T and x - T + 2Q grow by 2Q per stage.
-// STREAM: the per-lane twiddles are read from the shared-memory table chunk by chunk as the stages need them (at
-// most 8 registers live) instead of being preloaded into 2*E registers -- what lets 12 warps per SM fit the register file.
-#ifndef BFHE_STREAM_TW
-#define BFHE_STREAM_TW 1
-#endif
-#ifndef BFHE_PAIRED_DIGITS
-#define BFHE_PAIRED_DIGITS 1
-#endif
-#ifndef BFHE_PAIRED_MAXG
-#define BFHE_PAIRED_MAXG 2
-#endif
+// UNI: twiddles uniform over the warp (kernel parameters).  Otherwise the per-lane twiddles (smem table [C][32] of uint4, entry p of
+// lane t' = psi^br(m+i)) are read chunk by chunk as the stages need them (at most 8 registers live) instead of being preloaded into
+// 2*E registers -- what lets 12 warps per SM fit the register file.
+// SOLMASK: bit i = stage i uses mul_shoup<true>.
 __device__ __forceinline__ u32 comp4(const uint4 &v, int i) { return i == 0 ? v.x : i == 1 ? v.y : i == 2 ? v.z : v.w; }
 // PRE: the products of the FIRST stage arrive precomputed in pre[0 .. E/2) (digit transforms: twiddle * small digit comes
 // from a 128-entry table, see blind_rotate_kernel), x[E/2 ..) is not read.
-template <int E, bool UNI, int SOLMASK = 0, bool STREAM = false, bool PRE = false>
-__device__ __forceinline__ void ct_pass(u32 (&x)[E], const u32 *__restrict__ utw, const u32 *__restrict__ utws,
-                                        const u32 (&w)[E], const u32 (&ws)[E], u32 Q, u32 Q2, const u32 *tab = nullptr,
-                                        const u32 *tabs = nullptr, int lane = 0, const u32 *pre = nullptr, SolSh sh = SolSh{16, 11, 0}) {
+template <int E, bool UNI, int SOLMASK = 0, bool PRE = false>
+__device__ __forceinline__ void ct_pass(u32 (&x)[E], const u32 *__restrict__ utw, const u32 *__restrict__ utws, u32 Q, u32 Q2,
+                                        const u32 *tab = nullptr, const u32 *tabs = nullptr, int lane = 0, const u32 *pre = nullptr) {
   int si = 0;
   uint4 cw = make_uint4(0, 0, 0, 0), cws = cw;
 #pragma unroll
@@ -204,21 +95,21 @@ __device__ __forceinline__ void ct_pass(u32 (&x)[E], const u32 *__restrict__ utw
       const int p = E / (2 * t) + gi;
       u32 ww, wws;
       if (UNI) { ww = utw[p]; wws = utws[p]; }
-      else if (STREAM) {
+      else {
         if ((p & 3) == 0 || gi == 0) {
           cw = reinterpret_cast<const uint4 *>(tab)[(p >> 2) * 32 + lane];
           cws = reinterpret_cast<const uint4 *>(tabs)[(p >> 2) * 32 + lane];
         }
         ww = comp4(cw, p & 3); wws = comp4(cws, p & 3);
-      } else { ww = w[p]; wws = ws[p]; }
+      }
 #pragma unroll
       for (int j = 0; j < t; j++) {
         const int a = gi * 2 * t + j, b = a + t;
         u32 T;
         if (PRE && si == 0) T = pre[j];
-        else T = sol ? mul_shoup<true>(x[b], ww, wws, Q, sh) : mul_shoup<false>(x[b], ww, wws, Q);
+        else T = sol ? mul_shoup<true>(x[b], ww, wws, Q) : mul_shoup<false>(x[b], ww, wws, Q);
         x[b] = x[a] - T + Q2;
-        x[a] = add2(x[a], T, sh);
+        x[a] = x[a] + T;
       }
     }
   }
@@ -227,14 +118,14 @@ __device__ __forceinline__ void ct_pass(u32 (&x)[E], const u32 *__restrict__ utw
 // Gentleman-Sande (inverse, unscaled).  B = bound of the inputs in units of Q (<= 16).  Sums double
 // per stage; when they would pass 32Q (= just under 2^32) they are pulled back below 2Q with one
 // lazy Barrett step.  Differences go through the Shoup multiply, which accepts any 32-bit input.
-template <int E, int T, int B, bool UNI, int MAXLAST, int SOLMASK = 0, int SI = 0, bool STREAM = false> struct GsRun {
+// Twiddles as in ct_pass.
+template <int E, int T, int B, bool UNI, int MAXLAST> struct GsRun {
   static constexpr int NB = 2 * B;
   static constexpr bool LAST = (2 * T >= E);
   static constexpr bool RED = LAST ? (NB > MAXLAST) : (NB > 16); // pull the sums back below 2Q after this stage?
   static constexpr int OUTB = RED ? 2 : NB;
-  __device__ __forceinline__ static void run(u32 (&x)[E], const u32 *__restrict__ utw, const u32 *__restrict__ utws,
-                                             const u32 (&w)[E], const u32 (&ws)[E], u32 Q, u32 mu, const u32 *tab = nullptr,
-                                             const u32 *tabs = nullptr, int lane = 0, SolSh sh = SolSh{16, 11, 0}) {
+  __device__ __forceinline__ static void run(u32 (&x)[E], const u32 *__restrict__ utw, const u32 *__restrict__ utws, u32 Q,
+                                             const u32 *tab = nullptr, const u32 *tabs = nullptr, int lane = 0) {
     static_assert(B <= 16, "GS input bound too large");
     const u32 off = B * Q;
     uint4 cw = make_uint4(0, 0, 0, 0), cws = cw;
@@ -243,23 +134,23 @@ template <int E, int T, int B, bool UNI, int MAXLAST, int SOLMASK = 0, int SI = 
       const int p = E / (2 * T) + gi;
       u32 ww, wws;
       if (UNI) { ww = utw[p]; wws = utws[p]; }
-      else if (STREAM) {
+      else {
         if ((p & 3) == 0 || gi == 0) {
           cw = reinterpret_cast<const uint4 *>(tab)[(p >> 2) * 32 + lane];
           cws = reinterpret_cast<const uint4 *>(tabs)[(p >> 2) * 32 + lane];
         }
         ww = comp4(cw, p & 3); wws = comp4(cws, p & 3);
-      } else { ww = w[p]; wws = ws[p]; }
+      }
 #pragma unroll
       for (int j = 0; j < T; j++) {
         const int a = gi * 2 * T + j, b = a + T;
-        u32 S = add2(x[a], x[b], sh);
+        u32 S = x[a] + x[b];
         u32 D = x[a] - x[b] + off;
-        x[b] = mul_shoup<((SOLMASK >> SI) & 1) != 0>(D, ww, wws, Q, sh);
-        x[a] = RED ? lazy_reduce(S, Q, mu) : S;
+        x[b] = mul_shoup(D, ww, wws, Q);
+        x[a] = RED ? lazy_reduce(S, Q) : S;
       }
     }
-    if constexpr (!LAST) GsRun<E, 2 * T, OUTB, UNI, MAXLAST, SOLMASK, SI + 1, STREAM>::run(x, utw, utws, w, ws, Q, mu, tab, tabs, lane, sh);
+    if constexpr (!LAST) GsRun<E, 2 * T, OUTB, UNI, MAXLAST>::run(x, utw, utws, Q, tab, tabs, lane);
   }
 };
 // bound (in units of Q) of the values GsRun<E,1,B0,*,MAXLAST> leaves behind
@@ -281,15 +172,13 @@ struct TwTabs { // shared-memory per-lane twiddle tables, each N words
 };
 
 // forward: x in column layout (index lane+32k, coefficient form, values < Q) -> row layout (index E*lane+j,
-// evaluation form, lazy < (2*logN+1)Q).  buf: N-word smem scratch, left holding garbage.
-template <int LOGN, int SOLW = 0, int SOLN = 0, bool PRE = false>
+// evaluation form, lazy < (2*logN+1)Q).  buf: N-word smem scratch, left holding garbage.  SOLW / SOLN: SOLMASK of the wide / narrow pass.
+template <int LOGN, bool PRE = false, int SOLW = 0, int SOLN = 0>
 __device__ __forceinline__ void ntt_forward(u32 (&x)[(1 << LOGN) / 32], u32 *buf, const DevConst &P, const TwTabs &tt, int lane,
                                             const u32 *pre = nullptr) {
   constexpr int E = (1 << LOGN) / 32;
   const u32 Q = P.Q, Q2 = P.Q2;
-  const SolSh sh = sol_shifts(P);
-  u32 w[E], ws[E];
-  ct_pass<E, true, SOLW, false, PRE>(x, P.tw, P.tws, w, ws, Q, Q2, nullptr, nullptr, 0, pre, sh);
+  ct_pass<E, true, SOLW, PRE>(x, P.tw, P.tws, Q, Q2, nullptr, nullptr, 0, pre);
   if constexpr (LOGN & 1) { // span-16 stage across lanes (lane bit 4): group index = k, twiddle psi_br[16+k]
     const bool up = lane & 16;
 #pragma unroll
@@ -303,53 +192,37 @@ __device__ __forceinline__ void ntt_forward(u32 (&x)[(1 << LOGN) / 32], u32 *buf
   col_store<E>(buf, x, lane);
   __syncwarp();
   row_load<E>(buf, x, lane);
-  if constexpr (BFHE_STREAM_TW) {
-    ct_pass<E, false, SOLN, true>(x, P.tw, P.tws, w, ws, Q, Q2, tt.fw, tt.fws, lane, nullptr, sh);
-  } else {
-    load_lane_tw<E>(tt.fw, w, lane);
-    load_lane_tw<E>(tt.fws, ws, lane);
-    ct_pass<E, false, SOLN>(x, P.tw, P.tws, w, ws, Q, Q2, nullptr, nullptr, 0, nullptr, sh);
-  }
+  ct_pass<E, false, SOLN>(x, P.tw, P.tws, Q, Q2, tt.fw, tt.fws, lane);
 }
 
 // two forward transforms at once (two digit polynomials of the same accumulator component): twice the independent butterflies
 // per stage for the scheduler, which with two warps per scheduler is what a transform lacks to keep the FMA-heavy pipe busy
-template <int LOGN, int SOLW = 0, int SOLN = 0, bool PRE = false>
+template <int LOGN, bool PRE = false>
 __device__ __forceinline__ void ntt_forward2(u32 (&xa)[(1 << LOGN) / 32], u32 (&xb)[(1 << LOGN) / 32], u32 *bufa, u32 *bufb, const DevConst &P,
                                              const TwTabs &tt, int lane, const u32 *prea = nullptr, const u32 *preb = nullptr) {
   constexpr int E = (1 << LOGN) / 32;
   static_assert((LOGN & 1) == 0, "even log2 N only");
   const u32 Q = P.Q, Q2 = P.Q2;
-  const SolSh sh = sol_shifts(P);
-  u32 w[E], ws[E];
-  ct_pass<E, true, SOLW, false, PRE>(xa, P.tw, P.tws, w, ws, Q, Q2, nullptr, nullptr, 0, prea, sh);
-  ct_pass<E, true, SOLW, false, PRE>(xb, P.tw, P.tws, w, ws, Q, Q2, nullptr, nullptr, 0, preb, sh);
+  ct_pass<E, true, 0, PRE>(xa, P.tw, P.tws, Q, Q2, nullptr, nullptr, 0, prea);
+  ct_pass<E, true, 0, PRE>(xb, P.tw, P.tws, Q, Q2, nullptr, nullptr, 0, preb);
   __syncwarp();
   col_store<E>(bufa, xa, lane);
   col_store<E>(bufb, xb, lane);
   __syncwarp();
   row_load<E>(bufa, xa, lane);
   row_load<E>(bufb, xb, lane);
-  ct_pass<E, false, SOLN, true>(xa, P.tw, P.tws, w, ws, Q, Q2, tt.fw, tt.fws, lane, nullptr, sh);
-  ct_pass<E, false, SOLN, true>(xb, P.tw, P.tws, w, ws, Q, Q2, tt.fw, tt.fws, lane, nullptr, sh);
+  ct_pass<E, false>(xa, P.tw, P.tws, Q, Q2, tt.fw, tt.fws, lane);
+  ct_pass<E, false>(xb, P.tw, P.tws, Q, Q2, tt.fw, tt.fws, lane);
 }
 
 // inverse (unscaled: N * true value; the keys carry N^-1): x in row layout (evaluation form, values < B0*Q)
 // -> column layout, coefficient form, fully reduced to [0,Q).
-template <int LOGN, int B0, int SOLN = 0, int SOLW = 0>
+template <int LOGN, int B0>
 __device__ __forceinline__ void ntt_inverse(u32 (&x)[(1 << LOGN) / 32], u32 *buf, const DevConst &P, const TwTabs &tt, int lane) {
   constexpr int E = (1 << LOGN) / 32;
-  const u32 Q = P.Q, mu = P.mu;
-  const SolSh sh = sol_shifts(P);
-  u32 w[E], ws[E];
+  const u32 Q = P.Q;
   constexpr int ML = (LOGN & 1) ? 8 : 16; // what the next stage can take
-  if constexpr (BFHE_STREAM_TW) {
-    GsRun<E, 1, B0, false, ML, SOLN, 0, true>::run(x, P.itw, P.itws, w, ws, Q, mu, tt.iw, tt.iws, lane, sh);
-  } else {
-    load_lane_tw<E>(tt.iw, w, lane);
-    load_lane_tw<E>(tt.iws, ws, lane);
-    GsRun<E, 1, B0, false, ML, SOLN>::run(x, P.itw, P.itws, w, ws, Q, mu, nullptr, nullptr, 0, sh);
-  }
+  GsRun<E, 1, B0, false, ML>::run(x, P.itw, P.itws, Q, tt.iw, tt.iws, lane);
   constexpr int B1 = gs_out_bound(E, B0, ML);
   __syncwarp();
   row_store<E>(buf, x, lane);
@@ -367,12 +240,12 @@ __device__ __forceinline__ void ntt_inverse(u32 (&x)[(1 << LOGN) / 32], u32 *buf
       x[k] = up ? mul_shoup(D, P.itw[16 + k], P.itws[16 + k], Q) : (x[k] + o);
     }
     constexpr int B2 = 2 * B1;
-    GsRun<E, 1, B2, true, 32, SOLW>::run(x, P.itw, P.itws, w, ws, Q, mu, nullptr, nullptr, 0, sh);
+    GsRun<E, 1, B2, true, 32>::run(x, P.itw, P.itws, Q);
   } else {
-    GsRun<E, 1, B1, true, 32, SOLW>::run(x, P.itw, P.itws, w, ws, Q, mu, nullptr, nullptr, 0, sh);
+    GsRun<E, 1, B1, true, 32>::run(x, P.itw, P.itws, Q);
   }
 #pragma unroll
-  for (int k = 0; k < E; k++) x[k] = csub(lazy_reduce(x[k], Q, mu), Q);
+  for (int k = 0; k < E; k++) x[k] = csub(lazy_reduce(x[k], Q), Q);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -391,7 +264,7 @@ template <int LOGN, int DG, int LOGBG, int G, bool AP> struct BrCfg {
   static constexpr int NPAD = AP ? 1024 : 512; // per-gate index table (>= n*dR for AP, >= n for GINX)
   static constexpr size_t dct_words = (size_t)G * ROWS * N;
   // first-stage product table: twiddle * (digit - B/2) mod Q for the 2^LOGBG digit values, one copy per bank (STD128_OPT shape only)
-  static constexpr bool LUT = (LOGBG == 7 && LOGN == 10 && G <= 4);
+  static constexpr bool LUT = (LOGBG == 7 && LOGN == 10);
   static constexpr size_t lut_words = LUT ? (size_t)32 << LOGBG : 0;
   static constexpr size_t smem_bytes = (dct_words + 4 * N + (AP ? 0 : 2 * N) + lut_words) * 4 + (size_t)G * NPAD * 2;
 };
@@ -407,7 +280,7 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
   extern __shared__ __align__(128) unsigned char smem_raw[];
   u32 *dct = reinterpret_cast<u32 *>(smem_raw);                 // [G][ROWS][N]
   u32 *s_tw = dct + Cfg::dct_words;                             // fw | fws | iw | iws
-  u32 *s_psiM = s_tw + 4 * N;                                   // [2N] Montgomery psi^k (GINX)
+  u32 *s_psiM = s_tw + 4 * N;                                   // [2N] monomial-factor table (GINX; N entries used)
   u32 *s_lut = s_psiM + (AP ? 0 : 2 * N);                       // [2^LOGBG][32] (Cfg::LUT)
   u16 *s_idx = reinterpret_cast<u16 *>(s_lut + Cfg::lut_words); // [G][NPAD]
 
@@ -424,13 +297,8 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
   const u32 Q = P.Q, q = P.q, n = P.n;
 
   for (int i = tid; i < 4 * N; i += Cfg::THREADS) s_tw[i] = g_twl[i];
-  if (!AP) {
-    if constexpr (G > 4) { // register-lean form: psi^k table, factors by Montgomery product
-      for (int i = tid; i < 2 * N; i += Cfg::THREADS) s_psiM[i] = g_psiM[i];
-    } else { // monomial-factor table (psi^(2u) - 1), see the external product
-      for (int u = tid; u < N; u += Cfg::THREADS) s_psiM[f_phys((u32)u)] = (g_psiM[2 * u] + (P.Q - P.oneM)) % P.Q;
-    }
-  }
+  if (!AP) // monomial-factor table (psi^(2u) - 1), see the external product
+    for (int u = tid; u < N; u += Cfg::THREADS) s_psiM[f_phys((u32)u)] = (g_psiM[2 * u] + (P.Q - P.oneM)) % P.Q;
   const TwTabs tt{s_tw, s_tw + N, s_tw + 2 * N, s_tw + 3 * N};
 
   // ---- prologue: LWE prep (EvalBinGate's ct1+ct2 / 2(ct1-ct2) / Bootstrap's b+q/4, with fused EvalNOT) ----
@@ -487,9 +355,15 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
   u32 *mybuf = dct + ((size_t)g * ROWS + c) * N; // R[g][c] aliases dct row c of gate g
 
   // MAC work split: item -> (chunk qc, gate split)
-  constexpr bool LEAN = (G > 4); // 3 warps per scheduler: fit 168 registers (no digit array, one output component of keys at a time)
-  constexpr int GS = LEAN ? G / 2 : ((W >= C) ? (W / C) : 1);
+  constexpr int GS = (W >= C) ? (W / C) : 1;
   const u32 eA = 2 * brev(lane, 5) + 1; // lane part of the evaluation-point exponent 2*br(idx)+1
+  // two digits per pass (STD128_OPT shape): +8 % at two gates per CTA (71.3k -> 77.0k gates/s), nothing at four (79.3k vs 79.7k),
+  // where the phase is already within ~20 % of its pipe bound (tools/phase_timing.py) -- used for G <= 2 only
+  constexpr bool PAIRED = Cfg::LUT && DG % 2 == 0 && G <= 2;
+  // GINX, one digit per pass: the step's key words are requested BEFORE the warp's last digit transform, so the L2 round trip runs under
+  // the transform and the wait at the CTA barrier instead of in front of the product (535 cycles of a 27 k-cycle step sat there,
+  // tools/phase_timing.py; DESIGN.md 5.1)
+  constexpr bool KEY_HOIST = !AP && !PAIRED;
 
 #ifdef BFHE_PHASE_TIMING
   long long tpt[5] = {0, 0, 0, 0, 0}, tq0 = clock64(), tq1;
@@ -498,16 +372,16 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
 #define PT_T(i)
 #endif
   for (int step = 0; step < nsteps; step++) {
-    // key words of the external product (GINX: [sign][row][column]; AP: a double buffer over the gates, see below).  GINX, four gates per
-    // CTA: the first half is requested BEFORE the warp's last digit transform and the second half right after it, so the L2 round trip runs
-    // under the transform and the wait at the CTA barrier instead of in front of the product (BFHE_KEY_HOIST; 535 cycles of a 27 k-cycle step
-    // sat there, tools/phase_timing.py)
-    uint4 kr[2][ROWS][LEAN ? 1 : 2];
-    constexpr bool PAIRED_ANY = Cfg::LUT && !LEAN && (DG % 2 == 0) && G <= BFHE_PAIRED_MAXG && BFHE_PAIRED_DIGITS;
-    constexpr bool KEY_HOIST = !AP && !LEAN && !PAIRED_ANY && BFHE_KEY_HOIST;
-    // AP: hoisting the first gate's key the same way helps one wave (47.3 k -> 48.8 k gates/s at 592 gates) and hurts eight (47.4 k -> 45.5 k at
-    // 4 736: the 2 GB key does not stay in L2 and the earlier requests spread the CTAs' working set); off
-    constexpr bool AP_HOIST = AP && !LEAN && !PAIRED_ANY && BFHE_KEY_HOIST && BFHE_AP_HOIST;
+    // key words of the external product (GINX: [sign][row][column]; AP: a double buffer over the gates, see below)
+    uint4 kr[2][ROWS][2];
+#define BFHE_GX_LOAD(qc) /* GINX: this step's key words of chunk qc, both signs */                                    \
+  do {                                                                                                                 \
+    const u32 *kb_ = bk + (size_t)step * (2 * ROWS * 2) * N + ((qc) * 32 + lane) * 4;                                  \
+    _Pragma("unroll") for (int s = 0; s < 2; s++)                                                                      \
+      _Pragma("unroll") for (int r = 0; r < ROWS; r++)                                                                 \
+        _Pragma("unroll") for (int cc = 0; cc < 2; cc++)                                                               \
+          kr[s][r][cc] = __ldg(reinterpret_cast<const uint4 *>(kb_ + (size_t)((s * ROWS + r) * 2 + cc) * N));           \
+  } while (0)
     // AP: every gate has its own key (BK[i][digit][k]), so nothing is shared between the gates of the CTA; the two halves of kr[] are a
     // double buffer instead -- gate j's words are requested while gate j - 1 is multiplied (the first two before the barrier), which takes
     // the L2 round trip of 16 LDG.128 per gate and step off the critical path
@@ -521,7 +395,7 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
   do {                                                                                                                 \
     const u32 *kb_ = (kb);                                                                                             \
     _Pragma("unroll") for (int r = 0; r < ROWS; r++)                                                                   \
-      _Pragma("unroll") for (int cc = 0; cc < (LEAN ? 1 : 2); cc++)                                                    \
+      _Pragma("unroll") for (int cc = 0; cc < 2; cc++)                                                                 \
         kr[buf][r][cc] = __ldg(reinterpret_cast<const uint4 *>(kb_ + (size_t)(r * 2 + cc) * N));                        \
   } while (0)
 
@@ -532,7 +406,7 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
       if (pending) {
         u32 x[E];
         row_load<E>(mybuf, x, lane);
-        ntt_inverse<LOGN, AP ? 8 : 4, BFHE_SOL_THR_NARROW, BFHE_SOL_THR_WIDE>(x, mybuf, P, tt, lane);
+        ntt_inverse<LOGN, AP ? 8 : 4>(x, mybuf, P, tt, lane);
 #pragma unroll
         for (int k = 0; k < E; k++) acc[k] = AP ? x[k] : csub(acc[k] + x[k], Q);
       }
@@ -541,14 +415,9 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
       // position turns the balanced digits into the plain base-B digits of d + OFF, so digit l is one shift, one mask and
       // one subtraction with no dependency on the digits below it (the top digit wraps exactly like the reference's
       // sign-truncation when dG digits do not cover the centred range, e.g. TOY).
-      u32 dp[LEAN ? 1 : E];
-      if constexpr (!LEAN) {
+      u32 dp[E];
 #pragma unroll
-        for (int k = 0; k < E; k++) dp[k] = ((acc[k] < (Q >> 1)) ? acc[k] : acc[k] - Q) + DIGIT_OFF;
-      }
-      // two digits per pass (STD128_OPT shape): +8 % at two gates per CTA (71.3k -> 77.0k gates/s), nothing at four (79.3k vs 79.7k),
-      // where the phase is already within ~20 % of its pipe bound (tools/phase_timing.py) -- used for G <= 2 only
-      constexpr bool PAIRED = Cfg::LUT && !LEAN && (DG % 2 == 0) && G <= BFHE_PAIRED_MAXG && BFHE_PAIRED_DIGITS;
+      for (int k = 0; k < E; k++) dp[k] = ((acc[k] < (Q >> 1)) ? acc[k] : acc[k] - Q) + DIGIT_OFF;
       if constexpr (PAIRED) {
 #pragma unroll
         for (int l = 0; l < DG; l += 2) {
@@ -565,7 +434,7 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
             }
           }
           u32 *bufa = dct + ((size_t)g * ROWS + c + 2 * l) * N, *bufb = bufa + 2 * N;
-          ntt_forward2<LOGN, BFHE_SOL_THR_WIDE, BFHE_SOL_THR_NARROW, true>(xa, xb, bufa, bufb, P, tt, lane, prea, preb);
+          ntt_forward2<LOGN, true>(xa, xb, bufa, bufb, P, tt, lane, prea, preb);
           row_store<E>(bufa, xa, lane);
           row_store<E>(bufb, xb, lane);
         }
@@ -575,131 +444,37 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
         u32 x[E], pre[Cfg::LUT ? E / 2 : 1];
 #pragma unroll
         for (int k = 0; k < E; k++) {
-          const u32 dpk = LEAN ? (((acc[k] < (Q >> 1)) ? acc[k] : acc[k] - Q) + DIGIT_OFF) : dp[LEAN ? 0 : k];
-          const u32 dgt = (dpk >> (LOGBG * l)) & ((1u << LOGBG) - 1);
+          const u32 dgt = (dp[k] >> (LOGBG * l)) & ((1u << LOGBG) - 1);
           // digit - B/2 + Q: congruent to the signed digit, lazy in (Q - B/2, Q + B/2); the forward transform needs no canonical
           // input (values then stay below (2 logN + 2) Q < 2^32)
           if (Cfg::LUT && k >= E / 2) { pre[Cfg::LUT ? k - E / 2 : 0] = s_lut[(dgt << 5) + lane]; x[k] = 0; }
           else x[k] = dgt + (Q - (1u << (LOGBG - 1)));
         }
         u32 *buf = dct + ((size_t)g * ROWS + c + 2 * l) * N;
-        if (AP_HOIST && l == DG - 1 && warp < C * GS) BFHE_AP_LOAD(0, ap_key(warp / C, warp % C));
-        if (KEY_HOIST && l == DG - 1 && warp < C * GS) {
-          const u32 *kb = bk + (size_t)step * (2 * ROWS * 2) * N + ((warp % C) * 32 + lane) * 4;
-#pragma unroll
-          for (int sg = 0; sg < BFHE_KEY_HOIST; sg++)
-#pragma unroll
-          for (int r = 0; r < ROWS; r++)
-#pragma unroll
-            for (int cc = 0; cc < 2; cc++) kr[sg][r][cc] = __ldg(reinterpret_cast<const uint4 *>(kb + (size_t)((sg * ROWS + r) * 2 + cc) * N));
-        }
-        ntt_forward<LOGN, BFHE_SOL_THR_WIDE, BFHE_SOL_THR_NARROW, Cfg::LUT>(x, buf, P, tt, lane, pre);
+        if (KEY_HOIST && l == DG - 1 && warp < C * GS) BFHE_GX_LOAD(warp % C);
+        ntt_forward<LOGN, Cfg::LUT>(x, buf, P, tt, lane, pre);
         row_store<E>(buf, x, lane);
       }
       }
-    } else if (AP_HOIST && warp < C * GS) { // this warp's gate skips the step (digit 0) or does not exist: no transform to hide behind
-      BFHE_AP_LOAD(0, ap_key(warp / C, warp % C));
     } else if (KEY_HOIST && warp < C * GS) { // empty gate slot (ragged last CTA): no transform to hide behind, but the product still needs the words
-      const u32 *kb = bk + (size_t)step * (2 * ROWS * 2) * N + ((warp % C) * 32 + lane) * 4;
-#pragma unroll
-      for (int sg = 0; sg < BFHE_KEY_HOIST; sg++)
-#pragma unroll
-      for (int r = 0; r < ROWS; r++)
-#pragma unroll
-        for (int cc = 0; cc < 2; cc++) kr[sg][r][cc] = __ldg(reinterpret_cast<const uint4 *>(kb + (size_t)((sg * ROWS + r) * 2 + cc) * N));
+      BFHE_GX_LOAD(warp % C);
     }
     pending = pending || active;
     PT_T(0);
-    // GINX: this warp's first key chunk is requested BEFORE the barrier, so the L2 round trip overlaps the wait for
-    // the slower warps of the CTA instead of stalling the external product (ncu r1: 6 % of samples sat on these loads)
-    if (AP && !LEAN && warp < C * GS) {
-      if (!AP_HOIST) BFHE_AP_LOAD(0, ap_key(warp / C, warp % C));
+    // the first key words of this warp's chunk are requested BEFORE the barrier, so the L2 round trip overlaps the wait for the slower
+    // warps of the CTA instead of stalling the external product (ncu r1: 6 % of samples sat on these loads)
+    if (AP && warp < C * GS) {
+      BFHE_AP_LOAD(0, ap_key(warp / C, warp % C));
       if (JN > 1) BFHE_AP_LOAD(1, ap_key(warp / C + GS, warp % C));
     }
-    if (!AP && warp < C * GS) {
-      const u32 *kb = bk + (size_t)step * (2 * ROWS * 2) * N + ((warp % C) * 32 + lane) * 4;
-#pragma unroll
-      for (int s = KEY_HOIST ? BFHE_KEY_HOIST : 0; s < 2; s++)
-#pragma unroll
-        for (int r = 0; r < ROWS; r++)
-#pragma unroll
-          for (int cc = 0; cc < (LEAN ? 1 : 2); cc++)
-            kr[s][r][cc] = __ldg(reinterpret_cast<const uint4 *>(kb + (size_t)((s * ROWS + r) * 2 + cc) * N));
-    }
+    if (!AP && !KEY_HOIST && warp < C * GS) BFHE_GX_LOAD(warp % C);
     __syncthreads();
     PT_T(1);
 
     // ================= phase B: external product, slot-parallel over the CTA =================
-    if constexpr (LEAN) {
-      // register-lean form: keys of ONE output component (2 signs x ROWS uint4 = 64 registers) at a time, reused by
-      // the gates of this item's group; component-0 results wait in registers until component 1 has read the rows
-      for (int item = warp; item < C * GS; item += W) {
-        const int qc = item % C, gs0 = item / C;
-        u32 eB[4];
-#pragma unroll
-        for (int r = 0; r < 4; r++) eB[r] = 2 * ((brev(r, 2) << (LOGN - 2)) | (brev(qc, LOGN - 7) << 5));
-        u32 out0[G / GS][4];
-#pragma unroll
-        for (int cc = 0; cc < 2; cc++) {
-          if (item != warp || cc == 1) {
-            const u32 *kb = bk + (size_t)step * (2 * ROWS * 2) * N + (qc * 32 + lane) * 4;
-#pragma unroll
-            for (int s = 0; s < 2; s++)
-#pragma unroll
-              for (int r = 0; r < ROWS; r++) kr[s][r][0] = __ldg(reinterpret_cast<const uint4 *>(kb + (size_t)((s * ROWS + r) * 2 + cc) * N));
-          }
-#pragma unroll
-          for (int gl = 0; gl < G / GS; gl++) {
-            const int gg = gs0 + gl * GS;
-            if (gg >= gcount) continue;
-            u32 fp[4], fn[4];
-            const u32 m = s_idx[gg * NPAD + step], mask = 2 * N - 1;
-            const u32 ia = (m * eA) & mask;
-            const u32 A = s_psiM[ia], Ai = s_psiM[(2 * N - ia) & mask];
-            const u32 om = Q - P.oneM;
-#pragma unroll
-            for (int r = 0; r < 4; r++) {
-              const u32 ib = (m * eB[r]) & mask;
-              const u32 Bv = s_psiM[ib], Bi = s_psiM[(2 * N - ib) & mask];
-              fp[r] = redc((u64)A * Bv, Q, P.qinv_neg) + om;
-              fn[r] = redc((u64)Ai * Bi, Q, P.qinv_neg) + om;
-            }
-            u32 *gd = dct + (size_t)gg * ROWS * N + Lay<E>::chunk_off(lane, qc);
-            u64 sp[4] = {0, 0, 0, 0}, sn[4] = {0, 0, 0, 0};
-#pragma unroll
-            for (int r = 0; r < ROWS; r++) {
-              const uint4 dv = *reinterpret_cast<const uint4 *>(gd + (size_t)r * N);
-              const uint4 kp = kr[0][r][0], kn = kr[1][r][0];
-              sp[0] += (u64)dv.x * kp.x; sp[1] += (u64)dv.y * kp.y; sp[2] += (u64)dv.z * kp.z; sp[3] += (u64)dv.w * kp.w;
-              sn[0] += (u64)dv.x * kn.x; sn[1] += (u64)dv.y * kn.y; sn[2] += (u64)dv.z * kn.z; sn[3] += (u64)dv.w * kn.w;
-            }
-            u32 out[4];
-#pragma unroll
-            for (int sl = 0; sl < 4; sl++)
-              out[sl] = redc((u64)redc(sp[sl], Q, P.qinv_neg) * fp[sl] + (u64)redc(sn[sl], Q, P.qinv_neg) * fn[sl], Q, P.qinv_neg);
-            if (cc == 0) {
-#pragma unroll
-              for (int sl = 0; sl < 4; sl++) out0[gl][sl] = out[sl];
-            } else {
-              *reinterpret_cast<uint4 *>(gd) = make_uint4(out0[gl][0], out0[gl][1], out0[gl][2], out0[gl][3]);
-              *reinterpret_cast<uint4 *>(gd + (size_t)N) = make_uint4(out[0], out[1], out[2], out[3]);
-            }
-          }
-        }
-      }
-    } else {
     for (int item = warp; item < C * GS; item += W) {
       const int qc = item % C, gs0 = item / C;
-      if (!AP && item != warp) { // further chunks of this warp (fewer warps than chunks)
-        const u32 *kb = bk + (size_t)step * (2 * ROWS * 2) * N + (qc * 32 + lane) * 4;
-#pragma unroll
-        for (int s = 0; s < 2; s++)
-#pragma unroll
-          for (int r = 0; r < ROWS; r++)
-#pragma unroll
-            for (int cc = 0; cc < 2; cc++)
-              kr[s][r][cc] = __ldg(reinterpret_cast<const uint4 *>(kb + (size_t)((s * ROWS + r) * 2 + cc) * N));
-      }
+      if (!AP && item != warp) BFHE_GX_LOAD(qc); // further chunks of this warp (fewer warps than chunks)
       // exponent parts that depend on (chunk, slot-in-chunk)
       u32 eB[4];
 #pragma unroll
@@ -712,16 +487,13 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
 #pragma unroll
       for (int j = 0; j < JN; j++) {
         const int gg = gs0 + j * GS;
-        constexpr int KB0 = 0; // (silences unused warnings when AP is false)
-        (void)KB0;
         const bool ap_active = AP && gg < gcount && s_idx[(gg < gcount ? gg : 0) * NPAD + step] != 0;
         if (gg >= gcount || (AP && !ap_active)) { // nothing to multiply for this gate in this step; keep the double buffer moving
           if (AP && j + 2 < JN) { if ((j & 1) == 0) BFHE_AP_LOAD(0, ap_key(gs0 + (j + 2) * GS, qc)); else BFHE_AP_LOAD(1, ap_key(gs0 + (j + 2) * GS, qc)); }
           continue;
         }
         u32 fp[4], fn[4];
-        if (AP) {
-        } else {
+        if (!AP) {
           // monomial factors (X^m - 1), (X^-m - 1) at this thread's 4 evaluation points, Montgomery form
           // (exponents are even -- m is a multiple of 2N/q = 2 -- so the table has N entries, (psi^(2u) - 1) * 2^32 mod Q at f_phys(u): one
           // gather per factor instead of two gathers and a Montgomery product; the index fold keeps the 32 lanes of a warp, whose u differ
@@ -769,7 +541,6 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
         }
       }
     }
-    }
     PT_T(2);
     __syncthreads();
     PT_T(3);
@@ -780,7 +551,7 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
     if (pending) {
       u32 x[E];
       row_load<E>(mybuf, x, lane);
-      ntt_inverse<LOGN, AP ? 8 : 4, BFHE_SOL_THR_NARROW, BFHE_SOL_THR_WIDE>(x, mybuf, P, tt, lane);
+      ntt_inverse<LOGN, AP ? 8 : 4>(x, mybuf, P, tt, lane);
 #pragma unroll
       for (int k = 0; k < E; k++) acc[k] = AP ? x[k] : csub(acc[k] + x[k], Q);
     }
@@ -823,25 +594,25 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
 template <int T, int B> struct Gs8Stage { // one Gentleman-Sande stage on 8 registers, half-size T; B = input bound in units of Q
   static constexpr bool RED = (2 * B > 16);
   static constexpr int OUTB = RED ? 2 : 2 * B;
-  __device__ __forceinline__ static void run(u32 (&x)[8], const u32 (&w)[8], const u32 (&ws)[8], u32 Q, u32 mu) {
+  __device__ __forceinline__ static void run(u32 (&x)[8], const u32 (&w)[8], const u32 (&ws)[8], u32 Q) {
     static_assert(B <= 16, "bound");
 #pragma unroll
     for (int i = 0; i < 4; i++) {
       const int gi = i / T, a = gi * 2 * T + (i % T), b = a + T, p = 4 / T + gi;
       const u32 S = x[a] + x[b], D = x[a] - x[b] + B * Q;
       x[b] = mul_shoup(D, w[p], ws[p], Q);
-      x[a] = RED ? lazy_reduce(S, Q, mu) : S;
+      x[a] = RED ? lazy_reduce(S, Q) : S;
     }
   }
 };
 template <int B0> __device__ __forceinline__ void ntt_inverse_quad8(u32 (&x)[8], u32 *buf, const DevConst &P, const u32 *nat, const u32 *nats, int T,
                                                                    int bar_id) {
-  const u32 Q = P.Q, mu = P.mu;
+  const u32 Q = P.Q;
   u32 w[8], ws[8];
   auto run3 = [&](auto BC) { // three stages, returns nothing; bounds advance at compile time
     constexpr int B = decltype(BC)::value;
     using S1 = Gs8Stage<1, B>; using S2 = Gs8Stage<2, S1::OUTB>; using S3 = Gs8Stage<4, S2::OUTB>;
-    S1::run(x, w, ws, Q, mu); S2::run(x, w, ws, Q, mu); S3::run(x, w, ws, Q, mu);
+    S1::run(x, w, ws, Q); S2::run(x, w, ws, Q); S3::run(x, w, ws, Q);
   };
   constexpr int B1 = Gs8Stage<4, Gs8Stage<2, Gs8Stage<1, B0>::OUTB>::OUTB>::OUTB;
   constexpr int B2 = Gs8Stage<4, Gs8Stage<2, Gs8Stage<1, B1>::OUTB>::OUTB>::OUTB;
@@ -860,7 +631,7 @@ template <int B0> __device__ __forceinline__ void ntt_inverse_quad8(u32 (&x)[8],
     *reinterpret_cast<uint4 *>(p0) = make_uint4(x[0], x[1], x[2], x[3]);
     *reinterpret_cast<uint4 *>(p1) = make_uint4(x[4], x[5], x[6], x[7]);
   }
-  asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
+  bar_sync(bar_id, 128);
   { // middle pass: positions 64u + 8r + v
     const int u = T >> 3, v = T & 7;
     const int b = 64 * u + 8 * (u & 3) + 4 * (v >> 2) + (v & 3); // address of r = 0; r flips bits: 32 (r >> 2) + 8 (r & 3) + 4 (r >> 2)
@@ -875,7 +646,7 @@ template <int B0> __device__ __forceinline__ void ntt_inverse_quad8(u32 (&x)[8],
 #pragma unroll
     for (int r = 0; r < 8; r++) buf[b ^ (32 * (r >> 2) + 8 * (r & 3) + 4 * (r >> 2))] = x[r];
   }
-  asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
+  bar_sync(bar_id, 128);
   { // wide pass: positions T6 + 64 (k + 8 hi); the last stage across lanes 16 apart
     const int lane = T & 31, hi = lane >> 4, T6 = 16 * (T >> 5) + (lane & 15), l5 = T6 & 31, t5 = T6 >> 5;
 #pragma unroll
@@ -895,7 +666,7 @@ template <int B0> __device__ __forceinline__ void ntt_inverse_quad8(u32 (&x)[8],
       x[k] = hi ? m : x[k] + o;
     }
 #pragma unroll
-    for (int k = 0; k < 8; k++) x[k] = csub(lazy_reduce(x[k], Q, mu), Q);
+    for (int k = 0; k < 8; k++) x[k] = csub(lazy_reduce(x[k], Q), Q);
   }
 }
 
@@ -908,25 +679,6 @@ template <int B0> __device__ __forceinline__ void ntt_inverse_quad8(u32 (&x)[8],
 // (cp.async.bulk + mbarrier complete_tx) issued right after the previous step's external product, so the
 // L2 latency of the key is hidden behind the next step's transforms at no register or issue cost.
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ u32 smem_u32(const void *p) { return (u32)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(u64 *bar, u32 count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(u64 *bar, u32 bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, u32 bytes, u64 *bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(u64 *bar, u32 parity) {
-  asm volatile("{\n\t.reg .pred p;\n\tWAIT_%=:\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" ::"r"(
-                   smem_u32(bar)),
-               "r"(parity)
-               : "memory");
-}
-
 template <int LOGN, int DG, int LOGBG, bool AP> struct LatCfg {
   static constexpr int N = 1 << LOGN, E = N / 32, C = E / 4, ROWS = 2 * DG;
   static constexpr int W = ROWS, THREADS = 32 * W;
@@ -1081,7 +833,7 @@ blind_rotate_lat_kernel(const __grid_constant__ DevConst P, const DevGate *__res
         u32 x[E];
         u32 *rb = dct + (size_t)warp * N;
         row_load<E>(rb, x, lane);
-        ntt_inverse<LOGN, AP ? 8 : 4, BFHE_SOL_LAT_INV, BFHE_SOL_LAT_INV>(x, rb, P, tt, lane);
+        ntt_inverse<LOGN, AP ? 8 : 4>(x, rb, P, tt, lane);
 #pragma unroll
         for (int k = 0; k < E; k++) acc[k] = AP ? x[k] : csub(acc[k] + x[k], Q);
       }
@@ -1100,7 +852,7 @@ blind_rotate_lat_kernel(const __grid_constant__ DevConst P, const DevGate *__res
         x[k] = ((dig[c * N + lane + 32 * k] >> (LOGBG * l)) & ((1u << LOGBG) - 1)) + (Q - (1u << (LOGBG - 1))); // lazy: digit - B/2 + Q
       }
       u32 *buf = dct + (size_t)warp * N;
-      ntt_forward<LOGN, BFHE_SOL_LAT_WIDE, BFHE_SOL_LAT_NARROW>(x, buf, P, tt, lane);
+      ntt_forward<LOGN, false, SOL_LAT_WIDE, SOL_LAT_NARROW>(x, buf, P, tt, lane);
       row_store<E>(buf, x, lane);
     }
     PH_T(2);
@@ -1186,7 +938,7 @@ blind_rotate_lat_kernel(const __grid_constant__ DevConst P, const DevGate *__res
       u32 x[E];
       u32 *rb = dct + (size_t)warp * N;
       row_load<E>(rb, x, lane);
-      ntt_inverse<LOGN, AP ? 8 : 4, BFHE_SOL_LAT_INV, BFHE_SOL_LAT_INV>(x, rb, P, tt, lane);
+      ntt_inverse<LOGN, AP ? 8 : 4>(x, rb, P, tt, lane);
 #pragma unroll
       for (int k = 0; k < E; k++) acc[k] = AP ? x[k] : csub(acc[k] + x[k], Q);
     }
@@ -1217,12 +969,9 @@ static int launch_lat_inst(const DevConst &P, const DevGate *d_gates, int count,
   using Cfg = LatCfg<LOGN, DG, LOGBG, AP>;
   auto kern = blind_rotate_lat_kernel<LOGN, DG, LOGBG, AP>;
   static bool attr_done[64];
-  if (!attr_done[attr_device_slot()]) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::smem_bytes);
-    if (e != cudaSuccess) return (int)e;
-    attr_done[attr_device_slot()] = true;
-  }
-  if (count <= 0) return 0;
+  if (int rc = once_per_device(attr_done, [&] { return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::smem_bytes); }))
+    return rc;
+  if (count <= 0) return 0; // attribute warm-up only
   if (info) { info->gates_per_cta = 1; info->ctas = count; info->smem_bytes = Cfg::smem_bytes; }
   kern<<<count, Cfg::THREADS, Cfg::smem_bytes, st>>>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc);
   return (int)cudaGetLastError();
@@ -1234,11 +983,8 @@ static int launch_br_inst(const DevConst &P, const DevGate *d_gates, int count, 
   using Cfg = BrCfg<LOGN, DG, LOGBG, G, AP>;
   auto kern = blind_rotate_kernel<LOGN, DG, LOGBG, G, AP>;
   static bool attr_done[64];
-  if (!attr_done[attr_device_slot()]) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::smem_bytes);
-    if (e != cudaSuccess) return (int)e;
-    attr_done[attr_device_slot()] = true;
-  }
+  if (int rc = once_per_device(attr_done, [&] { return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::smem_bytes); }))
+    return rc;
   if (count <= 0) return 0; // attribute warm-up only
   const int ctas = (count + G - 1) / G;
   if (info) { info->gates_per_cta = G; info->ctas = ctas; info->smem_bytes = Cfg::smem_bytes; }
@@ -1252,7 +998,7 @@ static int launch_br_g(int G, const DevConst &P, const DevGate *d_gates, int cou
   switch (G) {
   case 1: return launch_br_inst<LOGN, DG, LOGBG, 1, AP>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc, st, info);
   case 2: return launch_br_inst<LOGN, DG, LOGBG, 2, AP>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc, st, info);
-  // (6 gates per CTA -- 3 warps per scheduler through the register-lean LEAN path -- measured 7 % slower than 4: not instantiated)
+  // (6 gates per CTA, 3 warps per scheduler with a register-lean product, measured 7 % slower than 4: DESIGN.md 5.4)
   default: return launch_br_inst<LOGN, DG, LOGBG, 4, AP>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc, st, info);
   }
 }
@@ -1268,11 +1014,9 @@ template <int LOGN, int DG, int LOGBG> static int br_attrs() {
   rc |= launch_lat_inst<LOGN, DG, LOGBG, true>(P, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
   return rc;
 }
-static int keyswitch_attrs();
 int blind_rotate_set_attrs() {
   int rc = br_attrs<10, 4, 7>();
   rc |= br_attrs<9, 3, 9>();
-  rc |= keyswitch_attrs();
   rc |= v2_set_attrs();
   rc |= clx_set_attrs();
   return rc;
@@ -1452,10 +1196,7 @@ __global__ void __launch_bounds__(COLS *RG) keyswitch_kernel(const __grid_consta
   peer_publish(px, gridDim.x);
 }
 
-#ifndef KS_CL4_UNROLL
-#define KS_CL4_UNROLL 16 // measured 8: 29.2 us, 16: 27.1 us, 32: 35.1 us per 33-gate wave
-#endif
-constexpr int ks_cl4_unroll = KS_CL4_UNROLL; // row gathers in flight per thread
+constexpr int ks_cl4_unroll = 16; // row gathers in flight per thread; measured 8: 29.2 us, 16: 27.1 us, 32: 35.1 us per 33-gate wave
 // The same key switch on a 4-CTA cluster per gate (packed uint16 KSK only): each CTA gathers a quarter of the N*dKS rows, rank 0 adds the
 // four partial sums out of its peers' shared memory (DSMEM) and finishes.  The one-CTA form is latency-bound (512 dependent row
 // gathers per thread, 55 us whatever the batch); narrow circuit waves (1.2 - 1.5 ms each) pay that every wave.
@@ -1468,8 +1209,7 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(COLS *RG) keyswitch_
   __shared__ u32 s_tot[COLS * 2];          // this CTA's sums, read by rank 0
   const int N = P.N, dKS = P.dKS, nrows = N * dKS, quarter = nrows / 4;
   const int tid = threadIdx.x, col = tid % COLS, rg = tid / COLS;
-  u32 rank;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
+  const u32 rank = cluster_rank();
   const size_t gate = blockIdx.x >> 2;
   const u32 *e = ext + gate * (N + 4);
   for (int r = tid; r < quarter; r += COLS * RG) {
@@ -1500,7 +1240,7 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(COLS *RG) keyswitch_
       s_tot[col * 2 + h] = t;
     }
   }
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+  cluster_sync_all();
   if (rank == 0 && rg == 0 && col < rowlen_words) {
     const u64 qKS = P.qKS, q = P.q;
     u32 *out = gates[gate].out;
@@ -1510,9 +1250,8 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(COLS *RG) keyswitch_
       if (k > n) break;
       u64 sum = s_tot[col * 2 + h];
       for (u32 pr = 1; pr < 4; pr++) {
-        u32 remote, v;
-        asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"((u32)__cvta_generic_to_shared(&s_tot[col * 2 + h])), "r"(pr));
-        asm volatile("ld.shared::cluster.u32 %0, [%1];" : "=r"(v) : "r"(remote) : "memory");
+        u32 v;
+        asm volatile("ld.shared::cluster.u32 %0, [%1];" : "=r"(v) : "r"(dsmem_addr(&s_tot[col * 2 + h], pr)) : "memory");
         sum += v;
       }
       sum %= qKS;
@@ -1524,14 +1263,9 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(COLS *RG) keyswitch_
     }
   }
   if (rank == 0) peer_publish(px, gridDim.x >> 2); // one count per gate
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory"); // peers stay until rank 0 has read
+  cluster_sync_all(); // peers stay until rank 0 has read
 }
 
-static int keyswitch_attrs() {
-  constexpr int COLS = 256, RG = 4;
-  const size_t smem = (size_t)(2048 + 2) * 4 + (size_t)RG * COLS * 2 * 8;
-  return (int)cudaFuncSetAttribute(keyswitch_kernel<true, COLS, RG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024));
-}
 int launch_keyswitch(const DevConst &P, const u32 *d_ext, const DevGate *d_gates, int count, const void *d_ksk, int elem_bytes,
                      void *stream, const PeerX *pxp) {
   if (count <= 0) return 0;
@@ -1541,9 +1275,7 @@ int launch_keyswitch(const DevConst &P, const u32 *d_ext, const DevGate *d_gates
   if (elem_bytes == 2) {
     constexpr int COLS = 256, RG = 4;
     const int rowlen_words = 256; // 512 uint16 per row
-    size_t smem = (size_t)((nrows + 1) & ~1) * 4 + (size_t)RG * COLS * 2 * 8;
-    static bool done[64];
-    if (!done[attr_device_slot()]) { keyswitch_attrs(); done[attr_device_slot()] = true; }
+    size_t smem = (size_t)((nrows + 1) & ~1) * 4 + (size_t)RG * COLS * 2 * 8; // STD128_OPT: 24 KB, within the default 48 KB limit
     // while every CTA of the cluster form has an SM to itself it wins (measured: 1 gate 47 -> 23 us, 30 gates 56 -> 29 us; 74 gates
     // 57 -> 54 us; 148 gates 56 -> 82 us): used up to SMs / 4 gates, wider batches keep one CTA per gate
     int dev = 0, sms = 148;
@@ -1640,7 +1372,7 @@ template <int LOGN> __global__ void __launch_bounds__(32) dbg_ntt_kernel(const _
   for (int k = 0; k < E; k++) x[k] = a[p * N + lane + 32 * k];
   ntt_forward<LOGN>(x, s_buf, P, tt, lane);
 #pragma unroll
-  for (int k = 0; k < E; k++) y[k] = csub(lazy_reduce(x[k], Q, P.mu), Q);
+  for (int k = 0; k < E; k++) y[k] = csub(lazy_reduce(x[k], Q), Q);
   {
     u32 z[E];
 #pragma unroll
@@ -1657,7 +1389,7 @@ template <int LOGN> __global__ void __launch_bounds__(32) dbg_ntt_kernel(const _
     __syncwarp();
     ntt_forward<LOGN>(z, s_buf, P, tt, lane);
 #pragma unroll
-    for (int k = 0; k < E; k++) z[k] = (u32)(((u64)csub(lazy_reduce(z[k], Q, P.mu), Q) * y[k]) % Q);
+    for (int k = 0; k < E; k++) z[k] = (u32)(((u64)csub(lazy_reduce(z[k], Q), Q) * y[k]) % Q);
     __syncwarp();
     ntt_inverse<LOGN, 2>(z, s_buf, P, tt, lane);
 #pragma unroll

@@ -38,8 +38,7 @@
 // Per-step timeline and phase costs: tools/phase_timing.py (build with -DBFHE_PHASE_TIMING), profiles/r2_clx_*.
 // No cluster-scope fence or barrier.cluster inside the step loop; receive buffers and their mbarriers alternate by step parity, so a
 // CTA that runs one step ahead cannot overwrite or miscount data its peer is still reading.
-#include "common.hpp"
-#include <cuda_runtime.h>
+#include "device.cuh"
 
 namespace bfhe {
 namespace clx {
@@ -48,7 +47,6 @@ constexpr int LOGN = 10, N = 1 << LOGN, DG = 4, LOGBG = 7, ROWS = 2 * DG, R = 4,
 constexpr int KEYPOLYS = 2 * ROWS * 2; // GINX: two RGSW ciphertexts (X^a, X^-a) per step; AP: one (KEYPOLYS / 2 polynomials)
 constexpr int NSTEP_PAD = 1024;     // >= n (GINX) and >= n * dR (AP)
 constexpr u32 DIGIT_OFF = 64u + (64u << 7) + (64u << 14) + (64u << 21);
-constexpr u32 SOLINAS_Q = (1u << 27) - (1u << 11) + 1;
 
 // per-rank twiddle block (host-generated, engine.cu): fw[TWF] | fws[TWF] | iw[TWI] | iws[TWI]
 //   fw:  [0, 8)            pass A (register stages across the 32-strided values), uniform over the warp: w[1], w[2..3], w[4..7]
@@ -58,51 +56,6 @@ constexpr u32 SOLINAS_Q = (1u << 27) - (1u << 11) + 1;
 //        [8 + 256 s, ..)   s = 0..4: the inverse stage with half-size 2^s for MAC slot t (the five stages done by shuffles), [t]
 constexpr int TWF = 8 + 2 * 256, TWI = 8 + 5 * 256, TWR = 2 * TWF + 2 * TWI;
 
-__device__ __forceinline__ u32 redc(u64 s, u32 Q, u32 qinv_neg) { // s * 2^-32 mod Q, lazy
-  const u32 m = (u32)s * qinv_neg;
-  return (u32)((s + (u64)m * Q) >> 32);
-}
-__device__ __forceinline__ u32 lazy_reduce(u32 x, u32 Q) { return x - (x >> 27) * Q; } // floor(2^32 / Q) = 32: any x -> [0, 2Q)
-__device__ __forceinline__ u32 csub(u32 x, u32 Q) { return min(x, x - Q); }
-__device__ __forceinline__ u32 mul_shoup(u32 x, u32 w, u32 ws, u32 Q) { return x * w - __umulhi(x, ws) * Q; } // [0, 2Q)
-__host__ __device__ __forceinline__ u32 f_index(u32 k) { return ((k >> 5) & 63u) | ((k & 31u) << 6); } // table of psi^k - 1, see kernels_v2.cu
-
-__device__ __forceinline__ u32 smem_u32(const void *p) { return (u32)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(u64 *bar, u32 count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count)); }
-__device__ __forceinline__ void mbar_expect_tx(u64 *bar, u32 bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, u32 bytes, u64 *bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)), "l"(src), "r"(bytes),
-               "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(u64 *bar, u32 parity) {
-  asm volatile("{\n\t.reg .pred p;\n\tWAIT_%=:\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" ::"r"(
-                   smem_u32(bar)),
-               "r"(parity)
-               : "memory");
-}
-__device__ __forceinline__ bool mbar_test(u64 *bar, u32 parity) { // one try, no loop
-  u32 ok;
-  asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ u32 cluster_rank() { u32 r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ u32 dsmem_addr(const void *local, u32 rank) { // shared::cluster address of `local` in CTA `rank`
-  u32 a;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(smem_u32(local)), "r"(rank));
-  return a;
-}
-// remote store whose arrival is counted on the destination CTA's mbarrier (complete_tx): the receiver needs no cluster-scope fence
-__device__ __forceinline__ void st_async2(u32 dsmem, uint2 v, u32 dsmem_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v2.b32 [%0], {%1, %2}, [%3];" ::"r"(dsmem), "r"(v.x), "r"(v.y), "r"(dsmem_bar)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(u64 *bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory"); }
 // ---- 8-value register stages.  Stage with half-size T pairs a = g * 2T + (i % T), b = a + T and uses twiddle w[8 / (2T) + g] ----
 template <int T> __device__ __forceinline__ void ct8_stage(u32 (&x)[8], const u32 (&w)[8], const u32 (&ws)[8], u32 Q, u32 Q2) {
   u32 t[4];
@@ -162,8 +115,6 @@ constexpr u32 RECV_TX_C = (u32)(R - 1) * NB * 4; // bytes the three peers push i
 
 // named barriers (0 is left to __syncthreads in the prologue)
 constexpr int BAR_DCT = 1, BAR_GROUP = 2 /* + c */, BAR_KEY = 4;
-__device__ __forceinline__ void bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-__device__ __forceinline__ void bar_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 
 template <bool AP>
 __global__ void __cluster_dims__(R, 1, 1) __launch_bounds__(THREADS, 1)
@@ -543,53 +494,27 @@ __global__ void bk_slice_clx_ap_kernel(const u32 *__restrict__ src, u32 *__restr
 } // namespace clx
 
 bool clx_supported(const DevConst &P, int method_ap) {
-  return P.N == 1024 && P.dG == 4 && P.logBG == 7 && P.Q == clx::SOLINAS_Q && P.n * (method_ap ? P.dR : 1u) <= (u32)clx::NSTEP_PAD;
+  return P.N == 1024 && P.dG == 4 && P.logBG == 7 && P.Q == SOLINAS_Q && P.n * (method_ap ? P.dR : 1u) <= (u32)clx::NSTEP_PAD;
 }
 size_t clx_tw_words() { return (size_t)clx::R * clx::TWR; }
-static int clx_device_slot() {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  return dev >= 0 && dev < 64 ? dev : 0;
-}
 int clx_set_attrs() {
   int rc = (int)cudaFuncSetAttribute(clx::blind_rotate_clx_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)clx::Smem::bytes);
   rc |= (int)cudaFuncSetAttribute(clx::blind_rotate_clx_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)clx::Smem::bytes);
   return rc;
 }
-static int clx_attrs_once() { // per device, and never under stream capture: at first use
+static int clx_attrs_once() {
   static bool done[64];
-  const int d = clx_device_slot();
-  if (done[d]) return 0;
-  const int rc = clx_set_attrs();
-  if (rc == 0) done[d] = true;
-  return rc;
+  return once_per_device(done, clx_set_attrs);
 }
-int clx_max_gates() { // 4-CTA clusters of this kernel the device keeps co-resident, one CTA per SM
-  static int cached[64];
+int clx_max_gates() { // 4-CTA clusters of this kernel the device keeps co-resident, one CTA per SM; queried once per device, a 0 included
   static bool have[64];
-  const int d = clx_device_slot();
-  if (!have[d]) {
-    int nmax = 0;
-    if (clx_attrs_once() == 0) {
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(clx::R * 148, 1, 1);
-      cfg.blockDim = dim3(clx::THREADS, 1, 1);
-      cfg.dynamicSmemBytes = clx::Smem::bytes;
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = clx::R; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      cfg.attrs = at;
-      cfg.numAttrs = 1;
-      if (cudaOccupancyMaxActiveClusters(&nmax, clx::blind_rotate_clx_kernel<false>, &cfg) != cudaSuccess) { cudaGetLastError(); nmax = 0; }
-      int dev = 0, sms = 148;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-      if (nmax > sms / clx::R) nmax = sms / clx::R;
-    }
-    cached[d] = nmax;
-    have[d] = true;
-  }
-  return cached[d];
+  static int gates[64];
+  const int d = device_slot();
+  once_per_device(have, [&] {
+    gates[d] = clx_attrs_once() ? 0 : max_active_clusters(clx::blind_rotate_clx_kernel<false>, clx::R, clx::THREADS, clx::Smem::bytes);
+    return cudaSuccess;
+  });
+  return gates[d];
 }
 // The occupancy query is exact for this kernel (B200: 33 clusters; measured 1.02 ms per wave up to 33 gates, 2.03 ms -- a second round --
 // from 34 on), so the whole co-resident maximum runs at full speed.

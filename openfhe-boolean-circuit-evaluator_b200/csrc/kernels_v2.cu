@@ -9,8 +9,7 @@
 // on every context; the row-split 4-CTA form (1.17 ms per wave) is superseded by the slot-sliced one in kernels_cl.cu (1.02 ms).  Both
 // were removed in round 2.  What remains of the shared machinery: one shared-memory row layout (phys()) that serves 32-bit column,
 // 64-bit pair and 128-bit row access conflict-free (tools/smem_layout_check.py), and the 16- / 8-value tile transforms.
-#include "common.hpp"
-#include <cuda_runtime.h>
+#include "device.cuh"
 #include <type_traits>
 
 namespace bfhe {
@@ -18,26 +17,10 @@ namespace v2 {
 
 constexpr int LOGN = 10, N = 1 << LOGN, DG = 4, LOGBG = 7, ROWS = 2 * DG, NPAD = 512;
 constexpr u32 DIGIT_OFF = 64u + (64u << 7) + (64u << 14) + (64u << 21);
-constexpr u32 SOLINAS_Q = (1u << 27) - (1u << 11) + 1;
 
-// BFHE_V2_SOL_*: per-stage masks that compute the t*Q term of the Shoup multiply as shifts and adds on the ALU pipe (Q = 2^27 - 2^11 + 1:
-// t*Q = t + ((t << 16) - t) << 11) instead of one IMAD on the FMA-heavy pipe.  Six masks measured within +-1.5 % of each other: default off.
-#ifndef BFHE_V2_SOL_FW
-#define BFHE_V2_SOL_FW 0x000 // bit i = forward stage i (0 = widest)
-#endif
-#ifndef BFHE_V2_SOL_INV
-#define BFHE_V2_SOL_INV 0x000 // bit i = inverse stage i (0 = narrowest)
-#endif
-__device__ __forceinline__ u32 redc(u64 s, u32 Q, u32 qinv_neg) { // s * 2^-32 mod Q, lazy
-  const u32 m = (u32)s * qinv_neg;
-  return (u32)((s + (u64)m * Q) >> 32);
-}
-__device__ __forceinline__ u32 lazy_reduce(u32 x, u32 Q) { return x - (x >> 27) * Q; } // floor(2^32/Q) = 32: any x -> [0,2Q)
 // ptxas turns many 2-input adds into IMAD.IADD "to balance the pipes" -- onto the FMA-heavy pipe, the unit that bounds
 // this kernel (it counts IMAD.HI as one slot; the hardware takes two).  A 3-input add with a run-time zero stays an IADD3.
 __device__ __forceinline__ u32 add3(u32 a, u32 b, u32 z) { return a + b + z; }
-__device__ __forceinline__ u32 csub(u32 x, u32 Q) { return min(x, x - Q); }
-__device__ __forceinline__ void bar_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 
 // position p of a polynomial (coefficient index going in, bit-reversed evaluation slot coming out) -> word offset in its
 // shared-memory row.  Rows of 16 words; 16-byte chunks XOR-swizzled by the row number; row pairs swapped by bit 3 of the row.
@@ -56,12 +39,10 @@ __host__ __device__ __forceinline__ int unphys(int o) {
 // Written batch-wise (all high products of a stage, then all low products, then the corrections, then the sums): ptxas keeps
 // close to source order inside these very long basic blocks, and butterfly-by-butterfly source order left every instruction
 // waiting on its predecessor (profiles/r1_v2_*: 27 % of warp cycles in fixed-latency "wait").
-template <int TBEG, int TEND, int SOLMASK = 0>
+template <int TBEG, int TEND>
 __device__ __forceinline__ void ct_stages(u32 (&x)[16], const u32 *__restrict__ w, const u32 *__restrict__ ws, u32 Q, u32 Q2, u32 Z) {
-  int si = 0;
 #pragma unroll
-  for (int t = TBEG; t >= TEND; t >>= 1, si++) {
-    const bool sol = (SOLMASK >> si) & 1;
+  for (int t = TBEG; t >= TEND; t >>= 1) {
     u32 hi[8], lo[8];
 #pragma unroll
     for (int i = 0; i < 8; i++) { // butterfly i: group gi = i / t, member j = i % t
@@ -74,14 +55,7 @@ __device__ __forceinline__ void ct_stages(u32 (&x)[16], const u32 *__restrict__ 
       lo[i] = x[b] * w[p];
     }
 #pragma unroll
-    for (int i = 0; i < 8; i++) {
-      if (sol) {
-        const u32 s = hi[i] - (hi[i] << 16);
-        lo[i] = (lo[i] - hi[i]) + (s << 11);
-      } else {
-        lo[i] = lo[i] - hi[i] * Q;
-      }
-    }
+    for (int i = 0; i < 8; i++) lo[i] = lo[i] - hi[i] * Q;
 #pragma unroll
     for (int i = 0; i < 8; i++) {
       const int gi = i / t, a = gi * 2 * t + (i % t), b = a + t;
@@ -99,7 +73,7 @@ __host__ __device__ constexpr int gs_bound(int T, int TEND, int B, int MAXOUT) {
   }
   return B;
 }
-template <int T, int TEND, int B, int MAXOUT, int SOLMASK = 0> struct Gs {
+template <int T, int TEND, int B, int MAXOUT> struct Gs {
   static constexpr int NB = 2 * B;
   static constexpr bool LAST = (T == TEND);
   static constexpr bool RED = LAST ? (NB > MAXOUT) : (NB > 16);
@@ -122,14 +96,9 @@ template <int T, int TEND, int B, int MAXOUT, int SOLMASK = 0> struct Gs {
 #pragma unroll
     for (int i = 0; i < 8; i++) {
       const int gi = i / T, b = gi * 2 * T + (i % T) + T;
-      if ((SOLMASK & 1) != 0) {
-        const u32 s = hi[i] - (hi[i] << 16);
-        x[b] = (D[i] - hi[i]) + (s << 11);
-      } else {
-        x[b] = D[i] - hi[i] * Q;
-      }
+      x[b] = D[i] - hi[i] * Q;
     }
-    if constexpr (!LAST) Gs<2 * T, TEND, OUTB, MAXOUT, (SOLMASK >> 1)>::run(x, w, ws, Q, Z);
+    if constexpr (!LAST) Gs<2 * T, TEND, OUTB, MAXOUT>::run(x, w, ws, Q, Z);
   }
 };
 
@@ -208,10 +177,6 @@ __device__ __forceinline__ void row_store(u32 *buf, const u32 (&x)[16], int T3) 
 
 
 
-// table of (psi^k - 1): the lanes of a warp own slots whose exponents differ in bits 4..8, so entry k is stored at the
-// 11-bit rotation of k by 5 (bank = bits 5..9 of k): 1.5 wavefronts per gather on average instead of 16
-__host__ __device__ __forceinline__ u32 f_index(u32 k) { return ((k >> 5) & 63u) | ((k & 31u) << 6); }
-
 // ------------------------------------------------------------------------------------------------------------------
 // Latency form on a 2-CTA thread-block cluster: ONE gate on TWO SMs (narrow circuit wavefronts: fewer gates than half the
 // SMs, where the time of a level is the latency of one bootstrap -- SHA-256 / MD5, and every circuit once its levels are
@@ -224,31 +189,6 @@ __host__ __device__ __forceinline__ u32 f_index(u32 k) { return ((k >> 5) & 63u)
 // DSMEM.  The CTA's half of the step's key tile (64 KB) is staged by TMA bulk copies behind an mbarrier, issued right after
 // the previous product.
 // ------------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ u32 smem_u32(const void *p) { return (u32)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(u64 *bar, u32 count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count)); }
-__device__ __forceinline__ void mbar_expect_tx(u64 *bar, u32 bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, u32 bytes, u64 *bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)), "l"(src), "r"(bytes),
-               "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(u64 *bar, u32 parity) {
-  asm volatile("{\n\t.reg .pred p;\n\tWAIT_%=:\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" ::"r"(
-                   smem_u32(bar)),
-               "r"(parity)
-               : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ u32 cluster_rank() { u32 r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ u32 dsmem_addr(const void *local, u32 rank) { // shared::cluster address of `local` in CTA `rank`
-  u32 a;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(smem_u32(local)), "r"(rank));
-  return a;
-}
 // ---- inverse transform on 8-value tiles by FOUR warps (T = 0..127): three register stages per pass, the widest stage (span 512)
 // across lanes 16 apart.  Same row layout; used by the cluster kernel, where the inverse transform of the one product row is the
 // serial part of a step.  On return x[k] = coefficient T6 + 64*(k + 8*hi), fully reduced (T6 = 16*warp + lane % 16, hi = lane / 16).
@@ -343,18 +283,6 @@ template <int B0> __device__ __forceinline__ void ntt_inverse_quad8(u32 (&x)[8],
   }
 }
 
-// remote store whose arrival is counted on the destination CTA's mbarrier (complete_tx): the receiver needs no cluster-scope
-// fence, it just waits for the phase of its own barrier
-__device__ __forceinline__ void st_async4(u32 dsmem, uint4 v, u32 dsmem_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];" ::"r"(dsmem), "r"(v.x), "r"(v.y),
-               "r"(v.z), "r"(v.w), "r"(dsmem_bar)
-               : "memory");
-}
-__device__ __forceinline__ void st_async2(u32 dsmem, uint2 v, u32 dsmem_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v2.b32 [%0], {%1, %2}, [%3];" ::"r"(dsmem), "r"(v.x), "r"(v.y), "r"(dsmem_bar)
-               : "memory");
-}
-
 // forward transform of one digit by TWO warps (T = 32*h + lane), one tile per thread and pass
 // push_dst != 0: the finished tile (16 consecutive words of the row) is not stored here but sent to the peer CTA at shared::cluster
 // address push_dst + 4 * (word offset in the row), counted on the peer's mbarrier push_bar
@@ -364,7 +292,7 @@ __device__ __forceinline__ void ntt_forward_split(const u32 *dp, int l, u32 *buf
   u32 x[16];
 #pragma unroll
   for (int k = 0; k < 16; k++) x[k] = ((dp[T + 64 * k] >> (LOGBG * l)) & ((1u << LOGBG) - 1)) + qoff;
-  ct_stages<8, 1, (BFHE_V2_SOL_FW & 15)>(x, P.tw, P.tws, Q, Q2, Z);
+  ct_stages<8, 1>(x, P.tw, P.tws, Q, Q2, Z);
   col_store(buf, x, T);
   bar_sync(bar_id, 64);
   {
@@ -372,7 +300,7 @@ __device__ __forceinline__ void ntt_forward_split(const u32 *dp, int l, u32 *buf
     load_tw_mid(tt.fw, w, T >> 2);
     load_tw_mid(tt.fws, ws, T >> 2);
     mid_load(buf, x, T);
-    ct_stages<8, 2, ((BFHE_V2_SOL_FW >> 4) & 7)>(x, w, ws, Q, Q2, Z);
+    ct_stages<8, 2>(x, w, ws, Q, Q2, Z);
     mid_store(buf, x, T);
   }
   bar_sync(bar_id, 64);
@@ -381,7 +309,7 @@ __device__ __forceinline__ void ntt_forward_split(const u32 *dp, int l, u32 *buf
     load_tw_narrow(tt.fw, w, T);
     load_tw_narrow(tt.fws, ws, T);
     row_load(buf, x, T);
-    ct_stages<4, 1, ((BFHE_V2_SOL_FW >> 7) & 7)>(x, w, ws, Q, Q2, Z);
+    ct_stages<4, 1>(x, w, ws, Q, Q2, Z);
     if (push_dst == 0) row_store(buf, x, T);
     else {
       const int b = row_base(T);
@@ -648,55 +576,31 @@ __global__ void bk_permute_v2_kernel(const u32 *__restrict__ src, u32 *__restric
 } // namespace v2
 
 bool v2_supported(const DevConst &P, int method_ap) {
-  return !method_ap && P.N == 1024 && P.dG == 4 && P.logBG == 7 && P.Q == v2::SOLINAS_Q && P.n <= (u32)v2::NPAD;
+  return !method_ap && P.N == 1024 && P.dG == 4 && P.logBG == 7 && P.Q == SOLINAS_Q && P.n <= (u32)v2::NPAD;
 }
 int v2_set_attrs() {
   return (int)cudaFuncSetAttribute(v2::blind_rotate_cl2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)v2::Cl2Cfg::smem_bytes);
 }
-template <typename K> static int max_active_clusters(K kern, int cluster, int threads, size_t smem) {
-  if (v2_set_attrs()) return 0;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(cluster * 148, 1, 1);
-  cfg.blockDim = dim3(threads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = cluster; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  int n = 0;
-  if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess) { cudaGetLastError(); n = 0; }
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return n < sms / cluster ? n : sms / cluster; // one CTA per SM: two co-resident CTAs of these kernels would just share the pipe
-}
-static int current_device_slot();
-static int v2_attrs_once() { // function attributes are per device and must not be set under stream capture: once, at first use
+static int v2_attrs_once() {
   static bool done[64];
-  const int d = current_device_slot();
-  if (done[d]) return 0;
-  const int rc = v2_set_attrs();
-  if (rc == 0) done[d] = true;
-  return rc;
-}
-static int current_device_slot() { // the limits are per device (one process may hold contexts on several)
-  int dev = 0;
-  cudaGetDevice(&dev);
-  return dev >= 0 && dev < 64 ? dev : 0;
+  return once_per_device(done, v2_set_attrs);
 }
 int launch_bk_split_cl4(const u32 *d_src, u32 *d_dst, size_t npoly, void *stream) {
   if (npoly == 0) return 0;
   v2::bk_split_cl4_kernel<<<148 * 8, 256, 0, (cudaStream_t)stream>>>(d_src, d_dst, npoly / v2::Cl2Cfg::KEYPOLYS);
   return (int)cudaGetLastError();
 }
-// how many gates the cluster form runs at once (2-CTA clusters must sit inside one GPC, so this can be less than SMs / 2)
+// how many gates the cluster form runs at once (2-CTA clusters must sit inside one GPC, so this can be less than SMs / 2); queried once
+// per device, a 0 included
 int cl2_max_gates() {
-  static int cached[64];
   static bool have[64];
-  const int d = current_device_slot();
-  if (!have[d]) { cached[d] = max_active_clusters(v2::blind_rotate_cl2_kernel, 2, v2::Cl2Cfg::THREADS, v2::Cl2Cfg::smem_bytes); have[d] = true; }
-  return cached[d];
+  static int gates[64];
+  const int d = device_slot();
+  once_per_device(have, [&] {
+    gates[d] = v2_attrs_once() ? 0 : max_active_clusters(v2::blind_rotate_cl2_kernel, 2, v2::Cl2Cfg::THREADS, v2::Cl2Cfg::smem_bytes);
+    return cudaSuccess;
+  });
+  return gates[d];
 }
 int launch_blind_rotate_cl2(const DevConst &P, const DevGate *d_gates, int count, const V2Bufs &vb, u32 *d_ext, u32 *d_acc_dbg, void *stream,
                             LaunchInfo *info) {

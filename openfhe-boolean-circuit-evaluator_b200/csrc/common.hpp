@@ -50,13 +50,15 @@ struct LaunchInfo { // filled by the launch helpers for the profiler hooks
   size_t smem_bytes;
 };
 
-// device buffers of the cluster kernels (kernels_v2.cu, kernels_cl.cu); all null when the parameter set is not covered
+// derived key copies and tables of the cluster kernels (kernels_v2.cu, kernels_cl.cu) and of the GINX throughput kernel (d_bkf); each null
+// when the parameter set is not covered
 struct V2Bufs {
   const u32 *d_bk4 = nullptr; // bootstrapping key, rows in kernels_v2.cu's physical slot order, split [step][quarter of the slots][polynomial][N/4]
   const u32 *d_tw2 = nullptr; // fwd w | fwd ws | inv w | inv ws, each N words (order: kernels_v2.cu Tabs)
   const u32 *d_F = nullptr;   // (psi^k - 1) * 2^32 mod Q, k < 2N
   const u32 *d_bkx = nullptr; // slot-sliced 4-CTA cluster kernel (kernels_cl.cu): key as [step][rank][polynomial][N/4]
   const u32 *d_twx = nullptr; // ... and its per-rank twiddle blocks
+  const u32 *d_bkf = nullptr; // STD128_OPT-shape GINX throughput kernel (kernels.cu): d_bk with the top digit folded in (launch_bk_fold)
 };
 
 // kernels.cu entry points (all asynchronous on `stream`; return cudaError_t as int)
@@ -105,6 +107,10 @@ int launch_peer_wait(const u32 *local_flags, const u32 *epoch, u32 world, u32 ra
 int launch_peer_signal(const PeerX &px, void *stream);
 int launch_eval_not(const DevConst &P, const u32 *const *d_in, u32 *const *d_out, int count, void *stream);
 int launch_bk_convert(const DevConst &P, const u32 *d_coef, u32 *d_dev, size_t npoly, const u32 *d_twl, void *stream);
+// key copy of the GINX throughput kernel at the STD128_OPT shape (N 1024, dG 4, base 2^7): the device-form key with its top digit row folded
+// into the others (kernels.cu bk_fold_kernel); nsteps = n
+bool bk_fold_supported(const DevConst &P, int method_ap);
+int launch_bk_fold(const DevConst &P, const u32 *d_bk, u32 *d_bkf, size_t nsteps, void *stream);
 int launch_dbg_ntt(const DevConst &P, const u32 *d_a, const u32 *d_b, u32 *d_rt, u32 *d_prod, int npoly, const u32 *d_twl,
                    void *stream);
 int launch_microbench(int which, u32 *d_sink, int iters, int *threads_total, int *ops_per_thread_iter, void *stream);

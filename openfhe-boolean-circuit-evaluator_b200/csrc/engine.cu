@@ -232,6 +232,7 @@ extern "C" void bfhe_destroy(bfhe_ctx *c) {
     cudaFree(c->d_gates_b); cudaFree(c->d_ext_b);
     cudaFree(c->d_bk4); cudaFree(c->d_tw2); cudaFree(c->d_F);
     cudaFree(c->d_bkx); cudaFree(c->d_twx);
+    cudaFree(c->d_bkf);
     for (int i = 0; i < 2; i++) {
       if (c->ev_br[i]) cudaEventDestroy(c->ev_br[i]);
       if (c->ev_ks[i]) cudaEventDestroy(c->ev_ks[i]);
@@ -421,6 +422,14 @@ int bfhe::ensure_device_keys(bfhe_ctx *c) {
     if (rc) return cuda_fail((cudaError_t)rc, "bk_slice_clx");
     BFHE_CUDA(cudaStreamSynchronize(c->stream));
     c->v2.d_bkx = c->d_bkx;
+  }
+  cudaFree(c->d_bkf); c->d_bkf = nullptr; c->v2.d_bkf = nullptr;
+  if (bk_fold_supported(c->P, p.method == BFHE_AP)) { // key copy of the GINX throughput kernel: the top digit folded into the other rows
+    BFHE_CUDA(cudaMalloc(&c->d_bkf, c->bk_words * 4));
+    int rc = launch_bk_fold(c->P, c->d_bk, c->d_bkf, p.n, c->stream);
+    if (rc) return cuda_fail((cudaError_t)rc, "bk_fold");
+    BFHE_CUDA(cudaStreamSynchronize(c->stream));
+    c->v2.d_bkf = c->d_bkf;
   }
   { // KSK: [i][j(digit value)][k(digit index)][n+1]  ->  [i][k][j][rowlen]
     const u32 rowlen = c->ksk_elem_bytes == 2 ? 512 : p.ct_stride; // elements per padded row

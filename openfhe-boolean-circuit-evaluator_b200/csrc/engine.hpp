@@ -48,6 +48,7 @@ struct bfhe_ctx {
   void *d_ksk = nullptr;
   bfhe::u32 *d_bk4 = nullptr, *d_tw2 = nullptr, *d_F = nullptr; // 2-CTA cluster kernel (kernels_v2.cu)
   bfhe::u32 *d_bkx = nullptr, *d_twx = nullptr; // slot-sliced cluster kernel (kernels_cl.cu)
+  bfhe::u32 *d_bkf = nullptr; // GINX throughput kernel at the STD128_OPT shape: top digit folded into the key (kernels.cu bk_fold_kernel)
   bfhe::V2Bufs v2{};
   bool dev_keys = false;
 

@@ -16,7 +16,7 @@
 //    Montgomery-reduces once (keys are stored pre-multiplied by 2^32 * N^-1).
 //  * The accumulator lives in COEFFICIENT form in the registers of the warp that owns it for the
 //    whole blind rotation: each step is INTT(previous product) -> add -> signed digit decomposition
-//    -> dG forward NTTs, all in registers of the same warp.
+//    -> dG forward NTTs, all in registers of the same warp (dG - 1 for STD128_OPT GINX, whose top digit is folded into a key copy).
 //  * A CTA carries G gates through the n blind-rotation steps in lock step so that every
 //    bootstrapping-key word loaded from L2 is reused G times from registers (GINX).
 #include "device.cuh"
@@ -195,26 +195,6 @@ __device__ __forceinline__ void ntt_forward(u32 (&x)[(1 << LOGN) / 32], u32 *buf
   ct_pass<E, false, SOLN>(x, P.tw, P.tws, Q, Q2, tt.fw, tt.fws, lane);
 }
 
-// two forward transforms at once (two digit polynomials of the same accumulator component): twice the independent butterflies
-// per stage for the scheduler, which with two warps per scheduler is what a transform lacks to keep the FMA-heavy pipe busy
-template <int LOGN, bool PRE = false>
-__device__ __forceinline__ void ntt_forward2(u32 (&xa)[(1 << LOGN) / 32], u32 (&xb)[(1 << LOGN) / 32], u32 *bufa, u32 *bufb, const DevConst &P,
-                                             const TwTabs &tt, int lane, const u32 *prea = nullptr, const u32 *preb = nullptr) {
-  constexpr int E = (1 << LOGN) / 32;
-  static_assert((LOGN & 1) == 0, "even log2 N only");
-  const u32 Q = P.Q, Q2 = P.Q2;
-  ct_pass<E, true, 0, PRE>(xa, P.tw, P.tws, Q, Q2, nullptr, nullptr, 0, prea);
-  ct_pass<E, true, 0, PRE>(xb, P.tw, P.tws, Q, Q2, nullptr, nullptr, 0, preb);
-  __syncwarp();
-  col_store<E>(bufa, xa, lane);
-  col_store<E>(bufb, xb, lane);
-  __syncwarp();
-  row_load<E>(bufa, xa, lane);
-  row_load<E>(bufb, xb, lane);
-  ct_pass<E, false>(xa, P.tw, P.tws, Q, Q2, tt.fw, tt.fws, lane);
-  ct_pass<E, false>(xb, P.tw, P.tws, Q, Q2, tt.fw, tt.fws, lane);
-}
-
 // inverse (unscaled: N * true value; the keys carry N^-1): x in row layout (evaluation form, values < B0*Q)
 // -> column layout, coefficient form, fully reduced to [0,Q).
 template <int LOGN, int B0>
@@ -266,6 +246,9 @@ template <int LOGN, int DG, int LOGBG, int G, bool AP> struct BrCfg {
   // first-stage product table: twiddle * (digit - B/2) mod Q for the 2^LOGBG digit values, one copy per bank (STD128_OPT shape only)
   static constexpr bool LUT = (LOGBG == 7 && LOGN == 10);
   static constexpr size_t lut_words = LUT ? (size_t)32 << LOGBG : 0;
+  // GINX at the same shape: the top digit is folded into the key (bk_fold_kernel), so each component transforms DG - 1 digits per step
+  // and dct rows 2(DG-1) + c hold N^-1 * NTT(acc_c) instead of a digit row (see blind_rotate_kernel)
+  static constexpr bool FOLD = LUT && !AP;
   static constexpr size_t smem_bytes = (dct_words + 4 * N + (AP ? 0 : 2 * N) + lut_words) * 4 + (size_t)G * NPAD * 2;
 };
 
@@ -277,6 +260,15 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
   using Cfg = BrCfg<LOGN, DG, LOGBG, G, AP>;
   constexpr int N = Cfg::N, E = Cfg::E, C = Cfg::C, ROWS = Cfg::ROWS, W = Cfg::W, NPAD = Cfg::NPAD;
   constexpr u32 DIGIT_OFF = digit_offset<DG, LOGBG>();
+  // FOLD: the DG digits of the centred accumulator a in [-(Q+1)/2, (Q-3)/2] are the base-B digits of a + DIGIT_OFF, each minus B/2.  When
+  // that sum always lies in [0, B^DG), they represent a exactly: acc_c = sum_l B^l d_{c,l} as integers, so in evaluation form the top digit
+  // is D_{c,DG-1} = B^-(DG-1) (A_c - sum_{l<DG-1} B^l D_{c,l}) mod Q, A_c = NTT(acc_c).  Substituted into the external product, the top key
+  // row moves into the other rows and into a row that multiplies A_hat_c = N^-1 A_c (bk_fold_kernel), and the step needs no transform of
+  // the top digit.  A_hat_c is kept current by adding the product's output row, which is N^-1 NTT of the accumulator's increment.
+  constexpr bool FOLD = Cfg::FOLD;
+  static_assert(!FOLD || (DIGIT_OFF >= (SOLINAS_Q + 1) / 2 && (u64)DIGIT_OFF + (SOLINAS_Q - 3) / 2 < (1ull << (LOGBG * DG))),
+                "the digits do not cover the centred accumulator: the top digit cannot be folded into the key");
+  constexpr int ND = FOLD ? DG - 1 : DG; // digit transforms per component and step
   extern __shared__ __align__(128) unsigned char smem_raw[];
   u32 *dct = reinterpret_cast<u32 *>(smem_raw);                 // [G][ROWS][N]
   u32 *s_tw = dct + Cfg::dct_words;                             // fw | fws | iw | iws
@@ -349,6 +341,16 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
       }
     }
   }
+  if (FOLD && gvalid) { // A_hat_c = N^-1 * NTT(acc_c) (zero for component 0), below 2Q, in the row the top digit of component c had
+    u32 x[E];
+#pragma unroll
+    for (int k = 0; k < E; k++) x[k] = acc[k];
+    u32 *abuf = dct + ((size_t)g * ROWS + 2 * (DG - 1) + c) * N;
+    ntt_forward<LOGN>(x, abuf, P, tt, lane);
+#pragma unroll
+    for (int k = 0; k < E; k++) x[k] = mul_shoup(x[k], P.ninv, P.ninvs, Q);
+    row_store<E>(abuf, x, lane);
+  }
 
   const int nsteps = AP ? n * P.dR : n;
   bool pending = false;
@@ -357,13 +359,9 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
   // MAC work split: item -> (chunk qc, gate split)
   constexpr int GS = (W >= C) ? (W / C) : 1;
   const u32 eA = 2 * brev(lane, 5) + 1; // lane part of the evaluation-point exponent 2*br(idx)+1
-  // two digits per pass (STD128_OPT shape): +8 % at two gates per CTA (71.3k -> 77.0k gates/s), nothing at four (79.3k vs 79.7k),
-  // where the phase is already within ~20 % of its pipe bound (tools/phase_timing.py) -- used for G <= 2 only
-  constexpr bool PAIRED = Cfg::LUT && DG % 2 == 0 && G <= 2;
-  // GINX, one digit per pass: the step's key words are requested BEFORE the warp's last digit transform, so the L2 round trip runs under
-  // the transform and the wait at the CTA barrier instead of in front of the product (535 cycles of a 27 k-cycle step sat there,
-  // tools/phase_timing.py; DESIGN.md 5.1)
-  constexpr bool KEY_HOIST = !AP && !PAIRED;
+  // GINX: the step's key words are requested BEFORE the warp's last digit transform, so the L2 round trip runs under the transform and the
+  // wait at the CTA barrier instead of in front of the product (535 cycles of a 27 k-cycle step sat there, tools/phase_timing.py; DESIGN.md 5.1)
+  constexpr bool KEY_HOIST = !AP;
 
 #ifdef BFHE_PHASE_TIMING
   long long tpt[5] = {0, 0, 0, 0, 0}, tq0 = clock64(), tq1;
@@ -414,33 +412,12 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
       // Closed form of the sequential peel (r = signed low digit; d = (d - r) >> LOGBG): adding B/2 at every digit
       // position turns the balanced digits into the plain base-B digits of d + OFF, so digit l is one shift, one mask and
       // one subtraction with no dependency on the digits below it (the top digit wraps exactly like the reference's
-      // sign-truncation when dG digits do not cover the centred range, e.g. TOY).
+      // sign-truncation when dG digits do not cover the centred range, e.g. TOY).  FOLD: the top digit is not needed.
       u32 dp[E];
 #pragma unroll
       for (int k = 0; k < E; k++) dp[k] = ((acc[k] < (Q >> 1)) ? acc[k] : acc[k] - Q) + DIGIT_OFF;
-      if constexpr (PAIRED) {
 #pragma unroll
-        for (int l = 0; l < DG; l += 2) {
-          u32 xa[E], xb[E], prea[E / 2], preb[E / 2];
-#pragma unroll
-          for (int k = 0; k < E; k++) {
-            const u32 sh = dp[k] >> (LOGBG * l), da = sh & ((1u << LOGBG) - 1), db = (sh >> LOGBG) & ((1u << LOGBG) - 1);
-            if (k >= E / 2) {
-              prea[k - E / 2] = s_lut[(da << 5) + lane]; xa[k] = 0;
-              preb[k - E / 2] = s_lut[(db << 5) + lane]; xb[k] = 0;
-            } else {
-              xa[k] = da + (Q - (1u << (LOGBG - 1)));
-              xb[k] = db + (Q - (1u << (LOGBG - 1)));
-            }
-          }
-          u32 *bufa = dct + ((size_t)g * ROWS + c + 2 * l) * N, *bufb = bufa + 2 * N;
-          ntt_forward2<LOGN, true>(xa, xb, bufa, bufb, P, tt, lane, prea, preb);
-          row_store<E>(bufa, xa, lane);
-          row_store<E>(bufb, xb, lane);
-        }
-      } else {
-#pragma unroll
-      for (int l = 0; l < DG; l++) {
+      for (int l = 0; l < ND; l++) {
         u32 x[E], pre[Cfg::LUT ? E / 2 : 1];
 #pragma unroll
         for (int k = 0; k < E; k++) {
@@ -451,10 +428,9 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
           else x[k] = dgt + (Q - (1u << (LOGBG - 1)));
         }
         u32 *buf = dct + ((size_t)g * ROWS + c + 2 * l) * N;
-        if (KEY_HOIST && l == DG - 1 && warp < C * GS) BFHE_GX_LOAD(warp % C);
+        if (KEY_HOIST && l == ND - 1 && warp < C * GS) BFHE_GX_LOAD(warp % C);
         ntt_forward<LOGN, Cfg::LUT>(x, buf, P, tt, lane, pre);
         row_store<E>(buf, x, lane);
-      }
       }
     } else if (KEY_HOIST && warp < C * GS) { // empty gate slot (ragged last CTA): no transform to hide behind, but the product still needs the words
       BFHE_GX_LOAD(warp % C);
@@ -467,7 +443,6 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
       BFHE_AP_LOAD(0, ap_key(warp / C, warp % C));
       if (JN > 1) BFHE_AP_LOAD(1, ap_key(warp / C + GS, warp % C));
     }
-    if (!AP && !KEY_HOIST && warp < C * GS) BFHE_GX_LOAD(warp % C);
     __syncthreads();
     PT_T(1);
 
@@ -535,6 +510,11 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
           }
           // R[gg][cc] overwrites dct row cc: this thread has already consumed that chunk of every row
           *reinterpret_cast<uint4 *>(gd + (size_t)cc * N) = make_uint4(out[0], out[1], out[2], out[3]);
+          if constexpr (FOLD) { // A_hat_cc += R[gg][cc], kept below 2Q (the products' bounds assume < 22Q)
+            const uint4 a = dv[ROWS - 2 + cc];
+            *reinterpret_cast<uint4 *>(gd + (size_t)(ROWS - 2 + cc) * N) =
+                make_uint4(lazy_reduce(a.x + out[0], Q), lazy_reduce(a.y + out[1], Q), lazy_reduce(a.z + out[2], Q), lazy_reduce(a.w + out[3], Q));
+          }
         }
         if (AP && j + 2 < JN) { // this buffer is free again: request the key of the gate after next
           if ((j & 1) == 0) BFHE_AP_LOAD(0, ap_key(gs0 + (j + 2) * GS, qc)); else BFHE_AP_LOAD(1, ap_key(gs0 + (j + 2) * GS, qc));
@@ -1036,11 +1016,12 @@ int launch_blind_rotate(const DevConst &P, int method_ap, const DevGate *d_gates
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   // Which variant?  Measured on B200, STD128_OPT GINX (profiles/): one gate on four SMs 0.98 ms per wave of up to 33 gates; one gate on two
   // SMs 1.48 ms up to 74; latency form (one gate per CTA) 2.22 ms per wave of `sms` gates; throughput form (4 gates per CTA share every
-  // key word) 6.7 ms per wave of 4 * sms gates.  Narrow circuit levels go to the cluster forms, wide batches to the throughput form.
+  // key word) 5.97 ms per wave of 4 * sms gates with the folded key (6.73 ms before).  Narrow circuit levels go to the cluster forms, wide
+  // batches to the throughput form.
   if (force_g == 0 && have_clx && count <= clx_fast_gates()) return launch_blind_rotate_clx(P, method_ap, d_gates, count, *v2, d_ext, d_acc_dbg, stream, info);
   if (force_g == 0 && have_cl2 && count <= cl2_max_gates()) return launch_blind_rotate_cl2(P, d_gates, count, *v2, d_ext, d_acc_dbg, stream, info);
   const long lat_cost = (long)((count + sms - 1) / sms) * 222;           // 2.22 ms per wave of `sms` gates
-  const long thr_cost = (long)((count + 4 * sms - 1) / (4 * sms)) * 670; // 6.70 ms per wave of 4 * sms gates
+  const long thr_cost = (long)((count + 4 * sms - 1) / (4 * sms)) * 597; // 5.97 ms per wave of 4 * sms gates
   const bool lat = force_g == 8 || (force_g == 0 && lat_cost <= thr_cost);
   if (lat) {
     if (P.N == 1024 && P.dG == 4 && P.logBG == 7)
@@ -1053,8 +1034,10 @@ int launch_blind_rotate(const DevConst &P, int method_ap, const DevGate *d_gates
   }
   int G = force_g > 0 ? force_g : 4;
   if (P.N == 1024 && P.dG == 4 && P.logBG == 7) {
-    return method_ap ? launch_br_g<10, 4, 7, true>(G, P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info)
-                     : launch_br_g<10, 4, 7, false>(G, P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info);
+    if (method_ap) return launch_br_g<10, 4, 7, true>(G, P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info);
+    static_assert(BrCfg<10, 4, 7, 4, false>::FOLD, "the GINX throughput kernel of this shape reads the folded key");
+    if (!v2 || !v2->d_bkf) return (int)cudaErrorInvalidValue;
+    return launch_br_g<10, 4, 7, false>(G, P, d_gates, count, v2->d_bkf, d_twl, d_psiM, d_ext, d_acc_dbg, st, info);
   }
   if (P.N == 512 && P.dG == 3 && P.logBG == 9) {
     return method_ap ? launch_br_g<9, 3, 9, true>(G, P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info)
@@ -1349,6 +1332,50 @@ int launch_bk_convert(const DevConst &P, const u32 *d_coef, u32 *d_dev, size_t n
   if (P.N == 1024) bk_convert_kernel<10><<<blocks, 128, 0, (cudaStream_t)stream>>>(P, d_coef, d_dev, npoly, d_twl);
   else if (P.N == 512) bk_convert_kernel<9><<<blocks, 128, 0, (cudaStream_t)stream>>>(P, d_coef, d_dev, npoly, d_twl);
   else return (int)cudaErrorInvalidValue;
+  return (int)cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------
+// folded key copy of the GINX throughput kernel (BrCfg::FOLD): device-form key [step][sign][row][column][N] -> the same layout with the
+// top digit's row folded into the others.  With K_r the row that multiplies digit l of accumulator component c (r = c + 2l), T = DG - 1:
+//   K'_{c+2l} = K_{c+2l} - B^(l-T) * K_{c+2T}  (l < T),      K'_{c+2T} = N * B^-T * K_{c+2T}      (mod Q, fully reduced)
+// Slot by slot, so the [chunk][lane][4] order within a polynomial does not matter.
+// ------------------------------------------------------------------------------------------
+struct FoldConst {
+  u32 w[8]; // w[l] = B^(l-T) mod Q for l < T, w[T] = N * B^-T mod Q
+};
+template <int DG> __global__ void __launch_bounds__(256) bk_fold_kernel(const u32 *__restrict__ bk, u32 *__restrict__ bkf, size_t total, u32 N, u32 Q,
+                                                                        const FoldConst F) {
+  constexpr int ROWS = 2 * DG, T = DG - 1;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    // i -> (step and sign, component c, column and slot); row r of polynomial (sign, r, column) sits at r * 2N
+    const size_t cs = i % (2 * (size_t)N), c = (i / (2 * (size_t)N)) & 1, ss = i / (4 * (size_t)N);
+    const size_t base = ss * ROWS * 2 * N + cs;
+    const u64 top = bk[base + (c + 2 * T) * 2 * N];
+#pragma unroll
+    for (int l = 0; l < T; l++) {
+      const size_t o = base + (c + 2 * l) * 2 * N;
+      bkf[o] = (u32)(((u64)bk[o] + Q - top * F.w[l] % Q) % Q);
+    }
+    bkf[base + (c + 2 * T) * 2 * N] = (u32)(top * F.w[T] % Q);
+  }
+}
+static u64 powmod_q(u64 b, u64 e, u64 Q) {
+  u64 r = 1;
+  for (b %= Q; e; e >>= 1, b = b * b % Q)
+    if (e & 1) r = r * b % Q;
+  return r;
+}
+bool bk_fold_supported(const DevConst &P, int method_ap) { return !method_ap && P.N == 1024 && P.dG == 4 && P.logBG == 7; }
+int launch_bk_fold(const DevConst &P, const u32 *d_bk, u32 *d_bkf, size_t nsteps, void *stream) {
+  if (!bk_fold_supported(P, 0)) return (int)cudaErrorInvalidValue;
+  constexpr int DG = 4, T = DG - 1;
+  FoldConst F{};
+  const u64 Q = P.Q, binv = powmod_q(1ull << P.logBG, Q - 2, Q);
+  for (int l = 0; l < T; l++) F.w[l] = (u32)powmod_q(binv, T - l, Q);
+  F.w[T] = (u32)((u64)P.N * powmod_q(binv, T, Q) % Q);
+  const size_t total = nsteps * 2 * 2 * 2 * (size_t)P.N; // (step, sign) x component x (column, slot)
+  bk_fold_kernel<DG><<<148 * 8, 256, 0, (cudaStream_t)stream>>>(d_bk, d_bkf, total, P.N, P.Q, F);
   return (int)cudaGetLastError();
 }
 

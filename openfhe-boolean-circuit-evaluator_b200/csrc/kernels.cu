@@ -14,9 +14,10 @@
 //    correction at all: values grow by 2Q per stage and stay below 2^32); the RGSW x RLWE
 //    external product accumulates 2*dG 32x32->64 products per slot in one IMAD.WIDE chain and
 //    Montgomery-reduces once (keys are stored pre-multiplied by 2^32 * N^-1).
-//  * The accumulator lives in COEFFICIENT form in the registers of the warp that owns it for the
-//    whole blind rotation: each step is INTT(previous product) -> add -> signed digit decomposition
-//    -> dG forward NTTs, all in registers of the same warp (dG - 1 for STD128_OPT GINX, whose top digit is folded into a key copy).
+//  * The throughput kernel keeps the accumulator in EVALUATION form only, as N^-1 * NTT(acc) in shared
+//    memory, updated by the external product: each step is INTT (= the accumulator) -> signed digit
+//    decomposition -> dG forward NTTs, all in registers of the warp that owns the polynomial (dG - 1 for
+//    STD128_OPT GINX, whose top digit is folded into a key copy).
 //  * A CTA carries G gates through the n blind-rotation steps in lock step so that every
 //    bootstrapping-key word loaded from L2 is reused G times from registers (GINX).
 #include "device.cuh"
@@ -239,17 +240,24 @@ template <int DG, int LOGBG> constexpr u32 digit_offset() { // (B/2) * (1 + B + 
 }
 
 template <int LOGN, int DG, int LOGBG, int G, bool AP> struct BrCfg {
-  static constexpr int N = 1 << LOGN, E = N / 32, C = E / 4, ROWS = 2 * DG;
+  static constexpr int N = 1 << LOGN, E = N / 32, C = E / 4, ROWS = 2 * DG; // ROWS: key rows per sign = dct rows the product multiplies
   static constexpr int W = 2 * G, THREADS = 32 * W;
   static constexpr int NPAD = AP ? 1024 : 512; // per-gate index table (>= n*dR for AP, >= n for GINX)
-  static constexpr size_t dct_words = (size_t)G * ROWS * N;
   // first-stage product table: twiddle * (digit - B/2) mod Q for the 2^LOGBG digit values, one copy per bank (STD128_OPT shape only)
   static constexpr bool LUT = (LOGBG == 7 && LOGN == 10);
   static constexpr size_t lut_words = LUT ? (size_t)32 << LOGBG : 0;
   // GINX at the same shape: the top digit is folded into the key (bk_fold_kernel), so each component transforms DG - 1 digits per step
-  // and dct rows 2(DG-1) + c hold N^-1 * NTT(acc_c) instead of a digit row (see blind_rotate_kernel)
+  // and the product multiplies A_hat_c = N^-1 * NTT(acc_c) in place of the top digit (see blind_rotate_kernel)
   static constexpr bool FOLD = LUT && !AP;
+  // dct rows of a gate: the digit rows (digit l of component c in row c + 2l) and A_hat_c, the accumulator in evaluation form, in row
+  // AROW + c.  GINX adds to A_hat, so it must survive the step's digit transforms: FOLD keeps it in the top digit's rows, which the product
+  // multiplies, TOY in two extra rows.  AP replaces A_hat by the product's output, so it lives in digit row c: phase A inverse-transforms
+  // it before digit 0 is written there, and a skipped step writes no digits.
+  static constexpr int DROWS = (FOLD || AP) ? ROWS : ROWS + 2;
+  static constexpr int AROW = AP ? 0 : DROWS - 2;
+  static constexpr size_t dct_words = (size_t)G * DROWS * N;
   static constexpr size_t smem_bytes = (dct_words + 4 * N + (AP ? 0 : 2 * N) + lut_words) * 4 + (size_t)G * NPAD * 2;
+  static_assert(smem_bytes <= 227 * 1024, "more dynamic shared memory than a block may have");
 };
 
 template <int LOGN, int DG, int LOGBG, int G, bool AP>
@@ -264,13 +272,20 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
   // that sum always lies in [0, B^DG), they represent a exactly: acc_c = sum_l B^l d_{c,l} as integers, so in evaluation form the top digit
   // is D_{c,DG-1} = B^-(DG-1) (A_c - sum_{l<DG-1} B^l D_{c,l}) mod Q, A_c = NTT(acc_c).  Substituted into the external product, the top key
   // row moves into the other rows and into a row that multiplies A_hat_c = N^-1 A_c (bk_fold_kernel), and the step needs no transform of
-  // the top digit.  A_hat_c is kept current by adding the product's output row, which is N^-1 NTT of the accumulator's increment.
+  // the top digit.
+  // Every form keeps the accumulator ONLY as A_hat_c, in dct row AROW + c: the product's output row is N^-1 NTT of the accumulator's
+  // increment (GINX: A_hat_c += output) or of the whole new accumulator (AP: A_hat_c = output), and phase A gets acc_c back, fully reduced,
+  // as the unscaled inverse transform of A_hat_c.
   constexpr bool FOLD = Cfg::FOLD;
   static_assert(!FOLD || (DIGIT_OFF >= (SOLINAS_Q + 1) / 2 && (u64)DIGIT_OFF + (SOLINAS_Q - 3) / 2 < (1ull << (LOGBG * DG))),
                 "the digits do not cover the centred accumulator: the top digit cannot be folded into the key");
   constexpr int ND = FOLD ? DG - 1 : DG; // digit transforms per component and step
+  constexpr int DROWS = Cfg::DROWS, AROW = Cfg::AROW;
+  static_assert(AP || AROW == 2 * ND, "GINX: the A_hat rows follow the digit rows");
+  // input bound (units of Q) of the inverse transform of A_hat: GINX keeps it below 2Q (lazy_reduce); AP stores one redc of ROWS products
+  constexpr int AB = AP ? 8 : 2;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  u32 *dct = reinterpret_cast<u32 *>(smem_raw);                 // [G][ROWS][N]
+  u32 *dct = reinterpret_cast<u32 *>(smem_raw);                 // [G][DROWS][N]
   u32 *s_tw = dct + Cfg::dct_words;                             // fw | fws | iw | iws
   u32 *s_psiM = s_tw + 4 * N;                                   // [2N] monomial-factor table (GINX; N entries used)
   u32 *s_lut = s_psiM + (AP ? 0 : 2 * N);                       // [2^LOGBG][32] (Cfg::LUT)
@@ -322,39 +337,35 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
   }
   __syncthreads();
 
-  // ---- accumulator init: acc = (0, testvector) in coefficient form, column layout ----
+  // ---- accumulator init: A_hat = N^-1 * NTT(0, testvector) ----
   const bool gvalid = g < gcount;
-  u32 acc[E];
+  u32 *ahat = dct + ((size_t)g * DROWS + AROW + c) * N; // A_hat_c of gate g
+  u32 *dbuf = dct + ((size_t)g * DROWS + c) * N;        // digit 0 of component c: scratch of the inverse transforms (AP: = ahat)
+  if (gvalid) {
+    u32 acc[E]; // coefficient form, column layout
 #pragma unroll
-  for (int k = 0; k < E; k++) acc[k] = 0;
-  if (gvalid && c == 1) {
-    const u32 gate = gates[gate0 + g].op & 0xff;
-    const u32 q1 = P.gate_const[gate == OP_BOOTSTRAP ? OP_AND : gate], q2 = (q1 + q / 2) % q;
-    const u32 b = s_b[g], Q8 = P.Q8, Q8n = Q - P.Q8;
+    for (int k = 0; k < E; k++) acc[k] = 0;
+    if (c == 1) {
+      const u32 gate = gates[gate0 + g].op & 0xff;
+      const u32 q1 = P.gate_const[gate == OP_BOOTSTRAP ? OP_AND : gate], q2 = (q1 + q / 2) % q;
+      const u32 b = s_b[g], Q8 = P.Q8, Q8n = Q - P.Q8;
 #pragma unroll
-    for (int k = 0; k < E; k++) {
-      const u32 idx = lane + 32 * k;
-      if (idx % P.factor == 0) {
-        const u32 t = (b + q - idx / P.factor) % q;
-        const bool in = (q1 < q2) ? (t >= q1 && t < q2) : !(t >= q2 && t < q1);
-        acc[k] = in ? Q8n : Q8;
+      for (int k = 0; k < E; k++) {
+        const u32 idx = lane + 32 * k;
+        if (idx % P.factor == 0) {
+          const u32 t = (b + q - idx / P.factor) % q;
+          const bool in = (q1 < q2) ? (t >= q1 && t < q2) : !(t >= q2 && t < q1);
+          acc[k] = in ? Q8n : Q8;
+        }
       }
     }
-  }
-  if (FOLD && gvalid) { // A_hat_c = N^-1 * NTT(acc_c) (zero for component 0), below 2Q, in the row the top digit of component c had
-    u32 x[E];
+    ntt_forward<LOGN>(acc, ahat, P, tt, lane);
 #pragma unroll
-    for (int k = 0; k < E; k++) x[k] = acc[k];
-    u32 *abuf = dct + ((size_t)g * ROWS + 2 * (DG - 1) + c) * N;
-    ntt_forward<LOGN>(x, abuf, P, tt, lane);
-#pragma unroll
-    for (int k = 0; k < E; k++) x[k] = mul_shoup(x[k], P.ninv, P.ninvs, Q);
-    row_store<E>(abuf, x, lane);
+    for (int k = 0; k < E; k++) acc[k] = mul_shoup(acc[k], P.ninv, P.ninvs, Q); // below 2Q
+    row_store<E>(ahat, acc, lane);
   }
 
   const int nsteps = AP ? n * P.dR : n;
-  bool pending = false;
-  u32 *mybuf = dct + ((size_t)g * ROWS + c) * N; // R[g][c] aliases dct row c of gate g
 
   // MAC work split: item -> (chunk qc, gate split)
   constexpr int GS = (W >= C) ? (W / C) : 1;
@@ -401,21 +412,18 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
     bool active = gvalid;
     if (AP && gvalid) active = s_idx[g * NPAD + step] != 0;
     if (active) {
-      if (pending) {
-        u32 x[E];
-        row_load<E>(mybuf, x, lane);
-        ntt_inverse<LOGN, AP ? 8 : 4>(x, mybuf, P, tt, lane);
-#pragma unroll
-        for (int k = 0; k < E; k++) acc[k] = AP ? x[k] : csub(acc[k] + x[k], Q);
-      }
+      // acc_c = INTT(A_hat_c) in [0, Q).  The transform's scratch is digit row c, rewritten below: GINX's A_hat_c, in other rows, stays as
+      // it is; AP's is that row and is replaced by the product anyway.
+      u32 dp[E];
+      row_load<E>(ahat, dp, lane);
+      ntt_inverse<LOGN, AB>(dp, dbuf, P, tt, lane);
       // SignedDigitDecompose (a12): centre, peel DG signed base-2^LOGBG digits, digit l of component c -> row c+2l
       // Closed form of the sequential peel (r = signed low digit; d = (d - r) >> LOGBG): adding B/2 at every digit
       // position turns the balanced digits into the plain base-B digits of d + OFF, so digit l is one shift, one mask and
       // one subtraction with no dependency on the digits below it (the top digit wraps exactly like the reference's
       // sign-truncation when dG digits do not cover the centred range, e.g. TOY).  FOLD: the top digit is not needed.
-      u32 dp[E];
 #pragma unroll
-      for (int k = 0; k < E; k++) dp[k] = ((acc[k] < (Q >> 1)) ? acc[k] : acc[k] - Q) + DIGIT_OFF;
+      for (int k = 0; k < E; k++) dp[k] = ((dp[k] < (Q >> 1)) ? dp[k] : dp[k] - Q) + DIGIT_OFF;
 #pragma unroll
       for (int l = 0; l < ND; l++) {
         u32 x[E], pre[Cfg::LUT ? E / 2 : 1];
@@ -427,7 +435,7 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
           if (Cfg::LUT && k >= E / 2) { pre[Cfg::LUT ? k - E / 2 : 0] = s_lut[(dgt << 5) + lane]; x[k] = 0; }
           else x[k] = dgt + (Q - (1u << (LOGBG - 1)));
         }
-        u32 *buf = dct + ((size_t)g * ROWS + c + 2 * l) * N;
+        u32 *buf = dct + ((size_t)g * DROWS + c + 2 * l) * N;
         if (KEY_HOIST && l == ND - 1 && warp < C * GS) BFHE_GX_LOAD(warp % C);
         ntt_forward<LOGN, Cfg::LUT>(x, buf, P, tt, lane, pre);
         row_store<E>(buf, x, lane);
@@ -435,7 +443,6 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
     } else if (KEY_HOIST && warp < C * GS) { // empty gate slot (ragged last CTA): no transform to hide behind, but the product still needs the words
       BFHE_GX_LOAD(warp % C);
     }
-    pending = pending || active;
     PT_T(0);
     // the first key words of this warp's chunk are requested BEFORE the barrier, so the L2 round trip overlaps the wait for the slower
     // warps of the CTA instead of stalling the external product (ncu r1: 6 % of samples sat on these loads)
@@ -481,10 +488,12 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
             fn[r] = s_psiM[f_phys((0u - u) & (N - 1))];
           }
         }
-        u32 *gd = dct + (size_t)gg * ROWS * N + Lay<E>::chunk_off(lane, qc);
-        uint4 dv[ROWS];
+        u32 *gd = dct + (size_t)gg * DROWS * N + Lay<E>::chunk_off(lane, qc);
+        // the ROWS multiplied rows, and for GINX the A_hat rows the output is added to (FOLD: the same rows)
+        constexpr int NLD = AP ? ROWS : DROWS;
+        uint4 dv[NLD];
 #pragma unroll
-        for (int r = 0; r < ROWS; r++) dv[r] = *reinterpret_cast<const uint4 *>(gd + (size_t)r * N);
+        for (int r = 0; r < NLD; r++) dv[r] = *reinterpret_cast<const uint4 *>(gd + (size_t)r * N);
 #pragma unroll
         for (int cc = 0; cc < 2; cc++) {
           u32 out[4];
@@ -508,11 +517,13 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
               out[sl] = redc((u64)pp * fp[sl] + (u64)pn * fn[sl], Q, P.qinv_neg);
             }
           }
-          // R[gg][cc] overwrites dct row cc: this thread has already consumed that chunk of every row
-          *reinterpret_cast<uint4 *>(gd + (size_t)cc * N) = make_uint4(out[0], out[1], out[2], out[3]);
-          if constexpr (FOLD) { // A_hat_cc += R[gg][cc], kept below 2Q (the products' bounds assume < 22Q)
-            const uint4 a = dv[ROWS - 2 + cc];
-            *reinterpret_cast<uint4 *>(gd + (size_t)(ROWS - 2 + cc) * N) =
+          // the output goes to A_hat_cc only (this thread has already consumed that chunk of every row).  GINX: A_hat_cc += output, kept
+          // below 2Q (FOLD: the products' bounds assume < 22Q).  AP: the output is the whole new accumulator.
+          u32 *ga = gd + (size_t)(AROW + cc) * N;
+          if constexpr (AP) *reinterpret_cast<uint4 *>(ga) = make_uint4(out[0], out[1], out[2], out[3]);
+          else {
+            const uint4 a = dv[AROW + cc];
+            *reinterpret_cast<uint4 *>(ga) =
                 make_uint4(lazy_reduce(a.x + out[0], Q), lazy_reduce(a.y + out[1], Q), lazy_reduce(a.z + out[2], Q), lazy_reduce(a.w + out[3], Q));
           }
         }
@@ -528,13 +539,9 @@ blind_rotate_kernel(const __grid_constant__ DevConst P, const DevGate *__restric
 
   // ---- epilogue: last inverse transform, sample extraction (a14) and ModSwitch Q -> qKS (a15) ----
   if (gvalid) {
-    if (pending) {
-      u32 x[E];
-      row_load<E>(mybuf, x, lane);
-      ntt_inverse<LOGN, AP ? 8 : 4>(x, mybuf, P, tt, lane);
-#pragma unroll
-      for (int k = 0; k < E; k++) acc[k] = AP ? x[k] : csub(acc[k] + x[k], Q);
-    }
+    u32 acc[E];
+    row_load<E>(ahat, acc, lane);
+    ntt_inverse<LOGN, AB>(acc, dbuf, P, tt, lane);
     const size_t gi = (size_t)gate0 + g;
     if (acc_dbg) {
 #pragma unroll
@@ -1016,12 +1023,11 @@ int launch_blind_rotate(const DevConst &P, int method_ap, const DevGate *d_gates
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   // Which variant?  Measured on B200, STD128_OPT GINX (profiles/): one gate on four SMs 0.98 ms per wave of up to 33 gates; one gate on two
   // SMs 1.48 ms up to 74; latency form (one gate per CTA) 2.22 ms per wave of `sms` gates; throughput form (4 gates per CTA share every
-  // key word) 5.97 ms per wave of 4 * sms gates with the folded key (6.73 ms before).  Narrow circuit levels go to the cluster forms, wide
-  // batches to the throughput form.
+  // key word) 5.68 ms per wave of 4 * sms gates.  Narrow circuit levels go to the cluster forms, wide batches to the throughput form.
   if (force_g == 0 && have_clx && count <= clx_fast_gates()) return launch_blind_rotate_clx(P, method_ap, d_gates, count, *v2, d_ext, d_acc_dbg, stream, info);
   if (force_g == 0 && have_cl2 && count <= cl2_max_gates()) return launch_blind_rotate_cl2(P, d_gates, count, *v2, d_ext, d_acc_dbg, stream, info);
   const long lat_cost = (long)((count + sms - 1) / sms) * 222;           // 2.22 ms per wave of `sms` gates
-  const long thr_cost = (long)((count + 4 * sms - 1) / (4 * sms)) * 597; // 5.97 ms per wave of 4 * sms gates
+  const long thr_cost = (long)((count + 4 * sms - 1) / (4 * sms)) * 568; // 5.68 ms per wave of 4 * sms gates
   const bool lat = force_g == 8 || (force_g == 0 && lat_cost <= thr_cost);
   if (lat) {
     if (P.N == 1024 && P.dG == 4 && P.logBG == 7)

@@ -71,7 +71,7 @@ struct Level {
 // tiny wait launch (~0.015 ms), or one ncclAllGather (~0.05 ms, BFHE_EXCHANGE=nccl).  The plan is made before the slabs exist, so the
 // peer-store figure is assumed unless NCCL was asked for; should the mapping fail later, the plan is merely a little optimistic.
 struct FormCosts {
-  double cl4 = 1.05, cl2 = 1.55, lat = 2.36, thr = 6.1, exchange = exchange_default();
+  double cl4 = 1.05, cl2 = 1.55, lat = 2.36, thr = 5.85, exchange = exchange_default();
   bool measured = false;
   static double exchange_default() { const char *m = std::getenv("BFHE_EXCHANGE"); return m && std::strcmp(m, "nccl") == 0 ? 0.05 : 0.015; }
 };

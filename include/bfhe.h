@@ -183,6 +183,26 @@ int bfhe_circuit_set_shard_threshold(bfhe_circuit *, int min_bootstraps);
 int bfhe_circuit_reset(bfhe_circuit *);                                     /* Circuit::Reset */
 int bfhe_circuit_set_input(bfhe_circuit *, const uint8_t *bits, size_t nbits, uint64_t seed); /* Circuit::SetInput (all input buses concatenated) */
 int bfhe_circuit_clock(bfhe_circuit *, uint8_t *out_bits, size_t cap, uint8_t *plain_out_bits); /* Circuit::Clock */
+/* ---- evaluation with the evaluation keys only (a context that imported bfhe_export_keys(..., include_sk = 0)) ----
+ * Circuit::SetInput on ciphertexts.  Needs evaluation keys only, never the secret key.  cts: nbits rows of ct_stride words, the input
+ * buses concatenated in SetInput's bit order; on_device != 0: memory on the context's device, read in order on the launch stream
+ * (bfhe_set_stream), else host memory.  Level 0 bootstraps them, exactly as it bootstraps SetInput's fresh encryptions.
+ * Input contract: every word a_0 .. a_{n-1}, b is below q, else BFHE_ERR_FORMAT naming the first bad row, and the circuit is left
+ * without input (Clock fails with BFHE_ERR_STATE until the next SetInput).  Padding words are ignored and stored as zero.
+ * Modes: encrypted mode with plaintext and verify mode off, else BFHE_ERR_STATE (ciphertext inputs have no plaintext).  Argument and
+ * state errors are reported before the device is touched.
+ * Flip-flops power up from the trivial encryption of 0 (all-zero row), bootstrapped into the latch row: they decrypt exactly as after
+ * SetInput(bits), whose power-up value is Encrypt(0), but the state rows' ciphertexts differ.
+ * Sharded circuits (world > 1): collective; rank 0's rows are used and broadcast with rank 0's validation status, so every rank returns
+ * the same code.  Other ranks may pass NULL.
+ * After this call bfhe_circuit_clock (bits) decrypts as usual when the context holds the secret key, and fails with BFHE_ERR_STATE
+ * before launching anything when it does not. */
+int bfhe_circuit_set_input_ct(bfhe_circuit *, const uint32_t *cts, size_t nbits, int on_device);
+/* Circuit::Clock with the outputs left encrypted: out_bits rows of ct_stride words (padding words zero) into out_cts, host or device
+ * memory (on_device as above).  An output that reads its wire through NOT comes out as EvalNOT of that row, so it decrypts to what
+ * bfhe_circuit_clock returns.  Encrypted mode without verify mode; works after either SetInput form and needs no secret key.  Every rank
+ * of a sharded circuit returns all outputs.  Returns after the rows are written. */
+int bfhe_circuit_clock_ct(bfhe_circuit *, uint32_t *out_cts, size_t cap_rows, int on_device);
 int bfhe_circuit_stats(const bfhe_circuit *, double *device_ms, double *host_ms, uint64_t *verify_mismatches);
 /* the schedule in use: wave capacity (0 = ASAP), levels incl. the input-bootstrap level, levels that are sharded, and the four launch
  * costs (ms: 4-CTA cluster, 2-CTA cluster, one gate per SM, four gates per SM) the planner used -- measured by a start-up probe on the

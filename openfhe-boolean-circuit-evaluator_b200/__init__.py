@@ -57,7 +57,7 @@ ABI_SYMBOLS = [
     "bfhe_circuit_dump_gate_count", "bfhe_circuit_load_netlist", "bfhe_circuit_get_netlist", "bfhe_circuit_write_out",
     "bfhe_circuit_load_netlist_ex", "bfhe_circuit_set_shard_threshold", "bfhe_circuit_dump_gate_count_ex",
     "bfhe_circuit_dump_text", "bfhe_circuit_dff_plan", "bfhe_circuit_get_schedule",
-    "bfhe_circuit_exchange_mode",
+    "bfhe_circuit_exchange_mode", "bfhe_circuit_set_input_ct", "bfhe_circuit_clock_ct",
     "bfhe_import_openfhe_json", "bfhe_export_openfhe_json", "bfhe_import_openfhe_ct_json", "bfhe_export_openfhe_ct_json",
 ]
 
@@ -120,6 +120,8 @@ def lib():
     L.bfhe_circuit_reset.argtypes = [vp]
     L.bfhe_circuit_set_input.argtypes = [vp, vp, sz, C.c_uint64]
     L.bfhe_circuit_clock.argtypes = [vp, vp, sz, vp]
+    L.bfhe_circuit_set_input_ct.argtypes = [vp, vp, sz, C.c_int]
+    L.bfhe_circuit_clock_ct.argtypes = [vp, vp, sz, C.c_int]
     L.bfhe_circuit_stats.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_uint64)]
     L.bfhe_circuit_level_plan.argtypes = [vp, C.c_uint32, C.c_int, C.c_int, vp, sz, u32p, u32p, u32p]
     L.bfhe_circuit_plan_misc.argtypes = [vp, u32p, u32p, u32p, vp, u32p, C.c_uint32, vp]
@@ -173,6 +175,42 @@ class Slab:
         if self.ptr:
             self.ctx.L.bfhe_slab_free(self.ctx.h, self.ptr)
             self.ptr = None
+
+    def range(self, first_row=0, rows=None):
+        """rows [first_row, first_row + rows) as a device buffer for Circuit.set_input_ct / clock_ct"""
+        rows = self.rows - first_row if rows is None else rows
+        if first_row < 0 or rows < 0 or first_row + rows > self.rows:
+            raise ValueError("rows %d..%d outside a slab of %d rows" % (first_row, first_row + rows, self.rows))
+        return SlabRows(self, first_row, rows)
+
+
+class SlabRows:
+    """A row range of a Slab (Slab.range)."""
+
+    def __init__(self, slab, first_row, rows):
+        self.slab, self.first_row, self.rows = slab, first_row, rows
+        self.ptr = slab.ptr + first_row * slab.ctx.stride * 4
+
+
+def _device_rows(buf, stride):
+    """(device pointer, rows) of a Slab, a SlabRows or an object exposing __cuda_array_interface__ with shape (rows, stride), 4-byte
+    integers and C-contiguous layout.  The library checks that the memory is on the context's device."""
+    if isinstance(buf, (Slab, SlabRows)):
+        if buf.ptr is None:
+            raise ValueError("slab has been freed")
+        return buf.ptr, buf.rows
+    cai = getattr(buf, "__cuda_array_interface__", None)
+    if cai is None:
+        raise TypeError("expected a Slab, Slab.range(...) or an object with __cuda_array_interface__, got %s" % type(buf).__name__)
+    shape = tuple(cai["shape"])
+    if len(shape) != 2 or shape[1] != stride:
+        raise ValueError("device buffer shape %s, expected (rows, %d)" % (shape, stride))
+    if cai["typestr"][1:] not in ("i4", "u4") or cai["typestr"][0] == ">":
+        raise TypeError("device buffer element type %s, expected 4-byte integers (int32 or uint32)" % cai["typestr"])
+    strides = cai.get("strides")
+    if strides is not None and tuple(strides) != (stride * 4, 4) and shape[0] > 1:
+        raise ValueError("device buffer is not C-contiguous (strides %s)" % (tuple(strides),))
+    return cai["data"][0], shape[0]
 
 
 class Context:
@@ -524,6 +562,35 @@ class Circuit:
         """inputs: list of bit lists, one per input bus (Inputs = vector<vector<unsigned>>, src/circuit.h:50)."""
         flat = np.ascontiguousarray(np.concatenate([np.asarray(i, dtype=np.uint8).ravel() for i in inputs]), dtype=np.uint8)
         self._ck(self.L.bfhe_circuit_set_input(self.h, _ptr(flat), flat.size, seed))
+
+    def set_input_ct(self, cts):
+        """SetInput on ciphertexts (bfhe_circuit_set_input_ct): needs the evaluation keys only.  cts: host numpy array (nbits, ct_stride)
+        of uint32 (int32 accepted), or a device buffer (Slab, Slab.range(...), or __cuda_array_interface__ with that shape).  Sharded
+        circuits: rank 0's rows are used; other ranks may pass None."""
+        stride = self.ctx.stride
+        if cts is None:
+            self._ck(self.L.bfhe_circuit_set_input_ct(self.h, None, sum(self.info()["input_bits"]), 0))
+        elif isinstance(cts, np.ndarray):
+            if cts.ndim != 2 or cts.shape[1] != stride:
+                raise ValueError("ciphertext array shape %s, expected (nbits, %d)" % (cts.shape, stride))
+            if cts.dtype not in (np.uint32, np.int32):
+                raise TypeError("ciphertext array dtype %s, expected uint32" % cts.dtype)
+            a = np.ascontiguousarray(cts).view(np.uint32)
+            self._ck(self.L.bfhe_circuit_set_input_ct(self.h, _ptr(a), a.shape[0], 0))
+        else:
+            ptr, rows = _device_rows(cts, stride)
+            self._ck(self.L.bfhe_circuit_set_input_ct(self.h, ptr, rows, 1))
+
+    def clock_ct(self, out=None):
+        """Clock with the outputs left encrypted (bfhe_circuit_clock_ct): a numpy array (out_bits, ct_stride) of uint32, or, with `out`
+        a device buffer as in set_input_ct with at least out_bits rows, the rows written there (and `out` returned)."""
+        if out is None:
+            host = np.zeros((self.info()["output_bits"], self.ctx.stride), dtype=np.uint32)
+            self._ck(self.L.bfhe_circuit_clock_ct(self.h, _ptr(host), host.shape[0], 0))
+            return host
+        ptr, rows = _device_rows(out, self.ctx.stride)
+        self._ck(self.L.bfhe_circuit_clock_ct(self.h, ptr, rows, 1))
+        return out
 
     def Clock(self):
         """returns Outputs = [[bits of OUT:0]]; the plaintext pass result is kept in self.plain_out"""

@@ -7,7 +7,6 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 HOST = os.path.join(HERE, "host")
 LIB = os.path.join(HERE, "libbfhe_b200.so")
-TB = os.path.join(HERE, "examples", "tb_circuit")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 CCBIN = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
 
@@ -48,9 +47,11 @@ def build(force=False, verbose=False):
         raise subprocess.CalledProcessError(1, failed[0])
     subprocess.check_call([NVCC, "-ccbin", CCBIN, "-shared", "-o", LIB] + objs + ["-lgomp", "-ldl", "-cudart", "static"])
     # C++ example written against the reference-shaped headers (host/circuit.h, host/binfhecontext.h)
-    ex = os.path.join(HERE, "examples", "tb_circuit.cpp")
-    if os.path.exists(ex):
-        subprocess.check_call([CCBIN, "-O2", "-std=c++17", "-o", TB, ex, "-L" + HERE, "-lbfhe_b200", "-Wl,-rpath," + HERE])
+    for name in ("tb_circuit", "tb_client_server"):
+        ex = os.path.join(HERE, "examples", name + ".cpp")
+        if os.path.exists(ex):
+            subprocess.check_call([CCBIN, "-O2", "-std=c++17", "-o", os.path.join(HERE, "examples", name), ex, "-L" + HERE, "-lbfhe_b200",
+                                   "-Wl,-rpath," + HERE])
     return LIB
 
 

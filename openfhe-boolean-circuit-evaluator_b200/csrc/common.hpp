@@ -106,6 +106,9 @@ int launch_peer_epoch_bump(u32 *epoch, void *stream);
 int launch_peer_wait(const u32 *local_flags, const u32 *epoch, u32 world, u32 rank, int index, u32 per_epoch, u32 *err, void *stream);
 int launch_peer_signal(const PeerX &px, void *stream);
 int launch_eval_not(const DevConst &P, const u32 *const *d_in, u32 *const *d_out, int count, void *stream);
+// count rows of ct_stride words from outside the program: zero the padding words, atomicMin the index of every row holding a word >= q
+// into *d_bad_row
+int launch_ct_ingest(const DevConst &P, u32 *d_rows, int count, u32 *d_bad_row, void *stream);
 int launch_bk_convert(const DevConst &P, const u32 *d_coef, u32 *d_dev, size_t npoly, const u32 *d_twl, void *stream);
 // key copy of the GINX throughput kernel at the STD128_OPT shape (N 1024, dG 4, base 2^7): the device-form key with its top digit row folded
 // into the others (kernels.cu bk_fold_kernel); nsteps = n

@@ -698,7 +698,7 @@ static int ensure_ptrs(bfhe_ctx *c, size_t count) {
   return BFHE_OK;
 }
 
-static int not_ptr_batch(bfhe_ctx *c, const std::vector<const u32 *> &in, const std::vector<u32 *> &out) {
+int bfhe::not_ptr_batch(bfhe_ctx *c, const std::vector<const u32 *> &in, const std::vector<u32 *> &out) {
   if (in.empty()) return BFHE_OK;
   int rc = ensure_ptrs(c, in.size());
   if (rc) return rc;

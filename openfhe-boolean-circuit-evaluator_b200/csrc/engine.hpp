@@ -86,4 +86,6 @@ namespace bfhe {
 // run one list of single-bootstrap gates (device pointers already resolved) through blind rotation + key switch
 int run_gate_list(bfhe_ctx *c, const DevGate *host_list, size_t count, u32 *acc_dbg_host);
 int ensure_device_keys(bfhe_ctx *c);
+// EvalNOT of in[i] into out[i] through the context's pointer buffers (low bit of in[i] set: plain copy); caller holds c->mtx
+int not_ptr_batch(bfhe_ctx *c, const std::vector<const u32 *> &in, const std::vector<u32 *> &out);
 } // namespace bfhe

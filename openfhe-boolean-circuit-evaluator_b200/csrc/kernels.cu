@@ -1303,6 +1303,26 @@ int launch_eval_not(const DevConst &P, const u32 *const *d_in, u32 *const *d_out
 }
 
 // ------------------------------------------------------------------------------------------
+// ciphertext ingest: rows that came from outside the program (bfhe_circuit_set_input_ct)
+// ------------------------------------------------------------------------------------------
+// every word a_0..a_{n-1}, b must be below q (the kernels assume reduced operands); the lowest offending row goes to *bad_row,
+// which the host set to 0xffffffff.  Padding words are zeroed.
+__global__ void ct_ingest_kernel(const __grid_constant__ DevConst P, u32 *__restrict__ rows, u32 *bad_row) {
+  u32 *row = rows + (size_t)blockIdx.x * P.ct_stride;
+  bool bad = false;
+  for (u32 i = threadIdx.x; i < P.ct_stride; i += blockDim.x) {
+    if (i > P.n) row[i] = 0;
+    else bad = bad || row[i] >= P.q;
+  }
+  if (__syncthreads_or(bad) && threadIdx.x == 0) atomicMin(bad_row, blockIdx.x);
+}
+int launch_ct_ingest(const DevConst &P, u32 *d_rows, int count, u32 *d_bad_row, void *stream) {
+  if (count <= 0) return 0;
+  ct_ingest_kernel<<<count, 128, 0, (cudaStream_t)stream>>>(P, d_rows, d_bad_row);
+  return (int)cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------
 // bootstrapping-key conversion: canonical coefficient form -> device form
 // (forward NTT in this kernel's slot order, times N^-1 * 2^32, laid out [chunk][lane][4] per polynomial)
 // ------------------------------------------------------------------------------------------

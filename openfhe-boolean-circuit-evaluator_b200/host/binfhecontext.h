@@ -77,6 +77,14 @@ public:
   }
   LWECiphertext Bootstrap(ConstLWECiphertext ct) const { return one_gate(BFHE_BOOTSTRAP, ct, ct); }
 
+  // the key blob of bfhe_export_keys (include/bfhe.h): without the secret key it is what an evaluator needs, and all it gets
+  std::vector<uint8_t> ExportKeys(bool include_sk) const {
+    std::vector<uint8_t> blob(bfhe_keyblob_size(raw()));
+    check(bfhe_export_keys(raw(), blob.data(), blob.size(), include_sk ? 1 : 0));
+    return blob;
+  }
+  void ImportKeys(const std::vector<uint8_t> &blob) { check(bfhe_import_keys(raw(), blob.data(), blob.size())); }
+
   bfhe_ctx *raw() const {
     if (!m_ctx) throw config_error("GenerateBinFHEContext has not been called");
     return m_ctx.get();

@@ -66,6 +66,12 @@ public:
     gep.sk = sk;
     h = bfhe_circuit_create(cc.raw());
   }
+  // evaluator over a context whose keys were imported (BinFHEContext::ImportKeys): no key generation, and the context may hold no
+  // secret key.  Inputs and outputs are then ciphertexts: SetInput(ciphertexts) and ClockCiphertexts().
+  explicit Circuit(const lbcrypto::BinFHEContext &context) : cc(context) {
+    gep.cc = cc;
+    h = bfhe_circuit_create(cc.raw());
+  }
   ~Circuit() { bfhe_circuit_destroy(h); }
   Circuit(const Circuit &) = delete;
   Circuit &operator=(const Circuit &) = delete;
@@ -87,6 +93,18 @@ public:
       for (auto b : bus) flat.push_back((uint8_t)b);
     }
     ok(bfhe_circuit_set_input(h, flat.data(), flat.size(), input_seed ? input_seed++ : 0));
+  }
+  // SetInput on ciphertexts (bfhe_circuit_set_input_ct): one ciphertext per input bit, buses in SetInput's order.  Needs encrypted
+  // mode and evaluation keys only; throws std::runtime_error on failure (a ciphertext word >= q, wrong count, wrong mode).
+  void SetInput(const std::vector<std::vector<lbcrypto::LWECiphertext>> &input) {
+    const size_t st = cc.params().ct_stride;
+    std::vector<uint32_t> rows;
+    for (auto &bus : input)
+      for (auto &ct : bus) {
+        if (!ct || ct->row.size() != st) throw std::runtime_error("SetInput: ciphertext is not a row of ct_stride words");
+        rows.insert(rows.end(), ct->row.begin(), ct->row.end());
+      }
+    check(bfhe_circuit_set_input_ct(h, rows.data(), rows.size() / st, 0));
   }
   void setPlaintext(bool f) { plaintext_flag = f; push_flags(); }
   bool getPlaintext() const { return plaintext_flag; }
@@ -114,6 +132,20 @@ public:
     plainOut.assign(1, std::vector<unsigned int>(pout.begin(), pout.end()));
     return o;
   }
+  // Clock with the outputs left encrypted (bfhe_circuit_clock_ct): one ciphertext per output bit; needs no secret key
+  std::vector<lbcrypto::LWECiphertext> ClockCiphertexts() {
+    uint32_t nout = 0;
+    bfhe_circuit_info(h, nullptr, nullptr, &nout, nullptr, nullptr, nullptr, nullptr);
+    const size_t st = cc.params().ct_stride;
+    std::vector<uint32_t> rows((size_t)nout * st);
+    check(bfhe_circuit_clock_ct(h, rows.data(), nout, 0));
+    std::vector<lbcrypto::LWECiphertext> out(nout);
+    for (uint32_t b = 0; b < nout; b++) {
+      out[b] = std::make_shared<lbcrypto::LWECiphertextImpl>();
+      out[b]->row.assign(rows.begin() + (size_t)b * st, rows.begin() + (size_t)(b + 1) * st);
+    }
+    return out;
+  }
   void dumpGateCount() {
     uint32_t i, o, a, r, x, n;
     bfhe_circuit_dump_gate_count(h, &i, &o, &a, &r, &x, &n);
@@ -139,6 +171,9 @@ private:
     bfhe_circuit_dump_text(h, what, &s[0], s.size(), &need);
     s.resize(need);
     return s;
+  }
+  static void check(int rc) {
+    if (rc != BFHE_OK) throw std::runtime_error(bfhe_last_error());
   }
   bool ok(int rc) {
     if (rc != BFHE_OK) std::cerr << bfhe_last_error() << std::endl;

@@ -75,9 +75,42 @@ int bfhe_btkeygen(bfhe_ctx *, uint64_t seed); /* bootstrapping + key-switching k
  *   sk[n] int32 | BK coefficient form uint32 | KSK [N][baseKS][dKS][n+1] uint16 (qKS<=2^16) or uint32 */
 size_t bfhe_keyblob_size(const bfhe_ctx *);
 int bfhe_export_keys(const bfhe_ctx *, void *buf, size_t cap, int include_sk);
+/* either blob, BFHEKEY1 or BFHEKEY2 (below); the parameters must match this context, else BFHE_ERR_FORMAT */
 int bfhe_import_keys(bfhe_ctx *, const void *buf, size_t len);
 int bfhe_save_keys(const bfhe_ctx *, const char *path, int include_sk);
 int bfhe_load_keys(bfhe_ctx *, const char *path);
+
+/* ---- compact evaluation keys: the public masks come from a seed ----
+ * Most of a key blob is uniform masks that carry no secret: n of the n+1 words of every KSK row, and column 0 of every RGSW row of the
+ * BK.  bfhe_btkeygen_compact generates the same kinds of keys as bfhe_btkeygen, with the same noise, and leaves the context in the same
+ * state, but every mask is the expansion of a 256-bit public MASK SEED that the context keeps.  Its blob, BFHEKEY2, then carries only the
+ * seed and the bodies: at STD128_OPT about 33.4 MB instead of 329.5 MB (GINX) and 1.02 GB instead of 2.30 GB (AP).
+ *   mask seed: seed == 0 -> 256 bits of OS entropy, drawn independently of the secret stream; seed != 0 -> 256 bits of a dedicated stream
+ *              of the secret SeedKey (reproducible for tests, and ChaCha20 output reveals nothing about its key).
+ *   expansion: mask row r is the ChaCha20 keystream (RFC 8439 block function, 64-bit block counter from 0 in words 12-13, 64-bit nonce
+ *              in words 14-15) with key = mask seed (eight little-endian words) and nonce = r.  Coefficient t of the row is the
+ *              little-endian 128-bit integer of keystream words 4t .. 4t+3, reduced mod the row's modulus m (qKS for the KSK, Q for the
+ *              BK): statistical distance from uniform below m / 2^128 per coefficient, no rejection, so one ChaCha block gives four
+ *              coefficients and any of them can be computed alone.
+ *   rows:      KSK row (i, j, k) (i < N, digit value j < baseKS, digit k < dKS) is r = (i * baseKS + j) * dKS + k; BK mask polynomial p is
+ *              r = 2^40 + p, where p counts the column-0 polynomials in BFHEKEY1 order (RGSW t, row l: p = t * 2dG + l).
+ *   bodies:    KSK b = <a,s> + e + z_i * j * baseKS^k mod qKS, as bfhe_btkeygen.  BK row l of an RGSW of m (m = 1 or 0 for GINX,
+ *              +-X^mm for AP): odd rows b = a*z + e + m*g^(l/2), as bfhe_btkeygen; even rows, whose message bfhe_btkeygen adds to the
+ *              mask, b = a*z + e - m*g^(l/2)*z, so the public mask never carries the message.  The phase b - a*z is unchanged, and the
+ *              kernels see an ordinary RGSW key.
+ * SECURITY: the mask seed is public.  It is drawn fresh by every call, so two key sets never share one; never reuse a mask seed for
+ * another key set (two key sets with one seed and different secrets would share their masks).
+ * Layout of BFHEKEY2: the BFHEKEY1 header with magic "BFHEKEY2", version 1 (the same fields and values) | mask seed, 32 bytes |
+ *   sk[n] int32 (zero without the secret key) | BK bodies: the column-1 polynomials in BFHEKEY1 order, coefficient form, uint32 |
+ *   KSK bodies [N][baseKS][dKS], uint16 when qKS <= 2^16 else uint32; each section padded to 8 bytes, as in BFHEKEY1.
+ * Import checks every body word against its modulus (BFHE_ERR_FORMAT naming the section and index, before any device work, leaving the
+ * previous keys in place).  A device context uploads the bodies and generates the masks on the GPU; it keeps the bodies, not the full
+ * keys, on the host, and bfhe_export_keys / bfhe_export_openfhe_json expand them on the host when called.  A host-only context expands
+ * them on import. */
+int bfhe_btkeygen_compact(bfhe_ctx *, uint64_t seed);
+size_t bfhe_keyblob_compact_size(const bfhe_ctx *);
+/* BFHE_ERR_STATE when the keys have no mask seed (bfhe_btkeygen, a BFHEKEY1 import, an OpenFHE JSON import) */
+int bfhe_export_keys_compact(const bfhe_ctx *, void *buf, size_t cap, int include_sk);
 
 /* ---- OpenFHE 1.0.x object exchange (SURVEY 8 row f-3; the reference's crypto is find_package(OpenFHE), CMakeLists.txt:8, "Tested with
  * OpenFHE v.1.0.1", Release_Notes.md:4) ----
@@ -138,6 +171,10 @@ int bfhe_dbg_blind_rotate(bfhe_ctx *, uint32_t *dev_slab, const bfhe_gate *gates
 int bfhe_dbg_set_gates_per_cta(bfhe_ctx *, int gates_per_cta);
 /* how many gates the 2-CTA / 4-CTA cluster forms keep co-resident on this device (cudaOccupancyMaxActiveClusters; differs between GPUs) */
 int bfhe_dbg_cluster_limits(bfhe_ctx *, int *cl2_gates, int *cl4_gates);
+/* imports a BFHEKEY2 blob as bfhe_import_keys does on a device context (same kernels and buffers) and writes the BFHEKEY1 blob the device
+ * expansion produced: the BK staging buffer as downloaded, the device KSK restored to [N][baseKS][dKS][n+1] on the host.  full_blob holds
+ * bfhe_keyblob_size bytes; the context keeps the imported keys. */
+int bfhe_dbg_expand_keys(bfhe_ctx *, const void *compact_blob, size_t len, void *full_blob, size_t cap);
 
 /* ---- circuit evaluator: mirrors class Circuit (src/circuit.h:56-72), level-synchronous ---- */
 typedef struct bfhe_circuit bfhe_circuit;

@@ -59,6 +59,7 @@ ABI_SYMBOLS = [
     "bfhe_circuit_dump_text", "bfhe_circuit_dff_plan", "bfhe_circuit_get_schedule",
     "bfhe_circuit_exchange_mode", "bfhe_circuit_set_input_ct", "bfhe_circuit_clock_ct",
     "bfhe_import_openfhe_json", "bfhe_export_openfhe_json", "bfhe_import_openfhe_ct_json", "bfhe_export_openfhe_ct_json",
+    "bfhe_btkeygen_compact", "bfhe_keyblob_compact_size", "bfhe_export_keys_compact", "bfhe_dbg_expand_keys",
 ]
 
 _lib = None
@@ -87,6 +88,11 @@ def lib():
     L.bfhe_keyblob_size.argtypes = [vp]
     L.bfhe_export_keys.argtypes = [vp, vp, sz, C.c_int]
     L.bfhe_import_keys.argtypes = [vp, vp, sz]
+    L.bfhe_btkeygen_compact.argtypes = [vp, C.c_uint64]
+    L.bfhe_keyblob_compact_size.restype = sz
+    L.bfhe_keyblob_compact_size.argtypes = [vp]
+    L.bfhe_export_keys_compact.argtypes = [vp, vp, sz, C.c_int]
+    L.bfhe_dbg_expand_keys.argtypes = [vp, vp, sz, vp, sz]
     L.bfhe_save_keys.argtypes = [vp, C.c_char_p, C.c_int]
     L.bfhe_load_keys.argtypes = [vp, C.c_char_p]
     L.bfhe_encrypt.argtypes = [vp, vp, sz, C.c_uint64, vp]
@@ -255,7 +261,19 @@ class Context:
         self._ck(self.L.bfhe_export_keys(self.h, _ptr(buf), n, int(include_sk)))
         return buf
 
+    def btkeygen_compact(self, seed=2):
+        """btkeygen with every public mask expanded from a fresh mask seed, so that export_keys_compact can ship seed and bodies only"""
+        self._ck(self.L.bfhe_btkeygen_compact(self.h, seed))
+
+    def export_keys_compact(self, include_sk=True):
+        """the BFHEKEY2 blob (include/bfhe.h): mask seed and bodies; keys from btkeygen_compact or a BFHEKEY2 import only"""
+        n = self.L.bfhe_keyblob_compact_size(self.h)
+        buf = np.empty(n, dtype=np.uint8)
+        self._ck(self.L.bfhe_export_keys_compact(self.h, _ptr(buf), n, int(include_sk)))
+        return buf
+
     def import_keys(self, blob):
+        """a BFHEKEY1 (export_keys) or BFHEKEY2 (export_keys_compact) blob"""
         blob = np.ascontiguousarray(blob, dtype=np.uint8)
         self._ck(self.L.bfhe_import_keys(self.h, _ptr(blob), blob.size))
 
@@ -383,6 +401,14 @@ class Context:
 
     def dbg_set_gates_per_cta(self, g):
         self._ck(self.L.bfhe_dbg_set_gates_per_cta(self.h, g))
+
+    def dbg_expand_keys(self, compact_blob):
+        """import a BFHEKEY2 blob through the device expansion and return the BFHEKEY1 blob it produced"""
+        blob = np.ascontiguousarray(compact_blob, dtype=np.uint8)
+        n = self.L.bfhe_keyblob_size(self.h)
+        out = np.zeros(n, dtype=np.uint8)
+        self._ck(self.L.bfhe_dbg_expand_keys(self.h, _ptr(blob), blob.size, _ptr(out), n))
+        return out
 
     def dbg_cluster_limits(self):
         a, b = C.c_int(), C.c_int()

@@ -114,6 +114,17 @@ int launch_bk_convert(const DevConst &P, const u32 *d_coef, u32 *d_dev, size_t n
 // into the others (kernels.cu bk_fold_kernel); nsteps = n
 bool bk_fold_supported(const DevConst &P, int method_ap);
 int launch_bk_fold(const DevConst &P, const u32 *d_bk, u32 *d_bkf, size_t nsteps, void *stream);
+// key_expand.cu: the public masks of a compact key blob (include/bfhe.h) from its 256-bit mask seed.  KSK mask row r has ChaCha20 stream id r,
+// BK mask polynomial p (the p-th column-0 polynomial of the BFHEKEY1 order) has stream id BK_MASK_STREAM + p.
+struct MaskKey {
+  u32 k[8];
+};
+constexpr u64 BK_MASK_STREAM = 1ull << 40;
+// the device KSK ([i][k][j][rowlen], as ensure_device_keys lays it out) from the bodies ([N][baseKS][dKS], elem_bytes each)
+int launch_ksk_expand(const MaskKey &key, const void *d_bodies, void *d_ksk, int elem_bytes, u32 N, u32 baseKS, u32 dKS, u32 n, u32 rowlen,
+                      u32 qKS, void *stream);
+// `pairs` (mask, body) polynomial pairs of the coefficient-form BK, starting at mask polynomial p_first, into d_stage (2 * pairs * N words)
+int launch_bk_mask_expand(const MaskKey &key, const u32 *d_bodies, u32 *d_stage, u64 p_first, size_t pairs, u32 N, u32 Q, void *stream);
 int launch_dbg_ntt(const DevConst &P, const u32 *d_a, const u32 *d_b, u32 *d_rt, u32 *d_prod, int npoly, const u32 *d_twl,
                    void *stream);
 int launch_microbench(int which, u32 *d_sink, int iters, int *threads_total, int *ops_per_thread_iter, void *stream);

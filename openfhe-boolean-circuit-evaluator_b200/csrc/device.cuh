@@ -40,6 +40,36 @@ template <bool SOL = false> __device__ __forceinline__ u32 mul_shoup(u32 x, u32 
 }
 
 // ------------------------------------------------------------------------------------------
+// key-mask expansion (include/bfhe.h "compact key blob"): ChaCha20 block function (RFC 8439) with a 64-bit block counter and a 64-bit
+// nonce, as the host's Rng (hostmath.hpp), and the reduction of four keystream words, read as one little-endian 128-bit integer, mod m
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ void chacha20_block(const u32 (&key)[8], u64 nonce, u64 counter, u32 (&out)[16]) {
+  u32 x[16] = {0x61707865u, 0x3320646eu, 0x79622d32u, 0x6b206574u, key[0], key[1], key[2], key[3], key[4], key[5], key[6], key[7],
+               (u32)counter, (u32)(counter >> 32), (u32)nonce, (u32)(nonce >> 32)};
+  u32 s[16];
+#pragma unroll
+  for (int i = 0; i < 16; i++) s[i] = x[i];
+#define BFHE_DQR(a, b, c, d)                                                                                           \
+  x[a] += x[b]; x[d] = __funnelshift_l(x[d] ^ x[a], x[d] ^ x[a], 16); x[c] += x[d]; x[b] = __funnelshift_l(x[b] ^ x[c], x[b] ^ x[c], 12); \
+  x[a] += x[b]; x[d] = __funnelshift_l(x[d] ^ x[a], x[d] ^ x[a], 8);  x[c] += x[d]; x[b] = __funnelshift_l(x[b] ^ x[c], x[b] ^ x[c], 7);
+#pragma unroll
+  for (int r = 0; r < 10; r++) {
+    BFHE_DQR(0, 4, 8, 12) BFHE_DQR(1, 5, 9, 13) BFHE_DQR(2, 6, 10, 14) BFHE_DQR(3, 7, 11, 15)
+    BFHE_DQR(0, 5, 10, 15) BFHE_DQR(1, 6, 11, 12) BFHE_DQR(2, 7, 8, 13) BFHE_DQR(3, 4, 9, 14)
+  }
+#undef BFHE_DQR
+#pragma unroll
+  for (int i = 0; i < 16; i++) out[i] = x[i] + s[i];
+}
+// (w0 + w1 2^32 + w2 2^64 + w3 2^96) mod m for any m < 2^32, by Horner steps of 32 bits
+__device__ __forceinline__ u32 reduce128(u32 w0, u32 w1, u32 w2, u32 w3, u32 m) {
+  u64 r = w3 % m;
+  r = ((r << 32) | w2) % m;
+  r = ((r << 32) | w1) % m;
+  return (u32)(((r << 32) | w0) % m);
+}
+
+// ------------------------------------------------------------------------------------------
 // mbarrier, TMA bulk copy, thread-block cluster
 // ------------------------------------------------------------------------------------------
 __device__ __forceinline__ u32 smem_u32(const void *p) { return (u32)__cvta_generic_to_shared(p); }

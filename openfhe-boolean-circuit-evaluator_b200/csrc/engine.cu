@@ -276,6 +276,7 @@ extern "C" int bfhe_keygen(bfhe_ctx *c, uint64_t seed) {
   c->has_sk = true;
   c->has_bt = false;
   c->dev_keys = false;
+  c->has_mask_seed = false;
   return BFHE_OK;
 }
 
@@ -283,10 +284,70 @@ static void ksk_put(bfhe_ctx *c, u64 idx, u32 v) {
   if (c->ksk_elem_bytes == 2) reinterpret_cast<u16 *>(c->ksk.data())[idx] = (u16)v;
   else reinterpret_cast<u32 *>(c->ksk.data())[idx] = v;
 }
+static u32 elem_get(const u8 *buf, size_t idx, u32 bytes) {
+  return bytes == 2 ? reinterpret_cast<const u16 *>(buf)[idx] : reinterpret_cast<const u32 *>(buf)[idx];
+}
+static void elem_put(u8 *buf, size_t idx, u32 v, u32 bytes) {
+  if (bytes == 2) reinterpret_cast<u16 *>(buf)[idx] = (u16)v;
+  else reinterpret_cast<u32 *>(buf)[idx] = v;
+}
 
-// one RGSW ciphertext of sign * X^mm (or of 0) under z, coefficient form: rows (a, a*z + e) + m*G
+// ---- mask expansion, host implementation (key_expand.cu is the device one; the rule is stated in include/bfhe.h) ----
+// coefficients 0..count-1 of mask row `stream`: keystream words 4t..4t+3 as one little-endian 128-bit integer, mod m
+template <typename F> static void expand_mask(const MaskKey &mask, u64 stream, u32 m, size_t count, F put) {
+  SeedKey key;
+  std::memcpy(key.k, mask.k, sizeof key.k);
+  Rng r(key, stream);
+  for (size_t t = 0; t < count; t++) {
+    u128 v = r.next32();
+    for (int w = 1; w < 4; w++) v |= (u128)r.next32() << (32 * w);
+    put(t, (u32)(v % m));
+  }
+}
+static size_t ksk_rows(const bfhe_ctx *c) { return (size_t)c->p.N * c->p.baseKS * c->p.dKS; }
+static bool compact_only(const bfhe_ctx *c) { return c->bk_coef.empty() && !c->bk_body.empty(); }
+void bfhe::host_full_bk(const bfhe_ctx *c, u32 *out) {
+  if (!compact_only(c)) { std::memcpy(out, c->bk_coef.data(), c->bk_words * 4); return; }
+  const size_t N = c->p.N;
+#pragma omp parallel for schedule(static)
+  for (i64 s = 0; s < (i64)(c->bk_words / (2 * N)); s++) {
+    u32 *a = out + 2 * (size_t)s * N;
+    expand_mask(c->mask_seed, BK_MASK_STREAM + (u64)s, (u32)c->p.Q, N, [&](size_t t, u32 v) { a[t] = v; });
+    std::memcpy(a + N, c->bk_body.data() + (size_t)s * N, N * 4);
+  }
+}
+void bfhe::host_full_ksk(const bfhe_ctx *c, u8 *out) {
+  if (!compact_only(c)) { std::memcpy(out, c->ksk.data(), c->ksk_elems * c->ksk_elem_bytes); return; }
+  const u32 n = c->p.n, eb = c->ksk_elem_bytes;
+#pragma omp parallel for schedule(static)
+  for (i64 r = 0; r < (i64)ksk_rows(c); r++) {
+    const size_t base = (size_t)r * (n + 1);
+    expand_mask(c->mask_seed, (u64)r, (u32)c->p.qKS, n, [&](size_t t, u32 v) { elem_put(out, base + t, v, eb); });
+    elem_put(out, base + n, elem_get(c->ksk_body.data(), (size_t)r, eb), eb);
+  }
+}
+static void clear_compact(bfhe_ctx *c) {
+  c->has_mask_seed = false;
+  std::vector<u32>().swap(c->bk_body);
+  std::vector<u8>().swap(c->ksk_body);
+}
+void bfhe::forget_mask_seed(bfhe_ctx *c) {
+  if (c->has_bt && compact_only(c)) {
+    std::vector<u32> bk(c->bk_words);
+    std::vector<u8> ksk(c->ksk_elems * c->ksk_elem_bytes);
+    host_full_bk(c, bk.data());
+    host_full_ksk(c, ksk.data());
+    c->bk_coef.swap(bk);
+    c->ksk.swap(ksk);
+  }
+  clear_compact(c);
+}
+
+// one RGSW ciphertext of sign * X^mm (or of 0) under z, coefficient form: rows (a, a*z + e) + m*G.
+// mask != nullptr: every a is the expansion of mask row BK_MASK_STREAM + p0 + row, and an even row, whose message would otherwise sit in
+// the public a, carries it in the body as -m*g^l*z instead (the same phase b - a*z = e - m*g^l*z)
 static void rgsw_encrypt(const bfhe_ctx *c, const std::vector<u32> &z_eval, bool msg, u32 mm, int sign, const SeedKey &seed, u64 stream,
-                         u32 *out) {
+                         u32 *out, const MaskKey *mask = nullptr, u64 p0 = 0) {
   const u32 N = c->p.N, rows = 2 * c->p.dG;
   const u32 Q = (u32)c->p.Q;
   Rng r(seed, stream);
@@ -294,7 +355,8 @@ static void rgsw_encrypt(const bfhe_ctx *c, const std::vector<u32> &z_eval, bool
   u64 gpow = 1;
   for (u32 row = 0; row < rows; row++) {
     u32 *a = out + ((size_t)row * 2 + 0) * N, *b = out + ((size_t)row * 2 + 1) * N;
-    for (u32 j = 0; j < N; j++) a[j] = (u32)r.uniform(Q);
+    if (mask) expand_mask(*mask, BK_MASK_STREAM + p0 + row, Q, N, [&](size_t t, u32 v) { a[t] = v; });
+    else for (u32 j = 0; j < N; j++) a[j] = (u32)r.uniform(Q);
     std::copy(a, a + N, tmp.begin());
     c->hntt.fwd(tmp.data());
     for (u32 j = 0; j < N; j++) tmp[j] = (u32)((u64)tmp[j] * z_eval[j] % Q);
@@ -303,7 +365,13 @@ static void rgsw_encrypt(const bfhe_ctx *c, const std::vector<u32> &z_eval, bool
       i64 e = gauss_table().sample(r);
       b[j] = (u32)(((i64)tmp[j] + e + Q) % Q);
     }
-    if (msg) {
+    if (msg && mask && !(row & 1)) { // b -= sign * g * X^mm * z  (negacyclic: X^N = -1)
+      const i64 g = (i64)(gpow % Q);
+      for (u32 j = 0; j < N; j++) {
+        const i64 zj = j >= mm ? c->z[j - mm] : -(i64)c->z[j + N - mm];
+        b[j] = (u32)((((i64)b[j] - sign * g * zj) % Q + Q) % Q);
+      }
+    } else if (msg) {
       u32 g = (u32)(gpow % Q);
       u32 *dst = (row & 1) ? b : a;
       dst[mm] = sign > 0 ? (u32)(((u64)dst[mm] + g) % Q) : (u32)(((u64)dst[mm] + Q - g) % Q);
@@ -312,7 +380,8 @@ static void rgsw_encrypt(const bfhe_ctx *c, const std::vector<u32> &z_eval, bool
   }
 }
 
-extern "C" int bfhe_btkeygen(bfhe_ctx *c, uint64_t seed64) {
+// BTKeyGen; mask != nullptr: every mask is the expansion of that public seed (bfhe_btkeygen_compact)
+static int btkeygen(bfhe_ctx *c, uint64_t seed64, const MaskKey *mask) {
   if (!c) return BFHE_ERR_ARG;
   if (!c->has_sk) { set_error("BTKeyGen before KeyGen"); return BFHE_ERR_STATE; }
   const bfhe_params &p = c->p;
@@ -336,12 +405,16 @@ extern "C" int bfhe_btkeygen(bfhe_ctx *c, uint64_t seed64) {
     Rng r(seed, 0x100000 + (u64)i);
     for (u32 j = 0; j < p.baseKS; j++)
       for (u32 k = 0; k < p.dKS; k++) {
-        const u64 base = (((u64)i * p.baseKS + j) * p.dKS + k) * (n + 1);
+        const u64 row = ((u64)i * p.baseKS + j) * p.dKS + k, base = row * (n + 1);
         i64 b = gauss_table().sample(r) + (i64)c->z[i] * (i64)((u64)j * Bpow[k] % qKS);
-        for (u32 t = 0; t < n; t++) {
-          u64 a = r.uniform(qKS);
-          ksk_put(c, base + t, (u32)a);
-          b += (i64)a * c->sk[t];
+        if (mask) {
+          expand_mask(*mask, row, (u32)qKS, n, [&](size_t t, u32 a) { ksk_put(c, base + t, a); b += (i64)a * c->sk[t]; });
+        } else {
+          for (u32 t = 0; t < n; t++) {
+            u64 a = r.uniform(qKS);
+            ksk_put(c, base + t, (u32)a);
+            b += (i64)a * c->sk[t];
+          }
         }
         b %= (i64)qKS;
         if (b < 0) b += qKS;
@@ -354,8 +427,10 @@ extern "C" int bfhe_btkeygen(bfhe_ctx *c, uint64_t seed64) {
   if (p.method == BFHE_GINX) { // ek[i] = (RGSW(s_i == 1), RGSW(s_i == -1))
 #pragma omp parallel for schedule(dynamic, 4)
     for (i64 i = 0; i < (i64)n; i++) {
-      rgsw_encrypt(c, z_eval, c->sk[i] == 1, 0, +1, seed, 0x200000 + 2 * (u64)i, c->bk_coef.data() + ((size_t)i * 2 + 0) * rw);
-      rgsw_encrypt(c, z_eval, c->sk[i] == -1, 0, +1, seed, 0x200000 + 2 * (u64)i + 1, c->bk_coef.data() + ((size_t)i * 2 + 1) * rw);
+      rgsw_encrypt(c, z_eval, c->sk[i] == 1, 0, +1, seed, 0x200000 + 2 * (u64)i, c->bk_coef.data() + ((size_t)i * 2 + 0) * rw, mask,
+                   ((u64)i * 2 + 0) * 2 * p.dG);
+      rgsw_encrypt(c, z_eval, c->sk[i] == -1, 0, +1, seed, 0x200000 + 2 * (u64)i + 1, c->bk_coef.data() + ((size_t)i * 2 + 1) * rw, mask,
+                   ((u64)i * 2 + 1) * 2 * p.dG);
     }
   } else { // ek[i][j][k] = RGSW(X^{(s_i * j * Br^k mod q) * 2N/q}), j in [1, Br)
     const i64 total = (i64)n * (p.baseR - 1) * p.dR;
@@ -368,39 +443,70 @@ extern "C" int bfhe_btkeygen(bfhe_ctx *c, uint64_t seed64) {
       i64 mm = (((m % (i64)p.q) + p.q) % p.q) * (2 * N / p.q);
       int sign = 1;
       if (mm >= (i64)N) { mm -= N; sign = -1; }
-      rgsw_encrypt(c, z_eval, true, (u32)mm, sign, seed, 0x300000 + (u64)t, c->bk_coef.data() + (size_t)t * rw);
+      rgsw_encrypt(c, z_eval, true, (u32)mm, sign, seed, 0x300000 + (u64)t, c->bk_coef.data() + (size_t)t * rw, mask, (u64)t * 2 * p.dG);
     }
   }
   c->z.clear();
+  clear_compact(c);
+  if (mask) { c->has_mask_seed = true; c->mask_seed = *mask; }
   c->has_bt = true;
   c->dev_keys = false;
   if (c->device >= 0) return ensure_device_keys(c);
   return BFHE_OK;
 }
 
-// upload: BK through the conversion kernel, KSK re-laid-out as [i][k][digit][row]
-int bfhe::ensure_device_keys(bfhe_ctx *c) {
+extern "C" int bfhe_btkeygen(bfhe_ctx *c, uint64_t seed64) { return btkeygen(c, seed64, nullptr); }
+
+extern "C" int bfhe_btkeygen_compact(bfhe_ctx *c, uint64_t seed64) {
+  if (!c) return BFHE_ERR_ARG;
+  if (!c->has_sk) { set_error("BTKeyGen before KeyGen"); return BFHE_ERR_STATE; }
+  MaskKey mask;
+  if (seed64 == 0) { // independent of the secret stream
+    if (!SeedKey::os_entropy(mask.k, sizeof mask.k)) { set_error("cannot read OS entropy (getrandom and /dev/urandom both failed)"); return BFHE_ERR_IO; }
+  } else { // reproducible: a stream of its own under the secret SeedKey (ChaCha20 output reveals nothing about the key)
+    SeedKey seed;
+    if (int rc = make_seed_key(seed64, seed)) return rc;
+    Rng r(seed, 0x4D41534B);
+    for (auto &w : mask.k) w = r.next32();
+  }
+  return btkeygen(c, seed64, &mask);
+}
+
+// upload: BK through the conversion kernel, KSK re-laid-out as [i][k][digit][row].  Keys held as mask seed + bodies (compact_only) have
+// their masks generated on the device, into the same coefficient-form staging buffer and straight into the device KSK.  dbg_bk / dbg_ksk
+// (bfhe_dbg_expand_keys, compact keys only): receive the staging buffer and the device KSK, in the BFHEKEY1 layouts.
+static int upload_keys(bfhe_ctx *c, u32 *dbg_bk, u8 *dbg_ksk) {
   if (c->dev_keys) return BFHE_OK;
   if (c->device < 0) { set_error("no CUDA device attached (this engine has no CPU fallback)"); return BFHE_ERR_CUDA; }
   if (!c->has_bt) { set_error("bootstrapping keys missing: call bfhe_btkeygen or bfhe_import_keys first"); return BFHE_ERR_STATE; }
   BFHE_CUDA(cudaSetDevice(c->device));
   const bfhe_params &p = c->p;
   const u32 N = p.N;
+  const bool compact = compact_only(c);
   cudaFree(c->d_bk); c->d_bk = nullptr;
   cudaFree(c->d_ksk); c->d_ksk = nullptr;
   BFHE_CUDA(cudaMalloc(&c->d_bk, c->bk_words * 4));
   { // convert in slices so the temporary coefficient-form copy stays small
-    const size_t npoly = c->bk_words / N, slice = 1 << 15;
-    u32 *d_coef = nullptr;
+    const size_t npoly = c->bk_words / N, slice = 1 << 15; // even: a slice holds whole (mask, body) pairs
+    u32 *d_coef = nullptr, *d_body = nullptr;
     BFHE_CUDA(cudaMalloc(&d_coef, std::min(npoly, slice) * N * 4));
+    if (compact) BFHE_CUDA(cudaMalloc(&d_body, std::min(npoly, slice) / 2 * N * 4));
     for (size_t p0 = 0; p0 < npoly; p0 += slice) {
       const size_t np = std::min(slice, npoly - p0);
-      BFHE_CUDA(cudaMemcpyAsync(d_coef, c->bk_coef.data() + p0 * N, np * N * 4, cudaMemcpyHostToDevice, c->stream));
+      if (compact) {
+        BFHE_CUDA(cudaMemcpyAsync(d_body, c->bk_body.data() + p0 / 2 * N, np / 2 * N * 4, cudaMemcpyHostToDevice, c->stream));
+        int rc = launch_bk_mask_expand(c->mask_seed, d_body, d_coef, p0 / 2, np / 2, N, (u32)p.Q, c->stream);
+        if (rc) return cuda_fail((cudaError_t)rc, "bk_mask_expand");
+        if (dbg_bk) BFHE_CUDA(cudaMemcpyAsync(dbg_bk + p0 * N, d_coef, np * N * 4, cudaMemcpyDeviceToHost, c->stream));
+      } else {
+        BFHE_CUDA(cudaMemcpyAsync(d_coef, c->bk_coef.data() + p0 * N, np * N * 4, cudaMemcpyHostToDevice, c->stream));
+      }
       int rc = launch_bk_convert(c->P, d_coef, c->d_bk + p0 * N, np, c->d_twl, c->stream);
       if (rc) return cuda_fail((cudaError_t)rc, "bk_convert");
       BFHE_CUDA(cudaStreamSynchronize(c->stream));
     }
     cudaFree(d_coef);
+    cudaFree(d_body);
   }
   cudaFree(c->d_bk4); c->d_bk4 = nullptr; c->v2.d_bk4 = nullptr;
   if (c->d_tw2 && v2_supported(c->P, p.method == BFHE_AP)) { // key copy of the 2-CTA cluster kernel: kernels_v2.cu's physical slot order
@@ -434,22 +540,42 @@ int bfhe::ensure_device_keys(bfhe_ctx *c) {
   { // KSK: [i][j(digit value)][k(digit index)][n+1]  ->  [i][k][j][rowlen]
     const u32 rowlen = c->ksk_elem_bytes == 2 ? 512 : p.ct_stride; // elements per padded row
     if (c->ksk_elem_bytes == 2 && p.n + 1 > 512) { set_error("LWE dimension too large for the packed key-switch kernel"); return BFHE_ERR_ARG; }
-    const size_t rows = (size_t)N * p.baseKS * p.dKS, bytes = rows * rowlen * c->ksk_elem_bytes;
-    std::vector<u8> dev(bytes, 0);
+    const size_t rows = ksk_rows(c), bytes = rows * rowlen * c->ksk_elem_bytes;
     const size_t src_row = (size_t)(p.n + 1) * c->ksk_elem_bytes, dst_row = (size_t)rowlen * c->ksk_elem_bytes;
+    auto relayout = [&](u8 *full, u8 *dev, bool to_dev) { // full [i][j][k][n+1] <-> device [i][k][j][rowlen]
 #pragma omp parallel for schedule(static)
-    for (i64 i = 0; i < (i64)N; i++)
-      for (u32 j = 0; j < p.baseKS; j++)
-        for (u32 k = 0; k < p.dKS; k++) {
-          const size_t s = (((size_t)i * p.baseKS + j) * p.dKS + k), d = (((size_t)i * p.dKS + k) * p.baseKS + j);
-          std::memcpy(dev.data() + d * dst_row, c->ksk.data() + s * src_row, src_row);
-        }
+      for (i64 i = 0; i < (i64)N; i++)
+        for (u32 j = 0; j < p.baseKS; j++)
+          for (u32 k = 0; k < p.dKS; k++) {
+            const size_t s = (((size_t)i * p.baseKS + j) * p.dKS + k), d = (((size_t)i * p.dKS + k) * p.baseKS + j);
+            if (to_dev) std::memcpy(dev + d * dst_row, full + s * src_row, src_row);
+            else std::memcpy(full + s * src_row, dev + d * dst_row, src_row);
+          }
+    };
     BFHE_CUDA(cudaMalloc(&c->d_ksk, bytes));
-    BFHE_CUDA(cudaMemcpy(c->d_ksk, dev.data(), bytes, cudaMemcpyHostToDevice));
+    if (compact) {
+      void *d_kb = nullptr;
+      BFHE_CUDA(cudaMalloc(&d_kb, c->ksk_body.size()));
+      BFHE_CUDA(cudaMemcpyAsync(d_kb, c->ksk_body.data(), c->ksk_body.size(), cudaMemcpyHostToDevice, c->stream));
+      int rc = launch_ksk_expand(c->mask_seed, d_kb, c->d_ksk, c->ksk_elem_bytes, N, p.baseKS, p.dKS, p.n, rowlen, (u32)p.qKS, c->stream);
+      if (rc) { cudaFree(d_kb); return cuda_fail((cudaError_t)rc, "ksk_expand"); }
+      BFHE_CUDA(cudaStreamSynchronize(c->stream));
+      cudaFree(d_kb);
+      if (dbg_ksk) {
+        std::vector<u8> dev(bytes);
+        BFHE_CUDA(cudaMemcpy(dev.data(), c->d_ksk, bytes, cudaMemcpyDeviceToHost));
+        relayout(dbg_ksk, dev.data(), false);
+      }
+    } else {
+      std::vector<u8> dev(bytes, 0);
+      relayout(c->ksk.data(), dev.data(), true);
+      BFHE_CUDA(cudaMemcpy(c->d_ksk, dev.data(), bytes, cudaMemcpyHostToDevice));
+    }
   }
   c->dev_keys = true;
   return BFHE_OK;
 }
+int bfhe::ensure_device_keys(bfhe_ctx *c) { return upload_keys(c, nullptr, nullptr); }
 
 // -------------------------------------------------------------------------------------------------
 // key blob
@@ -458,32 +584,100 @@ extern "C" size_t bfhe_keyblob_size(const bfhe_ctx *c) {
   if (!c) return 0;
   return sizeof(KeyBlobHeader) + pad8((size_t)c->p.n * 4) + pad8(c->bk_words * 4) + pad8(c->ksk_elems * c->ksk_elem_bytes);
 }
-extern "C" int bfhe_export_keys(const bfhe_ctx *c, void *buf, size_t cap, int include_sk) {
-  if (!c || !buf) return BFHE_ERR_ARG;
-  if (!c->has_bt) { set_error("no keys to export"); return BFHE_ERR_STATE; }
-  if (cap < bfhe_keyblob_size(c)) { set_error("export buffer too small"); return BFHE_ERR_ARG; }
+extern "C" size_t bfhe_keyblob_compact_size(const bfhe_ctx *c) {
+  if (!c) return 0;
+  return sizeof(KeyBlobHeader) + sizeof(MaskKey) + pad8((size_t)c->p.n * 4) + pad8(c->bk_words / 2 * 4) + pad8(ksk_rows(c) * c->ksk_elem_bytes);
+}
+// header (BFHEKEY1 / BFHEKEY2) and, for BFHEKEY2, the mask seed, then the sk section; returns the first byte after it
+static u8 *put_header(const bfhe_ctx *c, u8 *o, bool compact, bool include_sk) {
   KeyBlobHeader h{};
-  std::memcpy(h.magic, "BFHEKEY1", 8);
+  std::memcpy(h.magic, compact ? "BFHEKEY2" : "BFHEKEY1", 8);
   const bfhe_params &p = c->p;
   h.version = 1; h.paramset = p.paramset; h.method = p.method; h.n = p.n; h.N = p.N; h.q = p.q;
   h.baseKS = p.baseKS; h.dKS = p.dKS; h.baseG = p.baseG; h.dG = p.dG; h.baseR = p.baseR; h.dR = p.dR;
   h.has_sk = (include_sk && c->has_sk) ? 1 : 0; h.ksk_elem_bytes = c->ksk_elem_bytes;
   h.Q = p.Q; h.qKS = p.qKS; h.bk_words = c->bk_words; h.ksk_elems = c->ksk_elems;
-  u8 *o = (u8 *)buf;
   std::memcpy(o, &h, sizeof h); o += sizeof h;
+  if (compact) { std::memcpy(o, &c->mask_seed, sizeof c->mask_seed); o += sizeof c->mask_seed; }
   std::memset(o, 0, pad8((size_t)p.n * 4));
   if (h.has_sk) std::memcpy(o, c->sk.data(), (size_t)p.n * 4);
-  o += pad8((size_t)p.n * 4);
-  std::memcpy(o, c->bk_coef.data(), c->bk_words * 4); o += pad8(c->bk_words * 4);
-  std::memcpy(o, c->ksk.data(), c->ksk_elems * c->ksk_elem_bytes);
+  return o + pad8((size_t)p.n * 4);
+}
+extern "C" int bfhe_export_keys(const bfhe_ctx *c, void *buf, size_t cap, int include_sk) {
+  if (!c || !buf) return BFHE_ERR_ARG;
+  if (!c->has_bt) { set_error("no keys to export"); return BFHE_ERR_STATE; }
+  if (cap < bfhe_keyblob_size(c)) { set_error("export buffer too small"); return BFHE_ERR_ARG; }
+  u8 *o = put_header(c, (u8 *)buf, false, include_sk);
+  host_full_bk(c, (u32 *)o); o += pad8(c->bk_words * 4);
+  host_full_ksk(c, o);
   return BFHE_OK;
 }
-extern "C" int bfhe_import_keys(bfhe_ctx *c, const void *buf, size_t len) {
+extern "C" int bfhe_export_keys_compact(const bfhe_ctx *c, void *buf, size_t cap, int include_sk) {
   if (!c || !buf) return BFHE_ERR_ARG;
-  KeyBlobHeader h;
+  if (!c->has_bt) { set_error("no keys to export"); return BFHE_ERR_STATE; }
+  if (!c->has_mask_seed) { set_error("these keys have no mask seed (made by bfhe_btkeygen or imported in full): only bfhe_export_keys can export them"); return BFHE_ERR_STATE; }
+  if (cap < bfhe_keyblob_compact_size(c)) { set_error("export buffer too small"); return BFHE_ERR_ARG; }
+  u8 *o = put_header(c, (u8 *)buf, true, include_sk);
+  const size_t N = c->p.N, pairs = c->bk_words / (2 * N), rows = ksk_rows(c);
+  const u32 n = c->p.n, eb = c->ksk_elem_bytes;
+  u32 *bk = (u32 *)o;
+  u8 *ksk = o + pad8(pairs * N * 4);
+  if (compact_only(c)) {
+    std::memcpy(bk, c->bk_body.data(), pairs * N * 4);
+    std::memcpy(ksk, c->ksk_body.data(), rows * eb);
+  } else {
+    for (size_t s = 0; s < pairs; s++) std::memcpy(bk + s * N, c->bk_coef.data() + (2 * s + 1) * N, N * 4);
+    for (size_t r = 0; r < rows; r++) elem_put(ksk, r, elem_get(c->ksk.data(), r * (n + 1) + n, eb), eb);
+  }
+  std::memset(bk + pairs * N, 0, pad8(pairs * N * 4) - pairs * N * 4);
+  std::memset(ksk + rows * eb, 0, pad8(rows * eb) - rows * eb);
+  return BFHE_OK;
+}
+
+// BFHEKEY2 import: every check before the context changes; dbg_bk / dbg_ksk as upload_keys
+static int import_compact(bfhe_ctx *c, const KeyBlobHeader &h, const u8 *buf, size_t len, u32 *dbg_bk, u8 *dbg_ksk) {
+  if (len < bfhe_keyblob_compact_size(c)) { set_error("BFHEKEY2 key blob truncated"); return BFHE_ERR_FORMAT; }
+  const bfhe_params &p = c->p;
+  const size_t N = p.N, pairs = c->bk_words / (2 * N), rows = ksk_rows(c);
+  const u32 eb = c->ksk_elem_bytes;
+  MaskKey mask;
+  const u8 *in = buf + sizeof h;
+  std::memcpy(&mask, in, sizeof mask); in += sizeof mask;
+  const u8 *sk = in; in += pad8((size_t)p.n * 4);
+  const u32 *bk = (const u32 *)in; in += pad8(pairs * N * 4);
+  const u8 *ksk = in;
+  for (size_t i = 0; i < pairs * N; i++)
+    if (bk[i] >= p.Q) { set_error("BFHEKEY2: BK body word " + std::to_string(i) + " = " + std::to_string(bk[i]) + " is not below Q"); return BFHE_ERR_FORMAT; }
+  for (size_t i = 0; i < rows; i++)
+    if (elem_get(ksk, i, eb) >= p.qKS) {
+      set_error("BFHEKEY2: KSK body word " + std::to_string(i) + " = " + std::to_string(elem_get(ksk, i, eb)) + " is not below qKS");
+      return BFHE_ERR_FORMAT;
+    }
+  if (h.has_sk) { c->sk.resize(p.n); std::memcpy(c->sk.data(), sk, (size_t)p.n * 4); c->has_sk = true; }
+  c->has_mask_seed = true;
+  c->mask_seed = mask;
+  c->bk_body.assign(bk, bk + pairs * N);
+  c->ksk_body.assign(ksk, ksk + rows * eb);
+  std::vector<u32>().swap(c->bk_coef); // compact_only from here on
+  std::vector<u8>().swap(c->ksk);
+  c->has_bt = true;
+  c->dev_keys = false;
+  if (c->device >= 0) return upload_keys(c, dbg_bk, dbg_ksk);
+  std::vector<u32> full_bk(c->bk_words); // host-only context: the full forms, as after bfhe_btkeygen_compact
+  std::vector<u8> full_ksk(c->ksk_elems * eb);
+  host_full_bk(c, full_bk.data());
+  host_full_ksk(c, full_ksk.data());
+  c->bk_coef.swap(full_bk);
+  c->ksk.swap(full_ksk);
+  std::vector<u32>().swap(c->bk_body);
+  std::vector<u8>().swap(c->ksk_body);
+  return BFHE_OK;
+}
+static int read_header(const bfhe_ctx *c, const void *buf, size_t len, KeyBlobHeader &h, bool &compact) {
   if (len < sizeof h) { set_error("key blob truncated"); return BFHE_ERR_FORMAT; }
   std::memcpy(&h, buf, sizeof h);
-  if (std::memcmp(h.magic, "BFHEKEY1", 8) || h.version != 1) { set_error("not a BFHEKEY1 blob"); return BFHE_ERR_FORMAT; }
+  compact = !std::memcmp(h.magic, "BFHEKEY2", 8);
+  if ((!compact && std::memcmp(h.magic, "BFHEKEY1", 8)) || h.version != 1) { set_error("not a BFHEKEY1 or BFHEKEY2 blob"); return BFHE_ERR_FORMAT; }
   const bfhe_params &p = c->p;
   if (h.paramset != p.paramset || h.method != p.method || h.n != p.n || h.N != p.N || h.q != p.q || h.Q != p.Q || h.qKS != p.qKS ||
       h.baseKS != p.baseKS || h.dKS != p.dKS || h.baseG != p.baseG || h.dG != p.dG || h.baseR != p.baseR || h.dR != p.dR ||
@@ -491,7 +685,16 @@ extern "C" int bfhe_import_keys(bfhe_ctx *c, const void *buf, size_t len) {
     set_error("key blob parameters do not match this context");
     return BFHE_ERR_FORMAT;
   }
+  return BFHE_OK;
+}
+extern "C" int bfhe_import_keys(bfhe_ctx *c, const void *buf, size_t len) {
+  if (!c || !buf) return BFHE_ERR_ARG;
+  KeyBlobHeader h;
+  bool compact = false;
+  if (int rc = read_header(c, buf, len, h, compact)) return rc;
+  if (compact) return import_compact(c, h, (const u8 *)buf, len, nullptr, nullptr);
   if (len < bfhe_keyblob_size(c)) { set_error("key blob truncated"); return BFHE_ERR_FORMAT; }
+  const bfhe_params &p = c->p;
   const u8 *in = (const u8 *)buf + sizeof h;
   if (h.has_sk) { c->sk.resize(p.n); std::memcpy(c->sk.data(), in, (size_t)p.n * 4); c->has_sk = true; }
   in += pad8((size_t)p.n * 4);
@@ -499,9 +702,24 @@ extern "C" int bfhe_import_keys(bfhe_ctx *c, const void *buf, size_t len) {
   std::memcpy(c->bk_coef.data(), in, c->bk_words * 4); in += pad8(c->bk_words * 4);
   c->ksk.resize(c->ksk_elems * c->ksk_elem_bytes);
   std::memcpy(c->ksk.data(), in, c->ksk.size());
+  clear_compact(c);
   c->has_bt = true;
   c->dev_keys = false;
   if (c->device >= 0) return ensure_device_keys(c);
+  return BFHE_OK;
+}
+extern "C" int bfhe_dbg_expand_keys(bfhe_ctx *c, const void *compact_blob, size_t len, void *full_blob, size_t cap) {
+  if (!c || !compact_blob || !full_blob) return BFHE_ERR_ARG;
+  if (c->device < 0) { set_error("no CUDA device attached (bfhe_dbg_expand_keys runs the device expansion)"); return BFHE_ERR_CUDA; }
+  if (cap < bfhe_keyblob_size(c)) { set_error("expansion buffer too small"); return BFHE_ERR_ARG; }
+  KeyBlobHeader h;
+  bool compact = false;
+  if (int rc = read_header(c, compact_blob, len, h, compact)) return rc;
+  if (!compact) { set_error("not a BFHEKEY2 blob"); return BFHE_ERR_FORMAT; }
+  u8 *bk = (u8 *)full_blob + sizeof h + pad8((size_t)c->p.n * 4), *ksk = bk + pad8(c->bk_words * 4);
+  if (int rc = import_compact(c, h, (const u8 *)compact_blob, len, (u32 *)bk, ksk)) return rc;
+  put_header(c, (u8 *)full_blob, false, h.has_sk != 0);
+  std::memset(bk + c->bk_words * 4, 0, pad8(c->bk_words * 4) - c->bk_words * 4);
   return BFHE_OK;
 }
 extern "C" int bfhe_save_keys(const bfhe_ctx *c, const char *path, int include_sk) {

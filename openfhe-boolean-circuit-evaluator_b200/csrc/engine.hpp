@@ -40,6 +40,12 @@ struct bfhe_ctx {
   bool ofhe_have_bk = false, ofhe_have_ksk = false; // halves of the bootstrapping key imported from OpenFHE JSON (host/openfhe_json.cpp)
   std::vector<bfhe::u32> bk_coef;
   std::vector<bfhe::u8> ksk; // [N][baseKS][dKS][n+1], ksk_elem_bytes each
+  // keys whose masks are the expansion of a public mask seed (bfhe_btkeygen_compact, BFHEKEY2 import).  A device context that imported
+  // BFHEKEY2 keeps only the bodies here (bk_coef / ksk empty); the full forms are expanded on the host when an export asks for them.
+  bool has_mask_seed = false;
+  bfhe::MaskKey mask_seed{};
+  std::vector<bfhe::u32> bk_body; // column-1 polynomials of bk_coef, BFHEKEY1 order
+  std::vector<bfhe::u8> ksk_body; // [N][baseKS][dKS], ksk_elem_bytes each
   bfhe::u32 ksk_elem_bytes = 4;
   bfhe::u64 bk_words = 0, ksk_elems = 0;
 
@@ -86,6 +92,11 @@ namespace bfhe {
 // run one list of single-bootstrap gates (device pointers already resolved) through blind rotation + key switch
 int run_gate_list(bfhe_ctx *c, const DevGate *host_list, size_t count, u32 *acc_dbg_host);
 int ensure_device_keys(bfhe_ctx *c);
+// full coefficient-form BK / [N][baseKS][dKS][n+1] KSK of the context's keys: bk_coef / ksk, or expanded from the mask seed and the bodies
+void host_full_bk(const bfhe_ctx *c, u32 *out);
+void host_full_ksk(const bfhe_ctx *c, u8 *out);
+// the keys stop being the expansion of a mask seed (some of them are replaced): full host forms, no seed, no bodies
+void forget_mask_seed(bfhe_ctx *c);
 // EvalNOT of in[i] into out[i] through the context's pointer buffers (low bit of in[i] set: plain copy); caller holds c->mtx
 int not_ptr_batch(bfhe_ctx *c, const std::vector<const u32 *> &in, const std::vector<u32 *> &out);
 } // namespace bfhe

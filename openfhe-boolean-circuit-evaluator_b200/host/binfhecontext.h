@@ -57,6 +57,8 @@ public:
     return std::make_shared<LWEPrivateKeyImpl>();
   }
   void BTKeyGen(ConstLWEPrivateKey, uint64_t seed = 0) { check(bfhe_btkeygen(raw(), seed)); }
+  // BTKeyGen with every public mask expanded from a fresh mask seed, so that ExportKeys(..., true) ships seed and bodies only
+  void BTKeyGenCompact(ConstLWEPrivateKey, uint64_t seed = 0) { check(bfhe_btkeygen_compact(raw(), seed)); }
   LWECiphertext Encrypt(ConstLWEPrivateKey, const LWEPlaintext &m, BINFHE_OUTPUT output = BOOTSTRAPPED) const {
     auto ct = std::make_shared<LWECiphertextImpl>();
     ct->row.resize(m_p.ct_stride);
@@ -77,12 +79,15 @@ public:
   }
   LWECiphertext Bootstrap(ConstLWECiphertext ct) const { return one_gate(BFHE_BOOTSTRAP, ct, ct); }
 
-  // the key blob of bfhe_export_keys (include/bfhe.h): without the secret key it is what an evaluator needs, and all it gets
-  std::vector<uint8_t> ExportKeys(bool include_sk) const {
-    std::vector<uint8_t> blob(bfhe_keyblob_size(raw()));
-    check(bfhe_export_keys(raw(), blob.data(), blob.size(), include_sk ? 1 : 0));
+  // the key blob of bfhe_export_keys (include/bfhe.h): without the secret key it is what an evaluator needs, and all it gets.
+  // compact: the BFHEKEY2 blob of bfhe_export_keys_compact (keys from BTKeyGenCompact or a compact import only)
+  std::vector<uint8_t> ExportKeys(bool include_sk, bool compact = false) const {
+    std::vector<uint8_t> blob(compact ? bfhe_keyblob_compact_size(raw()) : bfhe_keyblob_size(raw()));
+    check(compact ? bfhe_export_keys_compact(raw(), blob.data(), blob.size(), include_sk ? 1 : 0)
+                  : bfhe_export_keys(raw(), blob.data(), blob.size(), include_sk ? 1 : 0));
     return blob;
   }
+  // either blob
   void ImportKeys(const std::vector<uint8_t> &blob) { check(bfhe_import_keys(raw(), blob.data(), blob.size())); }
 
   bfhe_ctx *raw() const {

@@ -264,6 +264,7 @@ extern "C" int bfhe_import_openfhe_json(bfhe_ctx *c, int what, const char *path)
     const size_t nkeys = polys.size() / per_key;
     const size_t want = p.method == BFHE_GINX ? (size_t)2 * p.n : (size_t)p.n * (p.baseR - 1) * p.dR;
     if (nkeys != want) return fmt_err("refresh key: " + std::to_string(nkeys) + " RGSW ciphertexts, expected " + std::to_string(want));
+    forget_mask_seed(c);
     c->bk_coef.assign(c->bk_words, 0);
     std::vector<u64> v;
     std::vector<u32> tmp(N);
@@ -289,6 +290,7 @@ extern "C" int bfhe_import_openfhe_json(bfhe_ctx *c, int what, const char *path)
     std::vector<const JVal *> cts;
     collect(root.get(), is_ct, cts);
     const size_t want = (size_t)p.N * p.baseKS * p.dKS;
+    forget_mask_seed(c);
     c->ksk.assign(c->ksk_elems * c->ksk_elem_bytes, 0);
     auto put = [&](size_t idx, u64 val) {
       if (c->ksk_elem_bytes == 2) reinterpret_cast<u16 *>(c->ksk.data())[idx] = (u16)val;
@@ -347,7 +349,8 @@ extern "C" int bfhe_export_openfhe_json(const bfhe_ctx *c, int what, const char 
   } else if (what == BFHE_OFHE_REFRESH_KEY) {
     const u32 N = p.N, rows = 2 * p.dG;
     const size_t per_key = (size_t)rows * 2;
-    std::vector<u32> tmp(N);
+    std::vector<u32> tmp(N), bk(c->bk_words);
+    host_full_bk(c, bk.data());
     v.resize(N);
     u32 id = 2;
     auto rgsw = [&](size_t src) { // shared_ptr<RingGSWEvalKeyImpl>
@@ -355,7 +358,7 @@ extern "C" int bfhe_export_openfhe_json(const bfhe_ctx *c, int what, const char 
       for (u32 r = 0; r < rows; r++) {
         o.s(r ? ",[" : "[");
         for (u32 cc = 0; cc < 2; cc++) {
-          std::memcpy(tmp.data(), c->bk_coef.data() + (src * per_key + (size_t)r * 2 + cc) * N, (size_t)N * 4);
+          std::memcpy(tmp.data(), bk.data() + (src * per_key + (size_t)r * 2 + cc) * N, (size_t)N * 4);
           c->hntt.fwd(tmp.data()); // EVALUATION format, as BTKeyGen leaves it
           for (u32 j = 0; j < N; j++) v[j] = tmp[j];
           if (cc) o.s(",");
@@ -392,8 +395,10 @@ extern "C" int bfhe_export_openfhe_json(const bfhe_ctx *c, int what, const char 
     }
     o.s("]");
   } else if (what == BFHE_OFHE_SWITCH_KEY) {
+    std::vector<u8> ksk(c->ksk_elems * c->ksk_elem_bytes);
+    host_full_ksk(c, ksk.data());
     auto get = [&](size_t idx) -> u64 {
-      return c->ksk_elem_bytes == 2 ? reinterpret_cast<const u16 *>(c->ksk.data())[idx] : reinterpret_cast<const u32 *>(c->ksk.data())[idx];
+      return c->ksk_elem_bytes == 2 ? reinterpret_cast<const u16 *>(ksk.data())[idx] : reinterpret_cast<const u32 *>(ksk.data())[idx];
     };
     v.resize(p.n);
     o.s("\"k\":[");

@@ -148,9 +148,19 @@ int bfhe_eval_bingate_batch(bfhe_ctx *, uint32_t *dev_slab, const bfhe_gate *gat
 /* Bootstrap(ct) for a batch (what Encrypt's BOOTSTRAPPED default applies to every input, src/circuit.cpp:506) */
 int bfhe_bootstrap_batch(bfhe_ctx *, uint32_t *dev_slab, const uint32_t *in_rows, const uint32_t *out_rows, size_t count);
 /* end-to-end form with HOST buffers: H2D of the input slab rows, the wavefront, D2H of the produced rows.
- * in_host holds rows [0, in_rows) of the slab; gate.out rows are >= in_rows and < in_rows + out_rows. */
+ * in_host holds rows [0, in_rows) of the slab; gate.out rows are >= in_rows and < in_rows + out_rows.  The padding words of every
+ * output row are zero.
+ * Concurrent calls on one context may be combined into one wave: a call that finds no batch in flight launches at once with whatever
+ * is queued; calls that arrive while a batch runs queue up and go together as the next batch.  Results are identical to separate calls
+ * (a gate's words do not depend on the batch it ran in), and each call returns after its own rows are written.  Each call's arguments
+ * (pointers, row ranges, op, the alias rule) are checked in its own thread before it joins, so a bad call fails alone; a CUDA failure
+ * during a batch fails every call in it, each with the message in its own bfhe_last_error(). */
 int bfhe_eval_bingate_host(bfhe_ctx *, const bfhe_gate *gates, size_t count, const uint32_t *in_host, size_t in_rows,
                            uint32_t *out_host, size_t out_rows);
+/* EvalNOT(ct) on the host, for count rows of HOST memory: needs no device and works on host-only contexts.  The words of the device
+ * EvalNOT: a_i -> (q - a_i) mod q, b -> (q/4 + q - b) mod q; padding words are written as zero.  Every input word a_0 .. a_{n-1}, b
+ * must be below q, else BFHE_ERR_FORMAT naming the first bad row, and nothing is written.  ct_out may equal ct_in. */
+int bfhe_eval_not_host(const bfhe_ctx *, const uint32_t *ct_in, size_t count, uint32_t *ct_out);
 
 /* ---- measurement hooks ---- */
 /* when enabled, every hot-path launch is bracketed by CUDA events on the launch stream */
@@ -175,6 +185,10 @@ int bfhe_dbg_cluster_limits(bfhe_ctx *, int *cl2_gates, int *cl4_gates);
  * expansion produced: the BK staging buffer as downloaded, the device KSK restored to [N][baseKS][dKS][n+1] on the host.  full_blob holds
  * bfhe_keyblob_size bytes; the context keeps the imported keys. */
 int bfhe_dbg_expand_keys(bfhe_ctx *, const void *compact_blob, size_t len, void *full_blob, size_t cap);
+/* test hook for the combining of bfhe_eval_bingate_host: while hold != 0, calls queue and nothing launches, not even from an idle
+ * context; hold = 0 launches everything queued as one batch (in one of the waiting callers' threads).  Returns the number of calls
+ * that were queued when it was called (>= 0), so a test can wait until every caller has joined, or BFHE_ERR_ARG. */
+int bfhe_dbg_hold_batches(bfhe_ctx *, int hold);
 
 /* ---- circuit evaluator: mirrors class Circuit (src/circuit.h:56-72), level-synchronous ---- */
 typedef struct bfhe_circuit bfhe_circuit;

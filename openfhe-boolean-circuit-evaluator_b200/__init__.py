@@ -60,6 +60,7 @@ ABI_SYMBOLS = [
     "bfhe_circuit_exchange_mode", "bfhe_circuit_set_input_ct", "bfhe_circuit_clock_ct",
     "bfhe_import_openfhe_json", "bfhe_export_openfhe_json", "bfhe_import_openfhe_ct_json", "bfhe_export_openfhe_ct_json",
     "bfhe_btkeygen_compact", "bfhe_keyblob_compact_size", "bfhe_export_keys_compact", "bfhe_dbg_expand_keys",
+    "bfhe_eval_not_host", "bfhe_dbg_hold_batches",
 ]
 
 _lib = None
@@ -105,6 +106,8 @@ def lib():
     L.bfhe_eval_bingate_batch.argtypes = [vp, vp, vp, sz]
     L.bfhe_bootstrap_batch.argtypes = [vp, vp, vp, vp, sz]
     L.bfhe_eval_bingate_host.argtypes = [vp, vp, sz, vp, sz, vp, sz]
+    L.bfhe_eval_not_host.argtypes = [vp, vp, sz, vp]
+    L.bfhe_dbg_hold_batches.argtypes = [vp, C.c_int]
     L.bfhe_profile_enable.argtypes = [vp, C.c_int]
     L.bfhe_profile_read.argtypes = [vp, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_uint64)]
     L.bfhe_microbench_int.argtypes = [vp, C.c_int, C.POINTER(C.c_double)]
@@ -356,13 +359,17 @@ class Context:
         g = np.array([(gate, 0, 1, 2)], dtype=GATE_DTYPE)
         return self.eval_bingate_host(g, np.ascontiguousarray(inp), 1)[0]
 
-    def EvalNOT(self, ct):
-        s = self.slab(2)
-        s.upload(np.asarray(ct, dtype=np.uint32).reshape(1, -1))
-        self.eval_not_batch(s, [0], [1])
-        out = s.download(1, 1)[0]
-        s.free()
+    def eval_not_host(self, cts):
+        """EvalNOT of host rows (bfhe_eval_not_host): no device needed; every word below q, else BfheError ERR_FORMAT"""
+        cts = np.ascontiguousarray(cts, dtype=np.uint32)
+        if cts.ndim != 2 or cts.shape[1] != self.stride:
+            raise ValueError("ciphertext array shape %s, expected (rows, %d)" % (cts.shape, self.stride))
+        out = np.empty_like(cts)
+        self._ck(self.L.bfhe_eval_not_host(self.h, _ptr(cts), cts.shape[0], _ptr(out)))
         return out
+
+    def EvalNOT(self, ct):
+        return self.eval_not_host(np.asarray(ct, dtype=np.uint32).reshape(1, -1))[0]
 
     def Bootstrap(self, ct):
         inp = np.ascontiguousarray(np.asarray(ct, dtype=np.uint32).reshape(1, -1))
@@ -401,6 +408,14 @@ class Context:
 
     def dbg_set_gates_per_cta(self, g):
         self._ck(self.L.bfhe_dbg_set_gates_per_cta(self.h, g))
+
+    def dbg_hold_batches(self, hold):
+        """while on, eval_bingate_host calls queue and nothing launches; off launches everything queued as one batch.
+        Returns how many calls were queued when it was called."""
+        rc = self.L.bfhe_dbg_hold_batches(self.h, int(hold))
+        if rc < 0:
+            self._ck(rc)
+        return rc
 
     def dbg_expand_keys(self, compact_blob):
         """import a BFHEKEY2 blob through the device expansion and return the BFHEKEY1 blob it produced"""

@@ -47,11 +47,11 @@ def build(force=False, verbose=False):
         raise subprocess.CalledProcessError(1, failed[0])
     subprocess.check_call([NVCC, "-ccbin", CCBIN, "-shared", "-o", LIB] + objs + ["-lgomp", "-ldl", "-cudart", "static"])
     # C++ example written against the reference-shaped headers (host/circuit.h, host/binfhecontext.h)
-    for name in ("tb_circuit", "tb_client_server"):
+    for name, flags in (("tb_circuit", []), ("tb_client_server", []), ("tb_omp_gates", ["-fopenmp"])):
         ex = os.path.join(HERE, "examples", name + ".cpp")
         if os.path.exists(ex):
-            subprocess.check_call([CCBIN, "-O2", "-std=c++17", "-o", os.path.join(HERE, "examples", name), ex, "-L" + HERE, "-lbfhe_b200",
-                                   "-Wl,-rpath," + HERE])
+            subprocess.check_call([CCBIN, "-O2", "-std=c++17"] + flags + ["-o", os.path.join(HERE, "examples", name), ex, "-L" + HERE,
+                                   "-lbfhe_b200", "-Wl,-rpath," + HERE])
     return LIB
 
 

@@ -1010,13 +1010,41 @@ extern "C" int bfhe_bootstrap_batch(bfhe_ctx *c, uint32_t *slab, const uint32_t 
   return eval_batch_locked(c, slab, g.data(), count, nullptr);
 }
 
-extern "C" int bfhe_eval_bingate_host(bfhe_ctx *c, const bfhe_gate *gates, size_t count, const uint32_t *in_host, size_t in_rows,
-                                      uint32_t *out_host, size_t out_rows) {
-  int rc = need_device(c);
-  if (rc) return rc;
-  if (!gates || !in_host || !out_host) return BFHE_ERR_ARG;
+// ---- combining of concurrent bfhe_eval_bingate_host calls (flat combining; DESIGN.md section 7) ----
+// Each call is validated in its own thread, then queued.  With no batch in flight the call leads at once with whatever is queued; calls
+// arriving while a batch runs queue up, and when it finishes the front of the queue leads the next batch with everything queued.  A
+// gate's output words do not depend on the batch it runs in, so a combined call returns exactly what it would have returned alone.
+
+// the checks of eval_batch_locked and the row ranges of one call, before it may join a batch
+static int check_host_call(const bfhe_gate *gates, size_t count, size_t in_rows, size_t out_rows) {
+  const size_t rows = in_rows + out_rows;
+  for (size_t i = 0; i < count; i++)
+    if (gates[i].out < in_rows || gates[i].out >= rows || gates[i].in0 >= rows || gates[i].in1 >= rows) {
+      set_error("bfhe_eval_bingate_host: gate rows out of range");
+      return BFHE_ERR_ARG;
+    }
+  for (size_t i = 0; i < count; i++) {
+    const u32 g = gates[i].op & 0xff;
+    if (g > BFHE_BOOTSTRAP) { set_error("unknown gate type"); return BFHE_ERR_ARG; }
+    if (g != BFHE_BOOTSTRAP && gates[i].in0 == gates[i].in1 && (((gates[i].op & BFHE_NEG0) != 0) == ((gates[i].op & BFHE_NEG1) != 0))) {
+      set_error("EvalBinGate: please only use independent ciphertexts as inputs (gate " + std::to_string(i) + ")");
+      return BFHE_ERR_ALIAS;
+    }
+  }
+  return BFHE_OK;
+}
+
+// one batch.  Staging slab: every request's input rows, in queue order, then every request's output rows, in the same order (a lone call
+// gets today's layout: its in_rows, then its out_rows).  One H2D copy per request, one memset of the output block (the kernels write
+// ciphertext words only, so padding words come out zero whatever the slab held before), one eval_batch_locked over the concatenated gate
+// list with every row translated to its request's block, one D2H copy per request, one synchronise.
+static int run_host_batch(bfhe_ctx *c, const std::vector<HostGateReq *> &batch) {
   std::lock_guard<std::mutex> lk(c->mtx);
-  const size_t st = c->p.ct_stride, rows = in_rows + out_rows;
+  const size_t st = c->p.ct_stride;
+  size_t in_total = 0, out_total = 0, count = 0;
+  for (const HostGateReq *r : batch) { in_total += r->in_rows; out_total += r->out_rows; count += r->count; }
+  const size_t rows = in_total + out_total;
+  if (rows > 0xffffffffu) { set_error("bfhe_eval_bingate_host: combined batch exceeds 2^32 rows"); return BFHE_ERR_ARG; }
   if (rows > c->e2e_rows) {
     BFHE_CUDA(cudaStreamSynchronize(c->stream));
     cudaFree(c->e2e_slab);
@@ -1025,16 +1053,110 @@ extern "C" int bfhe_eval_bingate_host(bfhe_ctx *c, const bfhe_gate *gates, size_
     BFHE_CUDA(cudaMalloc(&c->e2e_slab, rows * st * 4));
     c->e2e_rows = rows;
   }
-  for (size_t i = 0; i < count; i++)
-    if (gates[i].out < in_rows || gates[i].out >= rows || gates[i].in0 >= rows || gates[i].in1 >= rows) {
-      set_error("bfhe_eval_bingate_host: gate rows out of range");
-      return BFHE_ERR_ARG;
+  std::vector<bfhe_gate> all;
+  const bfhe_gate *list = batch[0]->gates; // a lone call: the translation is the identity
+  if (batch.size() > 1) {
+    all.reserve(count);
+    size_t ib = 0, ob = in_total;
+    for (const HostGateReq *r : batch) {
+      auto at = [&](u32 row) { return (u32)(row < r->in_rows ? ib + row : ob + (row - r->in_rows)); };
+      for (size_t i = 0; i < r->count; i++) {
+        const bfhe_gate &g = r->gates[i];
+        all.push_back(bfhe_gate{g.op, at(g.in0), at(g.in1), at(g.out)});
+      }
+      ib += r->in_rows;
+      ob += r->out_rows;
     }
-  BFHE_CUDA(cudaMemcpyAsync(c->e2e_slab, in_host, in_rows * st * 4, cudaMemcpyHostToDevice, c->stream));
-  rc = eval_batch_locked(c, c->e2e_slab, gates, count, nullptr);
+    list = all.data();
+  }
+  int rc = BFHE_OK;
+  size_t ib = 0;
+  for (const HostGateReq *r : batch) {
+    if (r->in_rows) {
+      cudaError_t e = cudaMemcpyAsync(c->e2e_slab + ib * st, r->in_host, r->in_rows * st * 4, cudaMemcpyHostToDevice, c->stream);
+      if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMemcpyAsync (bfhe_eval_bingate_host inputs)"); break; }
+    }
+    ib += r->in_rows;
+  }
+  if (!rc && out_total) {
+    cudaError_t e = cudaMemsetAsync(c->e2e_slab + in_total * st, 0, out_total * st * 4, c->stream);
+    if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemsetAsync (bfhe_eval_bingate_host outputs)");
+  }
+  if (!rc) rc = eval_batch_locked(c, c->e2e_slab, list, count, nullptr);
+  size_t ob = in_total;
+  for (const HostGateReq *r : batch) {
+    if (rc) break;
+    if (r->out_rows) {
+      cudaError_t e = cudaMemcpyAsync(r->out_host, c->e2e_slab + ob * st, r->out_rows * st * 4, cudaMemcpyDeviceToHost, c->stream);
+      if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync (bfhe_eval_bingate_host outputs)");
+    }
+    ob += r->out_rows;
+  }
+  // also after a failure: nothing may still read or write a caller's buffer once its call returns
+  cudaError_t e = cudaStreamSynchronize(c->stream);
+  if (!rc && e != cudaSuccess) rc = cuda_fail(e, "cudaStreamSynchronize (bfhe_eval_bingate_host)");
+  return rc;
+}
+
+// with c->q_mtx held: the front of the queue leads the next batch, unless a batch is in flight or the hold is on
+static void hand_off(bfhe_ctx *c) {
+  if (c->q_busy || c->q_hold || c->q.empty()) return;
+  c->q_busy = true;
+  c->q.front()->state = HostGateReq::LEAD;
+  c->q.front()->cv.notify_one();
+}
+
+extern "C" int bfhe_eval_bingate_host(bfhe_ctx *c, const bfhe_gate *gates, size_t count, const uint32_t *in_host, size_t in_rows,
+                                      uint32_t *out_host, size_t out_rows) {
+  int rc = need_device(c);
   if (rc) return rc;
-  BFHE_CUDA(cudaMemcpyAsync(out_host, c->e2e_slab + in_rows * st, out_rows * st * 4, cudaMemcpyDeviceToHost, c->stream));
-  BFHE_CUDA(cudaStreamSynchronize(c->stream));
+  if (!gates || !in_host || !out_host) return BFHE_ERR_ARG;
+  if ((rc = check_host_call(gates, count, in_rows, out_rows))) return rc;
+  HostGateReq req;
+  req.gates = gates; req.count = count;
+  req.in_host = in_host; req.in_rows = in_rows;
+  req.out_host = out_host; req.out_rows = out_rows;
+  std::unique_lock<std::mutex> lk(c->q_mtx);
+  c->q.push_back(&req);
+  hand_off(c);
+  while (req.state == HostGateReq::QUEUED) req.cv.wait(lk);
+  if (req.state == HostGateReq::LEAD) {
+    std::vector<HostGateReq *> batch(c->q.begin(), c->q.end());
+    c->q.clear();
+    lk.unlock();
+    rc = run_host_batch(c, batch);
+    const std::string err = rc ? bfhe_last_error() : std::string();
+    lk.lock();
+    for (HostGateReq *r : batch) { // a waiter returns once it sees DONE, after this lock is released; its request is not touched again
+      r->rc = rc;
+      r->err = err;
+      r->state = HostGateReq::DONE;
+      if (r != &req) r->cv.notify_one();
+    }
+    c->q_busy = false;
+    hand_off(c);
+  }
+  lk.unlock();
+  if (req.rc) set_error(req.err); // bfhe_last_error is per thread: every caller of a failed batch gets the message in its own
+  return req.rc;
+}
+
+extern "C" int bfhe_eval_not_host(const bfhe_ctx *c, const uint32_t *ct_in, size_t count, uint32_t *ct_out) {
+  if (!c || !ct_in || !ct_out) return BFHE_ERR_ARG;
+  const u32 n = c->p.n, q = c->p.q, st = c->p.ct_stride;
+  for (size_t r = 0; r < count; r++) // every row checked before any is written (ct_in == ct_out is allowed)
+    for (u32 i = 0; i <= n; i++)
+      if (ct_in[r * st + i] >= q) {
+        set_error("EvalNOT: input ciphertext row " + std::to_string(r) + " has a word >= q");
+        return BFHE_ERR_FORMAT;
+      }
+  for (size_t r = 0; r < count; r++) { // the words of eval_not_kernel
+    const u32 *x = ct_in + r * st;
+    u32 *y = ct_out + r * st;
+    for (u32 i = 0; i < n; i++) y[i] = (q - x[i]) % q;
+    y[n] = (q / 4 + q - x[n]) % q;
+    for (u32 i = n + 1; i < st; i++) y[i] = 0;
+  }
   return BFHE_OK;
 }
 
@@ -1134,4 +1256,12 @@ extern "C" int bfhe_dbg_set_gates_per_cta(bfhe_ctx *c, int g) {
   if (!c) return BFHE_ERR_ARG;
   c->force_g = g;
   return BFHE_OK;
+}
+extern "C" int bfhe_dbg_hold_batches(bfhe_ctx *c, int hold) {
+  if (!c) return BFHE_ERR_ARG;
+  std::lock_guard<std::mutex> lk(c->q_mtx);
+  const int queued = (int)c->q.size();
+  c->q_hold = hold != 0;
+  hand_off(c); // release: the front of the queue leads one batch of everything queued
+  return queued;
 }

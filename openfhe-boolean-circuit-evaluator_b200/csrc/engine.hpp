@@ -3,7 +3,9 @@
 #include "../../include/bfhe.h"
 #include "common.hpp"
 #include "hostmath.hpp"
+#include <condition_variable>
 #include <cuda_runtime.h>
+#include <deque>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -21,6 +23,20 @@ int cuda_fail(cudaError_t e, const char *what);
 struct ProfSpan {
   cudaEvent_t a, b;
   int kernel;
+};
+
+// one bfhe_eval_bingate_host call waiting to be combined with concurrent ones (engine.cu, "combining"); lives on the caller's stack
+struct HostGateReq {
+  const bfhe_gate *gates;
+  size_t count;
+  const u32 *in_host;
+  size_t in_rows;
+  u32 *out_host;
+  size_t out_rows;
+  enum { QUEUED, LEAD, DONE } state = QUEUED;
+  int rc = BFHE_OK;
+  std::string err;
+  std::condition_variable cv;
 };
 
 } // namespace bfhe
@@ -86,6 +102,13 @@ struct bfhe_ctx {
   bool profiling = false;
   std::vector<bfhe::ProfSpan> spans;
   std::mutex mtx; // the reference calls EvalBinGate concurrently from OpenMP tasks (src/circuit.cpp:698-710)
+
+  // combining of concurrent bfhe_eval_bingate_host calls: at most one batch in flight; calls arriving meanwhile queue (FIFO) and the
+  // front one leads the next batch.  q_mtx guards the queue only; the leader takes mtx for the device work.
+  std::mutex q_mtx;
+  std::deque<bfhe::HostGateReq *> q;
+  bool q_busy = false; // a batch is in flight (a leader has been chosen)
+  bool q_hold = false; // test hook bfhe_dbg_hold_batches: nothing launches
 };
 
 namespace bfhe {

@@ -5,7 +5,9 @@
 // EvalNOT (src/gate.cpp:112), EvalBinGate (src/gate.cpp:133), the enums BINFHE_PARAMSET / BINFHE_METHOD / BINGATE
 // (src/utils.cpp:165-190, src/gate.cpp:133,172) and the types LWECiphertext / LWEPrivateKey / LWEPlaintext
 // (src/wire.h:46, src/circuit.h:75-76, src/gate.cpp:71).  Pointing the reference's include path at this directory
-// makes gate.cpp-style code compile against the B200 engine: every single-gate call is a batch of one.
+// makes gate.cpp-style code compile against the B200 engine.  Every single-gate call is a batch of one, and calls that threads make
+// at the same time (the reference's one OpenMP task per ready gate, src/circuit.cpp:698-710) are combined into shared GPU waves by
+// bfhe_eval_bingate_host.
 // Header-only; link with libbfhe_b200.so.
 #pragma once
 #include "../../include/bfhe.h"
@@ -72,7 +74,14 @@ public:
     check(bfhe_decrypt(raw(), ct->row.data(), 1, &r));
     *result = r;
   }
-  LWECiphertext EvalNOT(ConstLWECiphertext ct) const { return one_gate(BFHE_BOOTSTRAP + 1, ct, ct); }
+  // on the host (bfhe_eval_not_host): no bootstrap and no device work
+  LWECiphertext EvalNOT(ConstLWECiphertext ct) const {
+    auto out = std::make_shared<LWECiphertextImpl>();
+    out->row.resize(m_p.ct_stride);
+    if (ct->row.size() != m_p.ct_stride) throw std::runtime_error("EvalNOT: ciphertext is not a row of ct_stride words");
+    check(bfhe_eval_not_host(raw(), ct->row.data(), 1, out->row.data()));
+    return out;
+  }
   LWECiphertext EvalBinGate(const BINGATE gate, ConstLWECiphertext ct1, ConstLWECiphertext ct2) const {
     if (ct1 == ct2) throw config_error("ERROR: Please only use independent ciphertexts as inputs.");
     return one_gate((uint32_t)gate, ct1, ct2);
@@ -113,17 +122,6 @@ private:
     const size_t st = m_p.ct_stride;
     auto out = std::make_shared<LWECiphertextImpl>();
     out->row.resize(st);
-    if (op == BFHE_BOOTSTRAP + 1) { // EvalNOT: no bootstrap, device kernel on a 2-row slab
-      uint32_t *slab = nullptr;
-      check(bfhe_slab_alloc(raw(), 2, &slab));
-      const uint32_t in = 0, o = 1;
-      int rc = bfhe_slab_upload(raw(), slab, 0, a->row.data(), 1);
-      if (!rc) rc = bfhe_eval_not_batch(raw(), slab, &in, &o, 1);
-      if (!rc) rc = bfhe_slab_download(raw(), slab, 1, out->row.data(), 1);
-      bfhe_slab_free(raw(), slab);
-      check(rc);
-      return out;
-    }
     std::vector<uint32_t> in(2 * st);
     std::copy(a->row.begin(), a->row.end(), in.begin());
     std::copy(b->row.begin(), b->row.end(), in.begin() + st);

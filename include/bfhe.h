@@ -112,6 +112,32 @@ size_t bfhe_keyblob_compact_size(const bfhe_ctx *);
 /* BFHE_ERR_STATE when the keys have no mask seed (bfhe_btkeygen, a BFHEKEY1 import, an OpenFHE JSON import) */
 int bfhe_export_keys_compact(const bfhe_ctx *, void *buf, size_t cap, int include_sk);
 
+/* ---- compact fresh ciphertexts: a client's inputs as a public mask seed and one body word per bit ----
+ * n of the n+1 words of a fresh encryption are its uniform mask, which carries no secret.  bfhe_encrypt_compact draws every mask from a
+ * public seed, so the blob, BFHECTS1, holds that seed and one body per bit: an AES-128 block (256 bits) is 576 bytes instead of 516 KB of
+ * full rows at STD128_OPT.  Only fresh encryptions can be compact; bootstrapped ciphertexts and the evaluator's outputs stay full rows.
+ *   mask seed: 256 bits, fresh on every call.  seed == 0 -> OS entropy, independent of the secret stream; seed != 0 -> a dedicated stream
+ *              of the secret SeedKey (reproducible and not confidential, as for every nonzero seed; a different stream from the mask
+ *              seed of bfhe_btkeygen_compact).
+ *   expansion: row g (g = 0 .. count-1) has mask row r = g under this seed, by the rule of the compact keys above: ChaCha20 keyed with the
+ *              seed, nonce r, coefficient t = keystream words 4t .. 4t+3 as a little-endian 128-bit integer mod q.  q is a power of two,
+ *              so the reduction is exact and uniform.
+ *   body:      b_g = <a_g, s> + e_g + (bits[g] % 4) * q/4 mod q, the message convention of bfhe_encrypt; e_g is the Gaussian noise of
+ *              bfhe_encrypt drawn from stream 2^48 + g of the secret SeedKey (a range no other call uses).
+ * Layout of BFHECTS1, little-endian: 64-byte header {magic "BFHECTS1", u32 version = 1, u32 paramset, u32 n, u32 q, u64 count, the 32-byte
+ *   mask seed} | count uint16 bodies, zero-padded to 8 bytes.  Size 64 + pad8(2 * count).
+ * Every reader checks on the host, before any device work, and answers BFHE_ERR_FORMAT naming what failed: magic and version; paramset,
+ *   n and q equal to the context's; the exact length; every body below q (naming the first bad index); zero padding bytes.
+ * SECURITY: the mask seed is public and the noise comes only from the secret stream.  Never reuse a mask seed for a second batch under
+ * the same key: identical masks expose the differences of the messages.  bfhe_encrypt_compact draws a new one on every call. */
+size_t bfhe_ct_compact_size(const bfhe_ctx *, size_t count);
+/* on the host, with the secret key (BFHE_ERR_STATE without it); works on host-only contexts.  blob holds bfhe_ct_compact_size bytes. */
+int bfhe_encrypt_compact(const bfhe_ctx *, const uint8_t *bits, size_t count, uint64_t seed, void *blob, size_t cap);
+/* the blob's count full rows of ct_stride words (padding words zero) into cts (cap_rows rows).  on_device == 0: host memory, works on any
+ * context, with or without keys.  on_device != 0: memory of the context's device, 16-byte aligned (else BFHE_ERR_ARG), written by one
+ * expansion launch on the launch stream; returns after the rows are written.  A host-only context gives BFHE_ERR_CUDA. */
+int bfhe_expand_cts(bfhe_ctx *, const void *blob, size_t len, uint32_t *cts, size_t cap_rows, int on_device);
+
 /* ---- OpenFHE 1.0.x object exchange (SURVEY 8 row f-3; the reference's crypto is find_package(OpenFHE), CMakeLists.txt:8, "Tested with
  * OpenFHE v.1.0.1", Release_Notes.md:4) ----
  * cereal JSON archives as OpenFHE's own Serial::SerializeToFile(path, obj, SerType::JSON) writes them (the reference itself never
@@ -249,6 +275,11 @@ int bfhe_circuit_clock(bfhe_circuit *, uint8_t *out_bits, size_t cap, uint8_t *p
  * After this call bfhe_circuit_clock (bits) decrypts as usual when the context holds the secret key, and fails with BFHE_ERR_STATE
  * before launching anything when it does not. */
 int bfhe_circuit_set_input_ct(bfhe_circuit *, const uint32_t *cts, size_t nbits, int on_device);
+/* bfhe_circuit_set_input_ct from a BFHECTS1 blob (bfhe_encrypt_compact): the masks are generated on the GPU straight into the circuit's
+ * fresh input rows.  Modes, flip-flop power-up and the "without input on error" rule are those of bfhe_circuit_set_input_ct.  The blob's
+ * checks give BFHE_ERR_FORMAT; count != the circuit's input bits gives BFHE_ERR_ARG.  Sharded circuits: collective; only rank 0's blob is
+ * read (other ranks may pass NULL), and a blob rank 0 refuses still goes through the broadcast, so every rank returns the same code. */
+int bfhe_circuit_set_input_compact(bfhe_circuit *, const void *blob, size_t len);
 /* Circuit::Clock with the outputs left encrypted: out_bits rows of ct_stride words (padding words zero) into out_cts, host or device
  * memory (on_device as above).  An output that reads its wire through NOT comes out as EvalNOT of that row, so it decrypts to what
  * bfhe_circuit_clock returns.  Encrypted mode without verify mode; works after either SetInput form and needs no secret key.  Every rank

@@ -61,6 +61,7 @@ ABI_SYMBOLS = [
     "bfhe_import_openfhe_json", "bfhe_export_openfhe_json", "bfhe_import_openfhe_ct_json", "bfhe_export_openfhe_ct_json",
     "bfhe_btkeygen_compact", "bfhe_keyblob_compact_size", "bfhe_export_keys_compact", "bfhe_dbg_expand_keys",
     "bfhe_eval_not_host", "bfhe_dbg_hold_batches",
+    "bfhe_ct_compact_size", "bfhe_encrypt_compact", "bfhe_expand_cts", "bfhe_circuit_set_input_compact",
 ]
 
 _lib = None
@@ -98,6 +99,11 @@ def lib():
     L.bfhe_load_keys.argtypes = [vp, C.c_char_p]
     L.bfhe_encrypt.argtypes = [vp, vp, sz, C.c_uint64, vp]
     L.bfhe_decrypt.argtypes = [vp, vp, sz, vp]
+    L.bfhe_ct_compact_size.restype = sz
+    L.bfhe_ct_compact_size.argtypes = [vp, sz]
+    L.bfhe_encrypt_compact.argtypes = [vp, vp, sz, C.c_uint64, vp, sz]
+    L.bfhe_expand_cts.argtypes = [vp, vp, sz, vp, sz, C.c_int]
+    L.bfhe_circuit_set_input_compact.argtypes = [vp, vp, sz]
     L.bfhe_slab_alloc.argtypes = [vp, sz, C.POINTER(vp)]
     L.bfhe_slab_free.argtypes = [vp, vp]
     L.bfhe_slab_upload.argtypes = [vp, vp, sz, vp, sz]
@@ -313,6 +319,34 @@ class Context:
         cts = np.ascontiguousarray(cts, dtype=np.uint32).reshape(-1, self.stride)
         out = np.zeros(cts.shape[0], dtype=np.uint8)
         self._ck(self.L.bfhe_decrypt(self.h, _ptr(cts), cts.shape[0], _ptr(out)))
+        return out
+
+    # compact fresh ciphertexts (BFHECTS1, include/bfhe.h)
+    def ct_compact_size(self, count):
+        return self.L.bfhe_ct_compact_size(self.h, count)
+
+    def encrypt_compact(self, bits, seed=0):
+        """the BFHECTS1 blob of fresh encryptions of `bits` (a public mask seed and one body per bit) as a np.uint8 array"""
+        bits = np.ascontiguousarray(np.asarray(bits).ravel(), dtype=np.uint8)
+        blob = np.empty(self.ct_compact_size(bits.size), dtype=np.uint8)
+        self._ck(self.L.bfhe_encrypt_compact(self.h, _ptr(bits), bits.size, seed, _ptr(blob), blob.size))
+        return blob
+
+    def expand_cts(self, blob, out=None):
+        """the full rows of a BFHECTS1 blob.  out None or a numpy array (count, ct_stride) of uint32: host rows, returned; a Slab,
+        Slab.range(...) or __cuda_array_interface__ object: rows written on the device, `out` returned."""
+        blob = np.ascontiguousarray(blob, dtype=np.uint8)
+        if out is None:
+            # the header's count, bounded by what the length allows (a blob whose count and length disagree is refused)
+            count = min(int(blob[24:32].view(np.uint64)[0]), (blob.size - 64) // 2) if blob.size >= 64 else 0
+            out = np.zeros((count, self.stride), dtype=np.uint32)
+        if isinstance(out, np.ndarray):
+            if out.ndim != 2 or out.shape[1] != self.stride or out.dtype != np.uint32 or not out.flags["C_CONTIGUOUS"]:
+                raise ValueError("host rows must be a C-contiguous uint32 array (rows, %d)" % self.stride)
+            self._ck(self.L.bfhe_expand_cts(self.h, _ptr(blob), blob.size, _ptr(out), out.shape[0], 0))
+            return out
+        ptr, rows = _device_rows(out, self.stride)
+        self._ck(self.L.bfhe_expand_cts(self.h, _ptr(blob), blob.size, ptr, rows, 1))
         return out
 
     # device
@@ -621,6 +655,15 @@ class Circuit:
         else:
             ptr, rows = _device_rows(cts, stride)
             self._ck(self.L.bfhe_circuit_set_input_ct(self.h, ptr, rows, 1))
+
+    def set_input_compact(self, blob):
+        """SetInput from a BFHECTS1 blob (Context.encrypt_compact), masks generated on the GPU; needs the evaluation keys only.
+        Sharded circuits: rank 0's blob is used; other ranks may pass None."""
+        if blob is None:
+            self._ck(self.L.bfhe_circuit_set_input_compact(self.h, None, 0))
+        else:
+            b = np.ascontiguousarray(blob, dtype=np.uint8)
+            self._ck(self.L.bfhe_circuit_set_input_compact(self.h, _ptr(b), b.size))
 
     def clock_ct(self, out=None):
         """Clock with the outputs left encrypted (bfhe_circuit_clock_ct): a numpy array (out_bits, ct_stride) of uint32, or, with `out`

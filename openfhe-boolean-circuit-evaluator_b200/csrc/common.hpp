@@ -123,6 +123,9 @@ constexpr u64 BK_MASK_STREAM = 1ull << 40;
 // the device KSK ([i][k][j][rowlen], as ensure_device_keys lays it out) from the bodies ([N][baseKS][dKS], elem_bytes each)
 int launch_ksk_expand(const MaskKey &key, const void *d_bodies, void *d_ksk, int elem_bytes, u32 N, u32 baseKS, u32 dKS, u32 n, u32 rowlen,
                       u32 qKS, void *stream);
+// `count` fresh ciphertext rows (stride words, 16-byte aligned) of a compact blob: row g is mask row g mod q, body d_bodies[g]; the
+// same kernel as launch_ksk_expand with baseKS = dKS = 1
+int launch_ct_expand(const MaskKey &key, const u32 *d_bodies, u32 *d_rows, size_t count, u32 n, u32 stride, u32 q, void *stream);
 // `pairs` (mask, body) polynomial pairs of the coefficient-form BK, starting at mask polynomial p_first, into d_stage (2 * pairs * N words)
 int launch_bk_mask_expand(const MaskKey &key, const u32 *d_bodies, u32 *d_stage, u64 p_first, size_t pairs, u32 N, u32 Q, void *stream);
 int launch_dbg_ntt(const DevConst &P, const u32 *d_a, const u32 *d_b, u32 *d_rt, u32 *d_prod, int npoly, const u32 *d_twl,

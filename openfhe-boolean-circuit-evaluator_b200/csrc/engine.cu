@@ -457,18 +457,25 @@ static int btkeygen(bfhe_ctx *c, uint64_t seed64, const MaskKey *mask) {
 
 extern "C" int bfhe_btkeygen(bfhe_ctx *c, uint64_t seed64) { return btkeygen(c, seed64, nullptr); }
 
+// a fresh public mask seed.  seed64 == 0: OS entropy, independent of the secret stream; else reproducible: 256 bits of stream `stream` of
+// the secret SeedKey (ChaCha20 output reveals nothing about the key)
+static int make_mask_seed(uint64_t seed64, u64 stream, MaskKey &mask) {
+  if (seed64 == 0) {
+    if (!SeedKey::os_entropy(mask.k, sizeof mask.k)) { set_error("cannot read OS entropy (getrandom and /dev/urandom both failed)"); return BFHE_ERR_IO; }
+    return BFHE_OK;
+  }
+  SeedKey seed;
+  if (int rc = make_seed_key(seed64, seed)) return rc;
+  Rng r(seed, stream);
+  for (auto &w : mask.k) w = r.next32();
+  return BFHE_OK;
+}
+
 extern "C" int bfhe_btkeygen_compact(bfhe_ctx *c, uint64_t seed64) {
   if (!c) return BFHE_ERR_ARG;
   if (!c->has_sk) { set_error("BTKeyGen before KeyGen"); return BFHE_ERR_STATE; }
   MaskKey mask;
-  if (seed64 == 0) { // independent of the secret stream
-    if (!SeedKey::os_entropy(mask.k, sizeof mask.k)) { set_error("cannot read OS entropy (getrandom and /dev/urandom both failed)"); return BFHE_ERR_IO; }
-  } else { // reproducible: a stream of its own under the secret SeedKey (ChaCha20 output reveals nothing about the key)
-    SeedKey seed;
-    if (int rc = make_seed_key(seed64, seed)) return rc;
-    Rng r(seed, 0x4D41534B);
-    for (auto &w : mask.k) w = r.next32();
-  }
+  if (int rc = make_mask_seed(seed64, 0x4D41534B, mask)) return rc;
   return btkeygen(c, seed64, &mask);
 }
 
@@ -826,6 +833,142 @@ extern "C" int bfhe_slab_download(bfhe_ctx *c, const uint32_t *slab, size_t firs
   if (rc) return rc;
   const size_t st = c->p.ct_stride;
   BFHE_CUDA(cudaMemcpyAsync(host, slab + first * st, rows * st * 4, cudaMemcpyDeviceToHost, c->stream));
+  BFHE_CUDA(cudaStreamSynchronize(c->stream));
+  return BFHE_OK;
+}
+int bfhe::check_device_buffer(const bfhe_ctx *c, const void *p, const char *what) {
+  cudaPointerAttributes pa{};
+  if (cudaPointerGetAttributes(&pa, p) != cudaSuccess || (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) ||
+      pa.device != c->device) {
+    cudaGetLastError();
+    set_error(std::string(what) + " is not memory of device " + std::to_string(c->device));
+    return BFHE_ERR_ARG;
+  }
+  return BFHE_OK;
+}
+
+// -------------------------------------------------------------------------------------------------
+// compact fresh ciphertexts (BFHECTS1, include/bfhe.h): a public mask seed and one body per bit
+// -------------------------------------------------------------------------------------------------
+struct CtBlobHeader {
+  char magic[8];
+  u32 version, paramset, n, q;
+  u64 count;
+  MaskKey seed;
+};
+static_assert(sizeof(CtBlobHeader) == 64, "the BFHECTS1 header is 64 bytes");
+static constexpr u64 CT_MASK_SEED_STREAM = 0x43544D534Bull; // stream of the secret SeedKey giving a reproducible mask seed (keys: 0x4D41534B)
+static constexpr u64 CT_NOISE_STREAM = 1ull << 48;          // + g: the noise of row g (bfhe_encrypt uses 0x900000 + g)
+
+static u32 ct_body(const u8 *bodies, size_t g) {
+  u16 v;
+  std::memcpy(&v, bodies + 2 * g, 2);
+  return v;
+}
+
+extern "C" size_t bfhe_ct_compact_size(const bfhe_ctx *c, size_t count) {
+  if (!c || count > (SIZE_MAX - sizeof(CtBlobHeader) - 8) / 2) return 0;
+  return sizeof(CtBlobHeader) + pad8(2 * count);
+}
+
+extern "C" int bfhe_encrypt_compact(const bfhe_ctx *c, const uint8_t *bits, size_t count, uint64_t seed, void *blob, size_t cap) {
+  if (!c || (!bits && count) || !blob) return BFHE_ERR_ARG;
+  if (!c->has_sk) { set_error("Encrypt before KeyGen"); return BFHE_ERR_STATE; }
+  const size_t size = bfhe_ct_compact_size(c, count);
+  if (!size || cap < size) { set_error("bfhe_encrypt_compact: blob buffer too small"); return BFHE_ERR_ARG; }
+  SeedKey key;
+  if (int rc = make_seed_key(seed, key)) return rc;
+  CtBlobHeader h{};
+  std::memcpy(h.magic, "BFHECTS1", 8);
+  h.version = 1; h.paramset = c->p.paramset; h.n = c->p.n; h.q = c->p.q; h.count = count;
+  if (int rc = make_mask_seed(seed, CT_MASK_SEED_STREAM, h.seed)) return rc;
+  const u32 n = c->p.n, q = c->p.q;
+  u8 *bodies = (u8 *)blob + sizeof h;
+#pragma omp parallel for schedule(static) if (count > 256)
+  for (i64 g = 0; g < (i64)count; g++) {
+    Rng r(key, CT_NOISE_STREAM + (u64)g);
+    i64 b = (i64)(bits[g] % 4) * (q / 4) + gauss_table().sample(r);
+    expand_mask(h.seed, (u64)g, q, n, [&](size_t t, u32 a) { b += (i64)a * c->sk[t]; });
+    b %= (i64)q;
+    if (b < 0) b += q;
+    const u16 v = (u16)b;
+    std::memcpy(bodies + 2 * (size_t)g, &v, 2);
+  }
+  std::memcpy(blob, &h, sizeof h);
+  std::memset(bodies + 2 * count, 0, pad8(2 * count) - 2 * count);
+  return BFHE_OK;
+}
+
+int bfhe::read_ct_blob(const bfhe_ctx *c, const void *blob, size_t len, CtBlob &out) {
+  CtBlobHeader h;
+  if (len < sizeof h) { set_error("BFHECTS1: " + std::to_string(len) + " bytes, shorter than the 64-byte header"); return BFHE_ERR_FORMAT; }
+  std::memcpy(&h, blob, sizeof h);
+  if (std::memcmp(h.magic, "BFHECTS1", 8)) { set_error("BFHECTS1: bad magic, not a compact ciphertext blob"); return BFHE_ERR_FORMAT; }
+  if (h.version != 1) { set_error("BFHECTS1: version " + std::to_string(h.version) + " is not 1"); return BFHE_ERR_FORMAT; }
+  const bfhe_params &p = c->p;
+  if (h.paramset != p.paramset || h.n != p.n || h.q != p.q) {
+    set_error("BFHECTS1: paramset " + std::to_string(h.paramset) + ", n " + std::to_string(h.n) + ", q " + std::to_string(h.q) +
+              " do not match this context (paramset " + std::to_string(p.paramset) + ", n " + std::to_string(p.n) + ", q " + std::to_string(p.q) + ")");
+    return BFHE_ERR_FORMAT;
+  }
+  if (h.count > (len - sizeof h) / 2 || len != sizeof h + pad8(2 * h.count)) {
+    set_error("BFHECTS1: length " + std::to_string(len) + " bytes does not match count " + std::to_string(h.count) + " (64 + pad8(2 count) bytes)");
+    return BFHE_ERR_FORMAT;
+  }
+  const u8 *bodies = (const u8 *)blob + sizeof h;
+  for (size_t g = 0; g < h.count; g++)
+    if (ct_body(bodies, g) >= p.q) {
+      set_error("BFHECTS1: body " + std::to_string(g) + " = " + std::to_string(ct_body(bodies, g)) + " is not below q = " + std::to_string(p.q));
+      return BFHE_ERR_FORMAT;
+    }
+  for (size_t i = 2 * h.count; i < len - sizeof h; i++)
+    if (bodies[i]) { set_error("BFHECTS1: nonzero padding byte at offset " + std::to_string(sizeof h + i)); return BFHE_ERR_FORMAT; }
+  out.seed = h.seed;
+  out.count = h.count;
+  out.bodies = bodies;
+  return BFHE_OK;
+}
+
+static int ensure_tmp(bfhe_ctx *c, size_t rows);
+int bfhe::expand_ct_rows(bfhe_ctx *c, const CtBlob &b, u32 *d_rows, std::vector<u32> &wide) {
+  if (b.count == 0) return BFHE_OK;
+  wide.resize(b.count);
+  for (size_t g = 0; g < b.count; g++) wide[g] = ct_body(b.bodies, g);
+  // the bodies go through the per-call scratch rows (kept between calls; a stream-ordered allocation would map fresh memory every time)
+  if (int rc = ensure_tmp(c, (b.count + c->p.ct_stride - 1) / c->p.ct_stride)) return rc;
+  BFHE_CUDA(cudaMemcpyAsync(c->d_tmp, wide.data(), b.count * 4, cudaMemcpyHostToDevice, c->stream));
+  int rc = launch_ct_expand(b.seed, c->d_tmp, d_rows, b.count, c->p.n, c->p.ct_stride, c->p.q, c->stream);
+  if (rc) return cuda_fail((cudaError_t)rc, "ct_expand");
+  return BFHE_OK;
+}
+
+extern "C" int bfhe_expand_cts(bfhe_ctx *c, const void *blob, size_t len, uint32_t *cts, size_t cap_rows, int on_device) {
+  if (!c || !blob) return BFHE_ERR_ARG;
+  CtBlob b;
+  if (int rc = read_ct_blob(c, blob, len, b)) return rc;
+  if (cap_rows < b.count) {
+    set_error("bfhe_expand_cts: the blob holds " + std::to_string(b.count) + " rows, the destination " + std::to_string(cap_rows));
+    return BFHE_ERR_ARG;
+  }
+  if (!cts && b.count) { set_error("bfhe_expand_cts: null destination"); return BFHE_ERR_ARG; }
+  if (!on_device) {
+    const u32 n = c->p.n, q = c->p.q, st = c->p.ct_stride;
+#pragma omp parallel for schedule(static) if (b.count > 256)
+    for (i64 g = 0; g < (i64)b.count; g++) {
+      u32 *row = cts + (size_t)g * st;
+      expand_mask(b.seed, (u64)g, q, n, [&](size_t t, u32 a) { row[t] = a; });
+      row[n] = ct_body(b.bodies, (size_t)g);
+      for (u32 i = n + 1; i < st; i++) row[i] = 0;
+    }
+    return BFHE_OK;
+  }
+  if (int rc = need_device(c)) return rc;
+  if (b.count == 0) return BFHE_OK;
+  std::lock_guard<std::mutex> lk(c->mtx);
+  if (int rc = check_device_buffer(c, cts, "bfhe_expand_cts: the destination")) return rc;
+  if ((uintptr_t)cts % 16) { set_error("bfhe_expand_cts: the destination is not 16-byte aligned"); return BFHE_ERR_ARG; }
+  std::vector<u32> wide;
+  if (int rc = expand_ct_rows(c, b, cts, wide)) return rc;
   BFHE_CUDA(cudaStreamSynchronize(c->stream));
   return BFHE_OK;
 }

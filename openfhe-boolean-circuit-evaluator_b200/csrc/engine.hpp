@@ -86,7 +86,7 @@ struct bfhe_ctx {
   cudaEvent_t stage_ev[2] = {nullptr, nullptr};
   int stage_next = 0;
   bfhe::u32 *d_ext = nullptr;            // CHUNK * (N+4)
-  bfhe::u32 *d_tmp = nullptr;            // composite-gate temporaries
+  bfhe::u32 *d_tmp = nullptr;            // composite-gate temporaries; the bodies of a compact ciphertext blob (expand_ct_rows)
   size_t tmp_rows = 0;
   const bfhe::u32 **d_ptr_in = nullptr;  // EvalNOT pointer lists
   bfhe::u32 **d_ptr_out = nullptr;
@@ -122,4 +122,17 @@ void host_full_ksk(const bfhe_ctx *c, u8 *out);
 void forget_mask_seed(bfhe_ctx *c);
 // EvalNOT of in[i] into out[i] through the context's pointer buffers (low bit of in[i] set: plain copy); caller holds c->mtx
 int not_ptr_batch(bfhe_ctx *c, const std::vector<const u32 *> &in, const std::vector<u32 *> &out);
+// a BFHECTS1 blob of compact fresh ciphertexts (include/bfhe.h) that passed every check of read_ct_blob; bodies points into the blob
+struct CtBlob {
+  MaskKey seed{};
+  size_t count = 0;
+  const u8 *bodies = nullptr; // count little-endian uint16, each below q
+};
+// the host checks of a BFHECTS1 blob against this context: BFHE_ERR_FORMAT naming what failed
+int read_ct_blob(const bfhe_ctx *c, const void *blob, size_t len, CtBlob &out);
+// enqueue on c->stream: the blob's count full rows into d_rows (device memory, ct_stride words per row, 16-byte aligned).  Caller holds
+// c->mtx with the context's device current, and keeps `wide` (the bodies widened to u32, the copy's source) until the stream is past it.
+int expand_ct_rows(bfhe_ctx *c, const CtBlob &b, u32 *d_rows, std::vector<u32> &wide);
+// BFHE_ERR_ARG, "<what> is not memory of device d", unless p is device (or managed) memory of the context's device
+int check_device_buffer(const bfhe_ctx *c, const void *p, const char *what);
 } // namespace bfhe

@@ -47,6 +47,14 @@ int launch_ksk_expand(const MaskKey &key, const void *d_bodies, void *d_ksk, int
   return (int)cudaGetLastError();
 }
 
+// Fresh ciphertexts of a BFHECTS1 blob: with baseKS = dKS = 1 the KSK layout is `count` plain rows and row i is mask row i, so the same
+// kernel writes them (mask words mod q below n, the body at n, zero padding up to the stride).
+int launch_ct_expand(const MaskKey &key, const u32 *d_bodies, u32 *d_rows, size_t count, u32 n, u32 stride, u32 q, void *stream) {
+  if (count == 0) return 0;
+  if (count > 0xffffffffu) return (int)cudaErrorInvalidValue;
+  return launch_ksk_expand(key, d_bodies, d_rows, 4, (u32)count, 1, 1, n, stride, q, stream);
+}
+
 // BK: `pairs` (mask, body) polynomial pairs of the coefficient-form key in BFHEKEY1 order, the first with mask number p_first (stream id
 // 2^40 + p_first).  Polynomial 2s of the staging buffer gets mask p_first + s, polynomial 2s + 1 gets body s of d_bodies.
 __global__ void __launch_bounds__(256) bk_mask_expand_kernel(const MaskKey key, const u32 *__restrict__ bodies, u32 *__restrict__ stage,

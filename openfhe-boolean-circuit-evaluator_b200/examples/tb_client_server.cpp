@@ -1,21 +1,25 @@
 // tb_client_server.cpp -- evaluation without the secret key, through host/binfhecontext.h and host/circuit.h.
 // The key holder (client) generates the keys on the host and hands the evaluator (server) the evaluation keys only; the evaluator runs
 // an adder circuit on the holder's ciphertexts on the GPU and returns ciphertexts; the holder decrypts and checks them against a ripple
-// adder computed in plain C++.  Exit code 0 and "ALL PASSED" when every check passes.
-//     usage: tb_client_server <adder .out file> [-s TOY|STD128_OPT] [-m AP|GINX] [-n loops]
+// adder computed in plain C++.  Exit code 0 and "ALL PASSED" when every check passes.  With -c the holder sends each test's inputs as
+// one compact blob (BinFHEContext::EncryptCompact, both buses concatenated in SetInput's order) instead of one full row per bit.
+//     usage: tb_client_server <adder .out file> [-s TOY|STD128_OPT] [-m AP|GINX] [-n loops] [-c]
 #include "../host/circuit.h"
 #include <cstdio>
 #include <cstring>
 
 int main(int argc, char **argv) {
-  if (argc < 2) { std::fprintf(stderr, "usage: %s <adder .out file> [-s set] [-m method] [-n loops]\n", argv[0]); return 2; }
+  if (argc < 2) { std::fprintf(stderr, "usage: %s <adder .out file> [-s set] [-m method] [-n loops] [-c]\n", argv[0]); return 2; }
   lbcrypto::BINFHE_PARAMSET set = lbcrypto::STD128_OPT;
   lbcrypto::BINFHE_METHOD method = lbcrypto::GINX;
   unsigned loops = 4;
-  for (int i = 2; i + 1 < argc; i += 2) {
-    if (!std::strcmp(argv[i], "-s")) set = !std::strcmp(argv[i + 1], "TOY") ? lbcrypto::TOY : lbcrypto::STD128_OPT;
-    else if (!std::strcmp(argv[i], "-m")) method = !std::strcmp(argv[i + 1], "AP") ? lbcrypto::AP : lbcrypto::GINX;
-    else if (!std::strcmp(argv[i], "-n")) loops = (unsigned)std::atoi(argv[i + 1]);
+  bool compact = false;
+  for (int i = 2; i < argc; i++) {
+    if (!std::strcmp(argv[i], "-c")) compact = true;
+    else if (i + 1 >= argc) break;
+    else if (!std::strcmp(argv[i], "-s")) set = !std::strcmp(argv[++i], "TOY") ? lbcrypto::TOY : lbcrypto::STD128_OPT;
+    else if (!std::strcmp(argv[i], "-m")) method = !std::strcmp(argv[++i], "AP") ? lbcrypto::AP : lbcrypto::GINX;
+    else if (!std::strcmp(argv[i], "-n")) loops = (unsigned)std::atoi(argv[++i]);
   }
   // key holder: no GPU needed, keys from OS entropy
   lbcrypto::BinFHEContext holder;
@@ -39,12 +43,9 @@ int main(int argc, char **argv) {
   for (unsigned t = 0; t < loops; t++) {
     srand(t);
     std::vector<unsigned> in1(n), in2(n);
-    std::vector<std::vector<lbcrypto::LWECiphertext>> cts(2);
     for (unsigned ix = 0; ix < n; ix++) {
       in1[ix] = rand() % 2;
       in2[ix] = rand() % 2;
-      cts[0].push_back(holder.Encrypt(sk, in1[ix], lbcrypto::FRESH)); // level 0 of the circuit bootstraps them
-      cts[1].push_back(holder.Encrypt(sk, in2[ix], lbcrypto::FRESH));
     }
     std::vector<unsigned> golden(n + 1, 0);
     unsigned c = 0;
@@ -56,7 +57,18 @@ int main(int argc, char **argv) {
     golden[n] = c;
     circ.Reset();
     circ.setEncrypted(true);
-    circ.SetInput(cts);
+    if (compact) {
+      std::vector<uint8_t> bits(in1.begin(), in1.end());
+      bits.insert(bits.end(), in2.begin(), in2.end());
+      circ.SetInputCompact(holder.EncryptCompact(sk, bits));
+    } else {
+      std::vector<std::vector<lbcrypto::LWECiphertext>> cts(2);
+      for (unsigned ix = 0; ix < n; ix++) {
+        cts[0].push_back(holder.Encrypt(sk, in1[ix], lbcrypto::FRESH)); // level 0 of the circuit bootstraps them
+        cts[1].push_back(holder.Encrypt(sk, in2[ix], lbcrypto::FRESH));
+      }
+      circ.SetInput(cts);
+    }
     const std::vector<lbcrypto::LWECiphertext> out = circ.ClockCiphertexts();
     bool ok = out.size() == n + 1;
     for (unsigned ix = 0; ok && ix <= n; ix++) {

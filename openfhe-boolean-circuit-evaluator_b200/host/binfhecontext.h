@@ -69,6 +69,13 @@ public:
     if (output == FRESH || !m_bootstrap_inputs) return ct;
     return Bootstrap(ct); // OpenFHE's default output = BOOTSTRAPPED
   }
+  // fresh encryptions of bits[i] % 4 as one BFHECTS1 blob (bfhe_encrypt_compact): a public mask seed and one body per bit, for
+  // Circuit::SetInputCompact on an evaluator.  seed 0 (default): OS entropy.
+  std::vector<uint8_t> EncryptCompact(ConstLWEPrivateKey, const std::vector<uint8_t> &bits, uint64_t seed = 0) const {
+    std::vector<uint8_t> blob(bfhe_ct_compact_size(raw(), bits.size()));
+    check(bfhe_encrypt_compact(raw(), bits.data(), bits.size(), seed, blob.data(), blob.size()));
+    return blob;
+  }
   void Decrypt(ConstLWEPrivateKey, ConstLWECiphertext ct, LWEPlaintext *result) const {
     uint8_t r = 0;
     check(bfhe_decrypt(raw(), ct->row.data(), 1, &r));

@@ -1172,8 +1172,10 @@ extern "C" int bfhe_circuit_reset(bfhe_circuit *c) {
 // The common tail of SetInput on bits and on ciphertexts, once the fresh rows are enqueued on the launch stream: broadcast rank 0's
 // rows [fresh_base, +bcast_words) where the ranks' rows may differ, bootstrap the flip-flops' power-up values into the latch rows,
 // synchronise.  ct: the rows came from outside the program; the status word after the slab's last row holds the lowest row the
-// ingest rejected (0xffffffff: none), and a rejected input leaves the circuit without input.
-static int commit_input(bfhe_circuit *c, bool init_state, size_t bcast_words, bool ct) {
+// ingest rejected (INGEST_OK: none), or INGEST_REJECTED | -code when rank 0 refused its compact blob on the host (reject_msg there;
+// empty on the other ranks).  A rejected input leaves the circuit without input.
+static constexpr u32 INGEST_OK = 0xffffffffu, INGEST_REJECTED = 0xfffffff0u;
+static int commit_input(bfhe_circuit *c, bool init_state, size_t bcast_words, bool ct, const std::string &reject_msg = std::string()) {
   bfhe_ctx *x = c->ctx;
   const size_t st = x->p.ct_stride;
   if (bcast_words) {
@@ -1191,10 +1193,14 @@ static int commit_input(bfhe_circuit *c, bool init_state, size_t bcast_words, bo
     if (rc) return rc;
     c->state_init_pending = false;
   }
-  u32 bad_row = 0xffffffffu;
+  u32 bad_row = INGEST_OK;
   if (ct) BFHE_CUDA(cudaMemcpyAsync(&bad_row, c->slab + (size_t)c->total_rows * st, sizeof bad_row, cudaMemcpyDeviceToHost, x->stream));
   BFHE_CUDA(cudaStreamSynchronize(x->stream));
-  if (bad_row != 0xffffffffu) {
+  if (bad_row != INGEST_OK && bad_row >= INGEST_REJECTED) {
+    set_error(reject_msg.empty() ? "SetInput: rank 0 rejected its compact input blob" : reject_msg);
+    return -(int)(bad_row & 0xf);
+  }
+  if (bad_row != INGEST_OK) {
     set_error("SetInput: input ciphertext row " + std::to_string(bad_row) + " has a word >= q");
     return BFHE_ERR_FORMAT;
   }
@@ -1247,7 +1253,13 @@ extern "C" int bfhe_circuit_set_input(bfhe_circuit *c, const uint8_t *bits, size
   return BFHE_OK;
 }
 
-extern "C" int bfhe_circuit_set_input_ct(bfhe_circuit *c, const uint32_t *cts, size_t nbits, int on_device) {
+// SetInput on ciphertexts, one body for both input forms; they differ only in how the fresh input rows are filled.  blob == nullptr: nbits
+// full rows from cts (host, or device memory when on_device), copied in and checked by ct_ingest_kernel.  Else a BFHECTS1 blob that the
+// caller already checked on the host (read_ct_blob; nbits = its count): the masks are generated straight into the fresh rows.
+// reject != 0: the source rank refused its blob with that code (message reject_msg).  A single rank returns it at once; a sharded circuit
+// still takes part in the broadcast, with the refusal in the status word, so every rank returns the same code and none waits alone.
+static int set_input_ciphertexts(bfhe_circuit *c, size_t nbits, const uint32_t *cts, int on_device, const CtBlob *blob, int reject,
+                                 const std::string &reject_msg) {
   if (!c) return BFHE_ERR_ARG;
   if (!c->loaded) { set_error("SetInput before a netlist was loaded"); return BFHE_ERR_STATE; }
   if (!c->encrypted || c->plaintext || c->verify) {
@@ -1259,13 +1271,19 @@ extern "C" int bfhe_circuit_set_input_ct(bfhe_circuit *c, const uint32_t *cts, s
     int rc = replan(c);
     if (rc) return rc;
   }
-  if (nbits != c->n_in) { set_error("SetInput: expected " + std::to_string(c->n_in) + " ciphertexts, got " + std::to_string(nbits)); return BFHE_ERR_ARG; }
   const bool source = c->world == 1 || c->rank == 0; // sharded: rank 0's rows are used, the other ranks' buffers are not read
-  if (source && !cts && nbits) { set_error("SetInput: null ciphertext buffer"); return BFHE_ERR_ARG; }
+  std::string msg = reject_msg;
+  if (!reject && (source || !blob) && nbits != c->n_in) {
+    msg = "SetInput: expected " + std::to_string(c->n_in) + " ciphertexts, got " + std::to_string(nbits);
+    if (!blob || c->world == 1) { set_error(msg); return BFHE_ERR_ARG; }
+    reject = BFHE_ERR_ARG; // only rank 0 knows its blob's count: the other ranks learn of it through the broadcast
+  }
+  if (!reject && source && !blob && !cts && nbits) { set_error("SetInput: null ciphertext buffer"); return BFHE_ERR_ARG; }
   c->in_bits_set.clear();
   c->ct_input = true;
   c->has_input = false;
   c->done = false;
+  if (reject && c->world == 1) { set_error(msg); return reject; }
   if (!c->dev_ready) {
     int rc = upload_plan(c);
     if (rc) return rc;
@@ -1276,29 +1294,50 @@ extern "C" int bfhe_circuit_set_input_ct(bfhe_circuit *c, const uint32_t *cts, s
   BFHE_CUDA(cudaSetDevice(x->device));
   const size_t st = x->p.ct_stride;
   const bool init_state = c->state_init_pending && c->n_dff > 0;
+  u32 status_word = INGEST_OK;
+  std::vector<u32> wide; // the compact bodies as uploaded; commit_input synchronises before they go
   if (source) {
-    if (on_device && nbits) {
-      cudaPointerAttributes pa{};
-      if (cudaPointerGetAttributes(&pa, cts) != cudaSuccess || (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) ||
-          pa.device != x->device) {
-        cudaGetLastError();
-        set_error("SetInput: the ciphertext buffer is not memory of device " + std::to_string(x->device));
-        return BFHE_ERR_ARG;
-      }
-    }
+    if (!reject && !blob && on_device && nbits)
+      if (int rc = check_device_buffer(x, cts, "SetInput: the ciphertext buffer")) return rc;
     u32 *fresh = c->slab + (size_t)c->fresh_base * st, *status = c->slab + (size_t)c->total_rows * st;
-    if (nbits)
-      BFHE_CUDA(cudaMemcpyAsync(fresh, cts, nbits * st * 4, on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, x->stream));
-    BFHE_CUDA(cudaMemsetAsync(status, 0xff, sizeof(u32), x->stream));
-    int rc = launch_ct_ingest(x->P, fresh, (int)nbits, status, x->stream);
-    if (rc) return cuda_fail((cudaError_t)rc, "ct_ingest launch");
+    if (reject) {
+      status_word = INGEST_REJECTED | (u32)-reject;
+    } else if (blob) {
+      int rc = expand_ct_rows(x, *blob, fresh, wide);
+      if (rc) return rc;
+    } else {
+      if (nbits)
+        BFHE_CUDA(cudaMemcpyAsync(fresh, cts, nbits * st * 4, on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, x->stream));
+      BFHE_CUDA(cudaMemsetAsync(status, 0xff, sizeof(u32), x->stream));
+      int rc = launch_ct_ingest(x->P, fresh, (int)nbits, status, x->stream);
+      if (rc) return cuda_fail((cudaError_t)rc, "ct_ingest launch");
+    }
+    if (reject || blob) BFHE_CUDA(cudaMemcpyAsync(status, &status_word, sizeof status_word, cudaMemcpyHostToDevice, x->stream));
     // no secret key, no Encrypt(0): flip-flops power up from the trivial encryption of 0.  The rows may still hold a bit-path
     // SetInput's Encrypt(0).
     if (init_state) BFHE_CUDA(cudaMemsetAsync(c->slab + (size_t)c->dff_fresh_base * st, 0, (size_t)c->n_dff * st * 4, x->stream));
   }
   // sharded: the input rows, the flip-flops' fresh rows and the status word are adjacent (build_plan_cap, upload_plan)
   const size_t bcast = c->world > 1 ? ((size_t)c->n_in + c->n_dff) * st + 1 : 0;
-  return commit_input(c, init_state, bcast, true);
+  return commit_input(c, init_state, bcast, true, source ? msg : std::string());
+}
+
+extern "C" int bfhe_circuit_set_input_ct(bfhe_circuit *c, const uint32_t *cts, size_t nbits, int on_device) {
+  return set_input_ciphertexts(c, nbits, cts, on_device, nullptr, BFHE_OK, std::string());
+}
+
+extern "C" int bfhe_circuit_set_input_compact(bfhe_circuit *c, const void *blob, size_t len) {
+  if (!c) return BFHE_ERR_ARG;
+  // every host check of the blob, on the rank whose blob is read, before any device work; the other ranks' blobs are not read
+  CtBlob b;
+  int reject = BFHE_OK;
+  std::string msg;
+  if (c->world == 1 || c->rank == 0) {
+    if (!blob) set_error("SetInput: null compact blob");
+    reject = blob ? read_ct_blob(c->ctx, blob, len, b) : BFHE_ERR_ARG;
+    if (reject) msg = bfhe_last_error();
+  }
+  return set_input_ciphertexts(c, b.count, nullptr, 0, &b, reject, msg);
 }
 
 // Circuit::Clock.  out_cts == nullptr: the outputs are decrypted into out_bits (cap bits); else they stay encrypted and go to out_cts

@@ -106,6 +106,9 @@ public:
       }
     check(bfhe_circuit_set_input_ct(h, rows.data(), rows.size() / st, 0));
   }
+  // SetInput from a BFHECTS1 blob (BinFHEContext::EncryptCompact, buses concatenated in SetInput's order): the masks are generated on
+  // the GPU.  Evaluation keys only; throws std::runtime_error on failure (a malformed blob, wrong count, wrong mode).
+  void SetInputCompact(const std::vector<uint8_t> &blob) { check(bfhe_circuit_set_input_compact(h, blob.data(), blob.size())); }
   void setPlaintext(bool f) { plaintext_flag = f; push_flags(); }
   bool getPlaintext() const { return plaintext_flag; }
   void setEncrypted(bool f) { encrypted_flag = f; push_flags(); }

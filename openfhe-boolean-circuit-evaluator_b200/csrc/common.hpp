@@ -44,39 +44,47 @@ struct DevGate {
 enum : u32 { OP_OR = 0, OP_AND = 1, OP_NOR = 2, OP_NAND = 3, OP_XOR_FAST = 4, OP_XNOR_FAST = 5, OP_XOR = 6, OP_XNOR = 7,
              OP_BOOTSTRAP = 8, OP_NEG0 = 0x100, OP_NEG1 = 0x200 };
 
-struct LaunchInfo { // filled by the launch helpers for the profiler hooks
-  int gates_per_cta;
-  int ctas;
-  size_t smem_bytes;
+// blind-rotation kernel forms; the values are the ones the test hook bfhe_dbg_set_gates_per_cta takes (THRn: n gates per CTA)
+enum class Form : int {
+  AUTO = 0,  // the launch's own choice by gate count
+  THR1 = 1,  // throughput form, 1, 2 or 4 gates per CTA
+  THR2 = 2,
+  THR4 = 4,
+  LAT = 8,   // latency form: one gate per CTA, TMA-staged key
+  CL2 = 32,  // one gate on a 2-CTA cluster (kernels_v2.cu)
+  CL4 = 128, // one gate on a 4-CTA cluster, slot-sliced (kernels_cl.cu)
+};
+// whether this parameter set has the form (parameters only: a circuit plans before the keys are on the device).  AUTO: some form exists.
+bool form_supported(const DevConst &P, int method_ap, Form f);
+
+// the device key set: everything the blind rotation and the key switch read.  A view; bfhe_ctx owns the buffers.  Null where the parameter
+// set has no use for a copy, and the key copies are null until the keys are uploaded.
+struct DevKeys {
+  const u32 *bk = nullptr;   // bootstrapping key in device form (bk_convert)
+  const u32 *bkf = nullptr;  // GINX throughput kernel at the STD128_OPT shape: bk with the top digit folded in (launch_bk_fold)
+  const u32 *bk4 = nullptr;  // 2-CTA cluster form: bk rows in kernels_v2.cu's physical slot order, split [step][quarter of the slots][polynomial][N/4]
+  const u32 *bkx = nullptr;  // 4-CTA cluster form (kernels_cl.cu): bk as [step][rank][polynomial][N/4]
+  const u32 *twl = nullptr;  // fwd w | fwd ws | inv w | inv ws, each N words: per-lane twiddles of the narrow pass
+  const u32 *psiM = nullptr; // psi^k in Montgomery form, k < 2N
+  const u32 *tw2 = nullptr;  // 2-CTA cluster form: fwd w | fwd ws | inv w | inv ws, each N words (order: kernels_v2.cu Tabs)
+  const u32 *F = nullptr;    // (psi^k - 1) * 2^32 mod Q, k < 2N: read by the 2-CTA form and by the GINX 4-CTA form
+  const u32 *twx = nullptr;  // 4-CTA cluster form: its per-rank twiddle blocks
+  const void *ksk = nullptr; // key-switching key, [i][digit][digit value][row], ksk_elem_bytes per element
+  int ksk_elem_bytes = 4;
 };
 
-// derived key copies and tables of the cluster kernels (kernels_v2.cu, kernels_cl.cu) and of the GINX throughput kernel (d_bkf); each null
-// when the parameter set is not covered
-struct V2Bufs {
-  const u32 *d_bk4 = nullptr; // bootstrapping key, rows in kernels_v2.cu's physical slot order, split [step][quarter of the slots][polynomial][N/4]
-  const u32 *d_tw2 = nullptr; // fwd w | fwd ws | inv w | inv ws, each N words (order: kernels_v2.cu Tabs)
-  const u32 *d_F = nullptr;   // (psi^k - 1) * 2^32 mod Q, k < 2N
-  const u32 *d_bkx = nullptr; // slot-sliced 4-CTA cluster kernel (kernels_cl.cu): key as [step][rank][polynomial][N/4]
-  const u32 *d_twx = nullptr; // ... and its per-rank twiddle blocks
-  const u32 *d_bkf = nullptr; // STD128_OPT-shape GINX throughput kernel (kernels.cu): d_bk with the top digit folded in (launch_bk_fold)
-};
-
-// kernels.cu entry points (all asynchronous on `stream`; return cudaError_t as int)
-// force_gates_per_cta: 0 = cost model; 1, 2, 4 = throughput form; 8 = latency form; 32 = cluster latency form (one gate on two SMs);
-// 128 = one gate on four SMs, slot-sliced (kernels_cl.cu).  (16 and 64 named two round-1 forms that no longer exist: invalid value.)
-int launch_blind_rotate(const DevConst &P, int method_ap, const DevGate *d_gates, int count, const u32 *d_bk,
-                        const u32 *d_twl /*fwd w | fwd ws | inv w | inv ws, each N words*/, const u32 *d_psiM,
-                        u32 *d_ext /*count * (N+4)*/, u32 *d_acc_dbg /*nullable: count*2*N*/, int force_gates_per_cta,
-                        void *stream, LaunchInfo *info, const V2Bufs *v2 = nullptr);
+// kernels.cu entry points (all asynchronous on `stream`; return cudaError_t as int).  A form this parameter set lacks: cudaErrorInvalidValue.
+int launch_blind_rotate(const DevConst &P, int method_ap, const DevGate *d_gates, int count, const DevKeys &keys,
+                        u32 *d_ext /*count * (N+4)*/, u32 *d_acc_dbg /*nullable: count*2*N*/, Form form, void *stream);
 // kernels_v2.cu
-bool v2_supported(const DevConst &P, int method_ap);
+bool cl2_supported(const DevConst &P, int method_ap); // parameters of the 2-CTA cluster form
 int v2_set_attrs();
 int launch_bk_permute_v2(const u32 *d_src, u32 *d_dst, size_t npoly, void *stream);
 int cl2_max_gates(); // gates the cluster form can run concurrently on this device (0 = unavailable)
 int launch_bk_split_cl4(const u32 *d_src, u32 *d_dst, size_t npoly, void *stream);
 // one gate on a 2-CTA cluster (two SMs): the latency form for wavefronts narrower than half the SM count
-int launch_blind_rotate_cl2(const DevConst &P, const DevGate *d_gates, int count, const V2Bufs &vb, u32 *d_ext, u32 *d_acc_dbg,
-                            void *stream, LaunchInfo *info);
+int launch_blind_rotate_cl2(const DevConst &P, const DevGate *d_gates, int count, const DevKeys &keys, u32 *d_ext, u32 *d_acc_dbg,
+                            void *stream);
 // kernels_cl.cu: one gate on a 4-CTA cluster, everything sliced by evaluation slot, one exchange per step
 bool clx_supported(const DevConst &P, int method_ap);
 size_t clx_tw_words();
@@ -84,8 +92,8 @@ int clx_set_attrs();
 int clx_max_gates();  // 4-CTA clusters the device keeps co-resident
 int clx_fast_gates(); // up to this many gates the 4-CTA form runs all clusters in one round at full speed
 int launch_bk_slice_clx(const u32 *d_src, u32 *d_dst, size_t npoly, int method_ap, void *stream);
-int launch_blind_rotate_clx(const DevConst &P, int method_ap, const DevGate *d_gates, int count, const V2Bufs &vb, u32 *d_ext,
-                            u32 *d_acc_dbg, void *stream, LaunchInfo *info);
+int launch_blind_rotate_clx(const DevConst &P, int method_ap, const DevGate *d_gates, int count, const DevKeys &keys, u32 *d_ext,
+                            u32 *d_acc_dbg, void *stream);
 // Multi-GPU exchange fused into the key switch (SURVEY 8(e)): every output ciphertext is stored into every rank's wire slab (the peers'
 // slabs are mapped through CUDA IPC, the stores travel over NVLink), and the last CTA of the launch raises this rank's flag in every
 // peer's flag array.  Flag values only grow: value(epoch, index) = epoch * per_epoch + index + 1, `epoch` read from device memory so
@@ -98,8 +106,8 @@ struct PeerX {
   const u32 *epoch = nullptr;  // local: Clock() count
   u32 world = 1, rank = 0, index = 0, per_epoch = 1;
 };
-int launch_keyswitch(const DevConst &P, const u32 *d_ext, const DevGate *d_gates, int count, const void *d_ksk,
-                     int ksk_elem_bytes, void *stream, const PeerX *px = nullptr);
+int launch_keyswitch(const DevConst &P, const u32 *d_ext, const DevGate *d_gates, int count, const DevKeys &keys, void *stream,
+                     const PeerX *px = nullptr);
 // exchange plumbing (one tiny launch each): epoch += 1; wait until every peer's flag has reached value(epoch, index) -- index -1 = the
 // end-of-Clock signal of the previous epoch -- with a timeout (30 s, BFHE_EXCHANGE_TIMEOUT_S) that sets *err instead of hanging; raise my flag at every peer
 int launch_peer_epoch_bump(u32 *epoch, void *stream);

@@ -50,6 +50,89 @@ static size_t pad8(size_t x) { return (x + 7) & ~(size_t)7; }
 // -------------------------------------------------------------------------------------------------
 static u32 shoup32(u64 w, u64 Q) { return (u32)((w << 32) / Q); }
 
+// the device side of a new context: the kernels' tables, the per-call buffers, the side stream and the events
+static int init_device(bfhe_ctx *c) {
+  const u32 N = c->p.N;
+  const u64 Q = c->p.Q;
+  const int ap = c->p.method == BFHE_AP;
+  // per-lane twiddle tables of the narrow pass: [chunk][lane][4]; entry p = groups + gi is
+  // psi^bitrev(groups*(32 + lane) + gi)  (see kernels.cu ct_pass)
+  const u32 E = N / 32;
+  std::vector<u32> tl(4 * (size_t)N, 0);
+  for (u32 lane = 0; lane < 32; lane++)
+    for (u32 pp = 1; pp < E; pp++) {
+      u32 groups = 1;
+      while (groups * 2 <= pp) groups *= 2;
+      u32 gi = pp - groups, idx = groups * (32 + lane) + gi;
+      size_t off = ((size_t)(pp / 4) * 32 + lane) * 4 + (pp % 4);
+      tl[off] = c->hntt.tw[idx]; tl[N + off] = shoup32(c->hntt.tw[idx], Q);
+      tl[2 * N + off] = c->hntt.itw[idx]; tl[3 * N + off] = shoup32(c->hntt.itw[idx], Q);
+    }
+  std::vector<u32> psiM(2 * (size_t)N);
+  u64 cur = (1ull << 32) % Q; // Montgomery form of psi^0
+  for (u32 k = 0; k < 2 * N; k++) { psiM[k] = (u32)cur; cur = mulmod64(cur, c->psi, Q); }
+  BFHE_CUDA(upload(c->d_twl, tl));
+  BFHE_CUDA(upload(c->d_psiM, psiM));
+  BFHE_CUDA(c->d_gates.alloc(bfhe_ctx::CHUNK));
+  BFHE_CUDA(c->d_ext.alloc(bfhe_ctx::CHUNK * (size_t)(N + 4)));
+  BFHE_CUDA(c->d_gates_b.alloc(bfhe_ctx::CHUNK));
+  BFHE_CUDA(c->d_ext_b.alloc(bfhe_ctx::CHUNK * (size_t)(N + 4)));
+  BFHE_CUDA(cudaStreamCreateWithFlags(&c->ks_stream, cudaStreamNonBlocking));
+  for (int i = 0; i < 2; i++) {
+    BFHE_CUDA(cudaEventCreateWithFlags(&c->ev_br[i], cudaEventDisableTiming));
+    BFHE_CUDA(cudaEventCreateWithFlags(&c->ev_ks[i], cudaEventDisableTiming));
+    BFHE_CUDA(c->h_gates[i].alloc(bfhe_ctx::CHUNK));
+    BFHE_CUDA(cudaEventCreateWithFlags(&c->stage_ev[i], cudaEventDisableTiming));
+  }
+  if (form_supported(c->P, ap, Form::CL2)) { // tables of the 2-CTA cluster form (F is read by the GINX 4-CTA form too)
+    std::vector<u32> t2(4 * (size_t)N), F(2 * (size_t)N);
+    for (u32 k = 0; k < N; k++) { // natural order, last stage de-interleaved (kernels_v2.cu load_tw_narrow)
+      u32 d = k;
+      if (k >= N / 2) { const u32 i = k - N / 2, t = i >> 3, j = i & 7; d = N / 2 + (N / 4) * (j >> 2) + 4 * t + (j & 3); }
+      t2[d] = c->hntt.tw[k]; t2[N + d] = shoup32(c->hntt.tw[k], Q);
+      t2[2 * N + d] = c->hntt.itw[k]; t2[3 * N + d] = shoup32(c->hntt.itw[k], Q);
+    }
+    const u64 oneM = (1ull << 32) % Q;
+    for (u32 k = 0; k < 2 * N; k++) // (psi^k - 1) in Montgomery form
+      F[f_index(k)] = (u32)((psiM[k] + Q - oneM) % Q);
+    BFHE_CUDA(upload(c->d_tw2, t2));
+    BFHE_CUDA(upload(c->d_F, F));
+  }
+  if (form_supported(c->P, ap, Form::CL4)) { // per-rank twiddle blocks of the slot-sliced cluster kernel (layout: kernels_cl.cu TWF / TWI)
+    // CTA k runs the sub-transform of block k (in-place positions 256 k + i, i < 256) as: pass A (lane holds i = lane + 32 m),
+    // pass B (lane = 4 blk + q holds i = 32 blk + q + 4 m), pass C (lane holds i = 8 lane + j).  A stage with G groups uses tw[G + group],
+    // group = position / (N / G) -- the table order of HostNtt (tw[k] = psi^bitrev(k)).  The inverse runs the five narrowest stages
+    // as shuffles in the external-product threads (slot t = position t) and the three widest in pass-A layout.
+    const size_t TWF = 8 + 2 * 256, TWI = 8 + 5 * 256, TWR = 2 * TWF + 2 * TWI;
+    std::vector<u32> tx(clx_tw_words(), 0);
+    for (u32 k = 0; k < 4; k++) {
+      u32 *fw = tx.data() + (size_t)k * TWR, *fws = fw + TWF, *iw = fw + 2 * TWF, *iws = iw + TWI;
+      auto putf = [&](size_t off, u32 idx) { fw[off] = c->hntt.tw[idx]; fws[off] = shoup32(c->hntt.tw[idx], Q); };
+      auto puti = [&](size_t off, u32 idx) { iw[off] = c->hntt.itw[idx]; iws[off] = shoup32(c->hntt.itw[idx], Q); };
+      putf(1, 4 + k); puti(1, 4 + k);
+      for (u32 g = 0; g < 2; g++) { putf(2 + g, 8 + 2 * k + g); puti(2 + g, 8 + 2 * k + g); }
+      for (u32 g = 0; g < 4; g++) { putf(4 + g, 16 + 4 * k + g); puti(4 + g, 16 + 4 * k + g); }
+      for (u32 lane = 0; lane < 32; lane++) {
+        const u32 blk = lane >> 2;
+        auto at = [&](int s, u32 e) { return 8 + 256 * (size_t)s + ((size_t)(e >> 2) * 32 + lane) * 4 + (e & 3); }; // [chunk][lane][4]
+        putf(at(0, 1), 32 + 8 * k + blk);
+        for (u32 g = 0; g < 2; g++) putf(at(0, 2 + g), 64 + 16 * k + 2 * blk + g);
+        for (u32 g = 0; g < 4; g++) putf(at(0, 4 + g), 128 + 32 * k + 4 * blk + g);
+        for (u32 g = 0; g < 2; g++) putf(at(1, 2 + g), 256 + 64 * k + 2 * lane + g);
+        for (u32 g = 0; g < 4; g++) putf(at(1, 4 + g), 512 + 128 * k + 4 * lane + g);
+      }
+      for (u32 s5 = 0; s5 < 5; s5++)
+        for (u32 t = 0; t < 256; t++) puti(8 + 256 * (size_t)s5 + t, (512u >> s5) + ((256 * k + t) >> (s5 + 1)));
+    }
+    BFHE_CUDA(upload(c->d_twx, tx));
+  }
+  int sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device);
+  c->chunk = std::max<size_t>(1, bfhe_ctx::CHUNK / (4 * (size_t)sms)) * 4 * (size_t)sms; // whole waves of 4-gate CTAs
+  if (c->chunk > bfhe_ctx::CHUNK) c->chunk = bfhe_ctx::CHUNK;
+  return BFHE_OK;
+}
+
 extern "C" bfhe_ctx *bfhe_create(int paramset, int method, int device) {
   bfhe_params p{};
   p.paramset = paramset;
@@ -131,89 +214,7 @@ extern "C" bfhe_ctx *bfhe_create(int paramset, int method, int device) {
       return nullptr;
     }
     c->stream = c->own_stream;
-    // per-lane twiddle tables of the narrow pass: [chunk][lane][4]; entry p = groups + gi is
-    // psi^bitrev(groups*(32 + lane) + gi)  (see kernels.cu ct_pass)
-    const u32 E = N / 32;
-    std::vector<u32> tl(4 * (size_t)N, 0);
-    for (u32 lane = 0; lane < 32; lane++)
-      for (u32 pp = 1; pp < E; pp++) {
-        u32 groups = 1;
-        while (groups * 2 <= pp) groups *= 2;
-        u32 gi = pp - groups, idx = groups * (32 + lane) + gi;
-        size_t off = ((size_t)(pp / 4) * 32 + lane) * 4 + (pp % 4);
-        tl[off] = c->hntt.tw[idx]; tl[N + off] = shoup32(c->hntt.tw[idx], Q);
-        tl[2 * N + off] = c->hntt.itw[idx]; tl[3 * N + off] = shoup32(c->hntt.itw[idx], Q);
-      }
-    std::vector<u32> psiM(2 * (size_t)N);
-    u64 cur = (1ull << 32) % Q; // Montgomery form of psi^0
-    for (u32 k = 0; k < 2 * N; k++) { psiM[k] = (u32)cur; cur = mulmod64(cur, c->psi, Q); }
-    bool ok = cudaMalloc(&c->d_twl, tl.size() * 4) == cudaSuccess && cudaMalloc(&c->d_psiM, psiM.size() * 4) == cudaSuccess &&
-              cudaMemcpy(c->d_twl, tl.data(), tl.size() * 4, cudaMemcpyHostToDevice) == cudaSuccess &&
-              cudaMemcpy(c->d_psiM, psiM.data(), psiM.size() * 4, cudaMemcpyHostToDevice) == cudaSuccess &&
-              cudaMalloc(&c->d_gates, bfhe_ctx::CHUNK * sizeof(DevGate)) == cudaSuccess &&
-              cudaMalloc(&c->d_ext, bfhe_ctx::CHUNK * (size_t)(N + 4) * 4) == cudaSuccess &&
-              cudaMalloc(&c->d_gates_b, bfhe_ctx::CHUNK * sizeof(DevGate)) == cudaSuccess &&
-              cudaMalloc(&c->d_ext_b, bfhe_ctx::CHUNK * (size_t)(N + 4) * 4) == cudaSuccess &&
-              cudaStreamCreateWithFlags(&c->ks_stream, cudaStreamNonBlocking) == cudaSuccess &&
-              cudaEventCreateWithFlags(&c->ev_br[0], cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&c->ev_br[1], cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&c->ev_ks[0], cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&c->ev_ks[1], cudaEventDisableTiming) == cudaSuccess &&
-              cudaMallocHost(&c->h_gates[0], bfhe_ctx::CHUNK * sizeof(DevGate)) == cudaSuccess &&
-              cudaMallocHost(&c->h_gates[1], bfhe_ctx::CHUNK * sizeof(DevGate)) == cudaSuccess &&
-              cudaEventCreateWithFlags(&c->stage_ev[0], cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&c->stage_ev[1], cudaEventDisableTiming) == cudaSuccess;
-    if (ok && v2_supported(P, method == BFHE_AP)) { // tables of the second-generation throughput kernel
-      std::vector<u32> t2(4 * (size_t)N), F(2 * (size_t)N);
-      for (u32 k = 0; k < N; k++) { // natural order, last stage de-interleaved (kernels_v2.cu load_tw_narrow)
-        u32 d = k;
-        if (k >= N / 2) { const u32 i = k - N / 2, t = i >> 3, j = i & 7; d = N / 2 + (N / 4) * (j >> 2) + 4 * t + (j & 3); }
-        t2[d] = c->hntt.tw[k]; t2[N + d] = shoup32(c->hntt.tw[k], Q);
-        t2[2 * N + d] = c->hntt.itw[k]; t2[3 * N + d] = shoup32(c->hntt.itw[k], Q);
-      }
-      const u64 oneM = (1ull << 32) % Q;
-      for (u32 k = 0; k < 2 * N; k++) // (psi^k - 1) in Montgomery form
-        F[f_index(k)] = (u32)((psiM[k] + Q - oneM) % Q);
-      ok = cudaMalloc(&c->d_tw2, t2.size() * 4) == cudaSuccess && cudaMalloc(&c->d_F, F.size() * 4) == cudaSuccess &&
-           cudaMemcpy(c->d_tw2, t2.data(), t2.size() * 4, cudaMemcpyHostToDevice) == cudaSuccess &&
-           cudaMemcpy(c->d_F, F.data(), F.size() * 4, cudaMemcpyHostToDevice) == cudaSuccess;
-      c->v2.d_tw2 = c->d_tw2; c->v2.d_F = c->d_F;
-    }
-    if (ok && clx_supported(P, method == BFHE_AP)) { // per-rank twiddle blocks of the slot-sliced cluster kernel (layout: kernels_cl.cu TWF / TWI)
-      // CTA k runs the sub-transform of block k (in-place positions 256 k + i, i < 256) as: pass A (lane holds i = lane + 32 m),
-      // pass B (lane = 4 blk + q holds i = 32 blk + q + 4 m), pass C (lane holds i = 8 lane + j).  A stage with G groups uses tw[G + group],
-      // group = position / (N / G) -- the table order of HostNtt (tw[k] = psi^bitrev(k)).  The inverse runs the five narrowest stages
-      // as shuffles in the external-product threads (slot t = position t) and the three widest in pass-A layout.
-      const size_t TWF = 8 + 2 * 256, TWI = 8 + 5 * 256, TWR = 2 * TWF + 2 * TWI;
-      std::vector<u32> tx(clx_tw_words(), 0);
-      for (u32 k = 0; k < 4; k++) {
-        u32 *fw = tx.data() + (size_t)k * TWR, *fws = fw + TWF, *iw = fw + 2 * TWF, *iws = iw + TWI;
-        auto putf = [&](size_t off, u32 idx) { fw[off] = c->hntt.tw[idx]; fws[off] = shoup32(c->hntt.tw[idx], Q); };
-        auto puti = [&](size_t off, u32 idx) { iw[off] = c->hntt.itw[idx]; iws[off] = shoup32(c->hntt.itw[idx], Q); };
-        putf(1, 4 + k); puti(1, 4 + k);
-        for (u32 g = 0; g < 2; g++) { putf(2 + g, 8 + 2 * k + g); puti(2 + g, 8 + 2 * k + g); }
-        for (u32 g = 0; g < 4; g++) { putf(4 + g, 16 + 4 * k + g); puti(4 + g, 16 + 4 * k + g); }
-        for (u32 lane = 0; lane < 32; lane++) {
-          const u32 blk = lane >> 2;
-          auto at = [&](int s, u32 e) { return 8 + 256 * (size_t)s + ((size_t)(e >> 2) * 32 + lane) * 4 + (e & 3); }; // [chunk][lane][4]
-          putf(at(0, 1), 32 + 8 * k + blk);
-          for (u32 g = 0; g < 2; g++) putf(at(0, 2 + g), 64 + 16 * k + 2 * blk + g);
-          for (u32 g = 0; g < 4; g++) putf(at(0, 4 + g), 128 + 32 * k + 4 * blk + g);
-          for (u32 g = 0; g < 2; g++) putf(at(1, 2 + g), 256 + 64 * k + 2 * lane + g);
-          for (u32 g = 0; g < 4; g++) putf(at(1, 4 + g), 512 + 128 * k + 4 * lane + g);
-        }
-        for (u32 s5 = 0; s5 < 5; s5++)
-          for (u32 t = 0; t < 256; t++) puti(8 + 256 * (size_t)s5 + t, (512u >> s5) + ((256 * k + t) >> (s5 + 1)));
-      }
-      ok = cudaMalloc(&c->d_twx, tx.size() * 4) == cudaSuccess && cudaMemcpy(c->d_twx, tx.data(), tx.size() * 4, cudaMemcpyHostToDevice) == cudaSuccess;
-      c->v2.d_twx = c->d_twx;
-    }
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    c->chunk = std::max<size_t>(1, bfhe_ctx::CHUNK / (4 * (size_t)sms)) * 4 * (size_t)sms; // whole waves of 4-gate CTAs
-    if (c->chunk > bfhe_ctx::CHUNK) c->chunk = bfhe_ctx::CHUNK;
-    if (!ok) {
-      cuda_fail(cudaGetLastError(), "bfhe_create: device allocation");
+    if (init_device(c)) {
       bfhe_destroy(c);
       return nullptr;
     }
@@ -227,24 +228,15 @@ extern "C" void bfhe_destroy(bfhe_ctx *c) {
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     for (auto &s : c->spans) { cudaEventDestroy(s.a); cudaEventDestroy(s.b); }
-    cudaFree(c->d_bk); cudaFree(c->d_twl); cudaFree(c->d_psiM); cudaFree(c->d_ksk); cudaFree(c->d_gates); cudaFree(c->d_ext);
-    cudaFree(c->d_tmp); cudaFree(c->d_ptr_in); cudaFree(c->d_ptr_out); cudaFree(c->e2e_slab);
-    cudaFree(c->d_gates_b); cudaFree(c->d_ext_b);
-    cudaFree(c->d_bk4); cudaFree(c->d_tw2); cudaFree(c->d_F);
-    cudaFree(c->d_bkx); cudaFree(c->d_twx);
-    cudaFree(c->d_bkf);
     for (int i = 0; i < 2; i++) {
       if (c->ev_br[i]) cudaEventDestroy(c->ev_br[i]);
       if (c->ev_ks[i]) cudaEventDestroy(c->ev_ks[i]);
-    }
-    if (c->ks_stream) cudaStreamDestroy(c->ks_stream);
-    for (int i = 0; i < 2; i++) {
-      if (c->h_gates[i]) cudaFreeHost(c->h_gates[i]);
       if (c->stage_ev[i]) cudaEventDestroy(c->stage_ev[i]);
     }
+    if (c->ks_stream) cudaStreamDestroy(c->ks_stream);
     if (c->own_stream) cudaStreamDestroy(c->own_stream);
   }
-  delete c;
+  delete c; // the buffers' owners release them, with the context's device current
 }
 
 extern "C" int bfhe_get_params(const bfhe_ctx *c, bfhe_params *out) {
@@ -490,59 +482,50 @@ static int upload_keys(bfhe_ctx *c, u32 *dbg_bk, u8 *dbg_ksk) {
   const bfhe_params &p = c->p;
   const u32 N = p.N;
   const bool compact = compact_only(c);
-  cudaFree(c->d_bk); c->d_bk = nullptr;
-  cudaFree(c->d_ksk); c->d_ksk = nullptr;
-  BFHE_CUDA(cudaMalloc(&c->d_bk, c->bk_words * 4));
+  const int ap = p.method == BFHE_AP;
+  c->d_bk.reset(); c->d_bkf.reset(); c->d_bk4.reset(); c->d_bkx.reset(); c->d_ksk.reset();
+  BFHE_CUDA(c->d_bk.alloc(c->bk_words));
   { // convert in slices so the temporary coefficient-form copy stays small
     const size_t npoly = c->bk_words / N, slice = 1 << 15; // even: a slice holds whole (mask, body) pairs
-    u32 *d_coef = nullptr, *d_body = nullptr;
-    BFHE_CUDA(cudaMalloc(&d_coef, std::min(npoly, slice) * N * 4));
-    if (compact) BFHE_CUDA(cudaMalloc(&d_body, std::min(npoly, slice) / 2 * N * 4));
+    DevBuf<u32> coef, body;
+    BFHE_CUDA(coef.alloc(std::min(npoly, slice) * N));
+    if (compact) BFHE_CUDA(body.alloc(std::min(npoly, slice) / 2 * N));
     for (size_t p0 = 0; p0 < npoly; p0 += slice) {
       const size_t np = std::min(slice, npoly - p0);
       if (compact) {
-        BFHE_CUDA(cudaMemcpyAsync(d_body, c->bk_body.data() + p0 / 2 * N, np / 2 * N * 4, cudaMemcpyHostToDevice, c->stream));
-        int rc = launch_bk_mask_expand(c->mask_seed, d_body, d_coef, p0 / 2, np / 2, N, (u32)p.Q, c->stream);
+        BFHE_CUDA(cudaMemcpyAsync(body.get(), c->bk_body.data() + p0 / 2 * N, np / 2 * N * 4, cudaMemcpyHostToDevice, c->stream));
+        int rc = launch_bk_mask_expand(c->mask_seed, body.get(), coef.get(), p0 / 2, np / 2, N, (u32)p.Q, c->stream);
         if (rc) return cuda_fail((cudaError_t)rc, "bk_mask_expand");
-        if (dbg_bk) BFHE_CUDA(cudaMemcpyAsync(dbg_bk + p0 * N, d_coef, np * N * 4, cudaMemcpyDeviceToHost, c->stream));
+        if (dbg_bk) BFHE_CUDA(cudaMemcpyAsync(dbg_bk + p0 * N, coef.get(), np * N * 4, cudaMemcpyDeviceToHost, c->stream));
       } else {
-        BFHE_CUDA(cudaMemcpyAsync(d_coef, c->bk_coef.data() + p0 * N, np * N * 4, cudaMemcpyHostToDevice, c->stream));
+        BFHE_CUDA(cudaMemcpyAsync(coef.get(), c->bk_coef.data() + p0 * N, np * N * 4, cudaMemcpyHostToDevice, c->stream));
       }
-      int rc = launch_bk_convert(c->P, d_coef, c->d_bk + p0 * N, np, c->d_twl, c->stream);
+      int rc = launch_bk_convert(c->P, coef.get(), c->d_bk.get() + p0 * N, np, c->d_twl.get(), c->stream);
       if (rc) return cuda_fail((cudaError_t)rc, "bk_convert");
       BFHE_CUDA(cudaStreamSynchronize(c->stream));
     }
-    cudaFree(d_coef);
-    cudaFree(d_body);
   }
-  cudaFree(c->d_bk4); c->d_bk4 = nullptr; c->v2.d_bk4 = nullptr;
-  if (c->d_tw2 && v2_supported(c->P, p.method == BFHE_AP)) { // key copy of the 2-CTA cluster kernel: kernels_v2.cu's physical slot order
-    u32 *tmp = nullptr;                                        // (a temporary), split [step][quarter][polynomial][N/4]
-    BFHE_CUDA(cudaMalloc(&tmp, c->bk_words * 4));
-    int rc = launch_bk_permute_v2(c->d_bk, tmp, c->bk_words / N, c->stream);
-    if (rc) { cudaFree(tmp); return cuda_fail((cudaError_t)rc, "bk_permute_v2"); }
-    if (cudaMalloc(&c->d_bk4, c->bk_words * 4) != cudaSuccess) { cudaFree(tmp); return cuda_fail(cudaGetLastError(), "cudaMalloc(d_bk4)"); }
-    rc = launch_bk_split_cl4(tmp, c->d_bk4, c->bk_words / N, c->stream);
-    if (rc) { cudaFree(tmp); return cuda_fail((cudaError_t)rc, "bk_split_cl4"); }
+  if (form_supported(c->P, ap, Form::CL2)) { // key copy of the 2-CTA cluster kernel: kernels_v2.cu's physical slot order
+    DevBuf<u32> tmp;                         // (a temporary), split [step][quarter][polynomial][N/4]
+    BFHE_CUDA(tmp.alloc(c->bk_words));
+    int rc = launch_bk_permute_v2(c->d_bk.get(), tmp.get(), c->bk_words / N, c->stream);
+    if (rc) return cuda_fail((cudaError_t)rc, "bk_permute_v2");
+    BFHE_CUDA(c->d_bk4.alloc(c->bk_words));
+    rc = launch_bk_split_cl4(tmp.get(), c->d_bk4.get(), c->bk_words / N, c->stream);
+    if (rc) return cuda_fail((cudaError_t)rc, "bk_split_cl4");
     cudaStreamSynchronize(c->stream);
-    cudaFree(tmp);
-    c->v2.d_bk4 = c->d_bk4;
   }
-  cudaFree(c->d_bkx); c->d_bkx = nullptr; c->v2.d_bkx = nullptr;
-  if (c->d_twx && clx_supported(c->P, p.method == BFHE_AP)) { // key copy of the slot-sliced cluster kernel: [step][rank][polynomial][N/4]
-    BFHE_CUDA(cudaMalloc(&c->d_bkx, c->bk_words * 4));
-    int rc = launch_bk_slice_clx(c->d_bk, c->d_bkx, c->bk_words / N, p.method == BFHE_AP, c->stream);
+  if (form_supported(c->P, ap, Form::CL4)) { // key copy of the slot-sliced cluster kernel: [step][rank][polynomial][N/4]
+    BFHE_CUDA(c->d_bkx.alloc(c->bk_words));
+    int rc = launch_bk_slice_clx(c->d_bk.get(), c->d_bkx.get(), c->bk_words / N, ap, c->stream);
     if (rc) return cuda_fail((cudaError_t)rc, "bk_slice_clx");
     BFHE_CUDA(cudaStreamSynchronize(c->stream));
-    c->v2.d_bkx = c->d_bkx;
   }
-  cudaFree(c->d_bkf); c->d_bkf = nullptr; c->v2.d_bkf = nullptr;
-  if (bk_fold_supported(c->P, p.method == BFHE_AP)) { // key copy of the GINX throughput kernel: the top digit folded into the other rows
-    BFHE_CUDA(cudaMalloc(&c->d_bkf, c->bk_words * 4));
-    int rc = launch_bk_fold(c->P, c->d_bk, c->d_bkf, p.n, c->stream);
+  if (bk_fold_supported(c->P, ap)) { // key copy of the GINX throughput kernel at this shape: the top digit folded into the other rows
+    BFHE_CUDA(c->d_bkf.alloc(c->bk_words));
+    int rc = launch_bk_fold(c->P, c->d_bk.get(), c->d_bkf.get(), p.n, c->stream);
     if (rc) return cuda_fail((cudaError_t)rc, "bk_fold");
     BFHE_CUDA(cudaStreamSynchronize(c->stream));
-    c->v2.d_bkf = c->d_bkf;
   }
   { // KSK: [i][j(digit value)][k(digit index)][n+1]  ->  [i][k][j][rowlen]
     const u32 rowlen = c->ksk_elem_bytes == 2 ? 512 : p.ct_stride; // elements per padded row
@@ -559,24 +542,23 @@ static int upload_keys(bfhe_ctx *c, u32 *dbg_bk, u8 *dbg_ksk) {
             else std::memcpy(full + s * src_row, dev + d * dst_row, src_row);
           }
     };
-    BFHE_CUDA(cudaMalloc(&c->d_ksk, bytes));
     if (compact) {
-      void *d_kb = nullptr;
-      BFHE_CUDA(cudaMalloc(&d_kb, c->ksk_body.size()));
-      BFHE_CUDA(cudaMemcpyAsync(d_kb, c->ksk_body.data(), c->ksk_body.size(), cudaMemcpyHostToDevice, c->stream));
-      int rc = launch_ksk_expand(c->mask_seed, d_kb, c->d_ksk, c->ksk_elem_bytes, N, p.baseKS, p.dKS, p.n, rowlen, (u32)p.qKS, c->stream);
-      if (rc) { cudaFree(d_kb); return cuda_fail((cudaError_t)rc, "ksk_expand"); }
+      BFHE_CUDA(c->d_ksk.alloc(bytes));
+      DevBuf<u8> kb;
+      BFHE_CUDA(kb.alloc(c->ksk_body.size()));
+      BFHE_CUDA(cudaMemcpyAsync(kb.get(), c->ksk_body.data(), c->ksk_body.size(), cudaMemcpyHostToDevice, c->stream));
+      int rc = launch_ksk_expand(c->mask_seed, kb.get(), c->d_ksk.get(), c->ksk_elem_bytes, N, p.baseKS, p.dKS, p.n, rowlen, (u32)p.qKS, c->stream);
+      if (rc) return cuda_fail((cudaError_t)rc, "ksk_expand");
       BFHE_CUDA(cudaStreamSynchronize(c->stream));
-      cudaFree(d_kb);
       if (dbg_ksk) {
         std::vector<u8> dev(bytes);
-        BFHE_CUDA(cudaMemcpy(dev.data(), c->d_ksk, bytes, cudaMemcpyDeviceToHost));
+        BFHE_CUDA(cudaMemcpy(dev.data(), c->d_ksk.get(), bytes, cudaMemcpyDeviceToHost));
         relayout(dbg_ksk, dev.data(), false);
       }
     } else {
       std::vector<u8> dev(bytes, 0);
       relayout(c->ksk.data(), dev.data(), true);
-      BFHE_CUDA(cudaMemcpy(c->d_ksk, dev.data(), bytes, cudaMemcpyHostToDevice));
+      BFHE_CUDA(upload(c->d_ksk, dev));
     }
   }
   c->dev_keys = true;
@@ -929,15 +911,14 @@ int bfhe::read_ct_blob(const bfhe_ctx *c, const void *blob, size_t len, CtBlob &
   return BFHE_OK;
 }
 
-static int ensure_tmp(bfhe_ctx *c, size_t rows);
 int bfhe::expand_ct_rows(bfhe_ctx *c, const CtBlob &b, u32 *d_rows, std::vector<u32> &wide) {
   if (b.count == 0) return BFHE_OK;
   wide.resize(b.count);
   for (size_t g = 0; g < b.count; g++) wide[g] = ct_body(b.bodies, g);
   // the bodies go through the per-call scratch rows (kept between calls; a stream-ordered allocation would map fresh memory every time)
-  if (int rc = ensure_tmp(c, (b.count + c->p.ct_stride - 1) / c->p.ct_stride)) return rc;
-  BFHE_CUDA(cudaMemcpyAsync(c->d_tmp, wide.data(), b.count * 4, cudaMemcpyHostToDevice, c->stream));
-  int rc = launch_ct_expand(b.seed, c->d_tmp, d_rows, b.count, c->p.n, c->p.ct_stride, c->p.q, c->stream);
+  BFHE_CUDA(c->d_tmp.reserve(b.count, c->stream));
+  BFHE_CUDA(cudaMemcpyAsync(c->d_tmp.get(), wide.data(), b.count * 4, cudaMemcpyHostToDevice, c->stream));
+  int rc = launch_ct_expand(b.seed, c->d_tmp.get(), d_rows, b.count, c->p.n, c->p.ct_stride, c->p.q, c->stream);
   if (rc) return cuda_fail((cudaError_t)rc, "ct_expand");
   return BFHE_OK;
 }
@@ -992,8 +973,8 @@ static void prof_end(bfhe_ctx *c, cudaStream_t st = nullptr) {
 
 int bfhe::run_gate_list(bfhe_ctx *c, const DevGate *list, size_t count, u32 *acc_dbg_host) {
   const u32 N = c->p.N;
-  u32 *d_acc = nullptr;
-  if (acc_dbg_host) BFHE_CUDA(cudaMalloc(&d_acc, std::min(count, c->chunk) * 2 * N * 4));
+  DevBuf<u32> d_acc;
+  if (acc_dbg_host) BFHE_CUDA(d_acc.alloc(std::min(count, c->chunk) * 2 * N));
   // Gates of one list are independent, so with several chunks the (HBM-bound) key switch of chunk k runs on a side
   // stream underneath the (integer-bound) blind rotation of chunk k+1; two sets of descriptor / ext buffers.
   const bool overlap = count > c->chunk && !acc_dbg_host;
@@ -1001,22 +982,21 @@ int bfhe::run_gate_list(bfhe_ctx *c, const DevGate *list, size_t count, u32 *acc
   for (size_t off = 0; off < count; off += c->chunk, k++) {
     const size_t m = std::min(c->chunk, count - off);
     const int b = overlap ? (k & 1) : 0;
-    DevGate *dg = b ? c->d_gates_b : c->d_gates;
-    u32 *de = b ? c->d_ext_b : c->d_ext;
+    DevGate *dg = (b ? c->d_gates_b : c->d_gates).get();
+    u32 *de = (b ? c->d_ext_b : c->d_ext).get();
     if (overlap && k >= 2) BFHE_CUDA(cudaStreamWaitEvent(c->stream, c->ev_ks[b], 0)); // buffers of chunk k-2 are free again
     const int sb = c->stage_next;
     c->stage_next ^= 1;
     BFHE_CUDA(cudaEventSynchronize(c->stage_ev[sb])); // staging buffer free again?
-    std::memcpy(c->h_gates[sb], list + off, m * sizeof(DevGate));
-    BFHE_CUDA(cudaMemcpyAsync(dg, c->h_gates[sb], m * sizeof(DevGate), cudaMemcpyHostToDevice, c->stream));
+    std::memcpy(c->h_gates[sb].get(), list + off, m * sizeof(DevGate));
+    BFHE_CUDA(cudaMemcpyAsync(dg, c->h_gates[sb].get(), m * sizeof(DevGate), cudaMemcpyHostToDevice, c->stream));
     BFHE_CUDA(cudaEventRecord(c->stage_ev[sb], c->stream));
     prof_begin(c, 0);
-    int rc = launch_blind_rotate(c->P, c->p.method == BFHE_AP, dg, (int)m, c->d_bk, c->d_twl, c->d_psiM, de, d_acc, c->force_g,
-                                 c->stream, nullptr, &c->v2);
+    int rc = launch_blind_rotate(c->P, c->p.method == BFHE_AP, dg, (int)m, c->keys(), de, d_acc.get(), (Form)c->force_g, c->stream);
     prof_end(c);
     if (rc) return cuda_fail((cudaError_t)rc, "blind_rotate launch");
     if (acc_dbg_host) {
-      BFHE_CUDA(cudaMemcpyAsync(acc_dbg_host + off * 2 * N, d_acc, m * 2 * N * 4, cudaMemcpyDeviceToHost, c->stream));
+      BFHE_CUDA(cudaMemcpyAsync(acc_dbg_host + off * 2 * N, d_acc.get(), m * 2 * N * 4, cudaMemcpyDeviceToHost, c->stream));
       BFHE_CUDA(cudaStreamSynchronize(c->stream));
     }
     cudaStream_t kst = overlap ? c->ks_stream : c->stream;
@@ -1025,7 +1005,7 @@ int bfhe::run_gate_list(bfhe_ctx *c, const DevGate *list, size_t count, u32 *acc
       BFHE_CUDA(cudaStreamWaitEvent(c->ks_stream, c->ev_br[b], 0));
     }
     prof_begin(c, 1, kst);
-    rc = launch_keyswitch(c->P, de, dg, (int)m, c->d_ksk, c->ksk_elem_bytes, kst);
+    rc = launch_keyswitch(c->P, de, dg, (int)m, c->keys(), kst);
     prof_end(c, kst);
     if (rc) return cuda_fail((cudaError_t)rc, "keyswitch launch");
     if (overlap) BFHE_CUDA(cudaEventRecord(c->ev_ks[b], c->ks_stream));
@@ -1034,41 +1014,20 @@ int bfhe::run_gate_list(bfhe_ctx *c, const DevGate *list, size_t count, u32 *acc
     BFHE_CUDA(cudaStreamWaitEvent(c->stream, c->ev_ks[0], 0));
     if (k >= 2) BFHE_CUDA(cudaStreamWaitEvent(c->stream, c->ev_ks[1], 0));
   }
-  if (d_acc) { cudaStreamSynchronize(c->stream); cudaFree(d_acc); }
-  return BFHE_OK;
-}
-
-static int ensure_tmp(bfhe_ctx *c, size_t rows) {
-  if (rows <= c->tmp_rows) return BFHE_OK;
-  BFHE_CUDA(cudaStreamSynchronize(c->stream));
-  cudaFree(c->d_tmp);
-  c->d_tmp = nullptr;
-  c->tmp_rows = 0;
-  BFHE_CUDA(cudaMalloc(&c->d_tmp, rows * c->p.ct_stride * 4));
-  c->tmp_rows = rows;
-  return BFHE_OK;
-}
-static int ensure_ptrs(bfhe_ctx *c, size_t count) {
-  if (count <= c->ptr_cap) return BFHE_OK;
-  BFHE_CUDA(cudaStreamSynchronize(c->stream));
-  cudaFree(c->d_ptr_in); cudaFree(c->d_ptr_out);
-  c->ptr_cap = 0;
-  BFHE_CUDA(cudaMalloc(&c->d_ptr_in, count * sizeof(void *)));
-  BFHE_CUDA(cudaMalloc(&c->d_ptr_out, count * sizeof(void *)));
-  c->ptr_cap = count;
+  if (acc_dbg_host) cudaStreamSynchronize(c->stream);
   return BFHE_OK;
 }
 
 int bfhe::not_ptr_batch(bfhe_ctx *c, const std::vector<const u32 *> &in, const std::vector<u32 *> &out) {
   if (in.empty()) return BFHE_OK;
-  int rc = ensure_ptrs(c, in.size());
-  if (rc) return rc;
+  BFHE_CUDA(c->d_ptr_in.reserve(in.size(), c->stream));
+  BFHE_CUDA(c->d_ptr_out.reserve(in.size(), c->stream));
   // pointer lists are small; a synchronous copy keeps the host vectors' lifetime trivial
-  BFHE_CUDA(cudaMemcpyAsync(c->d_ptr_in, in.data(), in.size() * sizeof(void *), cudaMemcpyHostToDevice, c->stream));
-  BFHE_CUDA(cudaMemcpyAsync(c->d_ptr_out, out.data(), out.size() * sizeof(void *), cudaMemcpyHostToDevice, c->stream));
+  BFHE_CUDA(cudaMemcpyAsync(c->d_ptr_in.get(), in.data(), in.size() * sizeof(void *), cudaMemcpyHostToDevice, c->stream));
+  BFHE_CUDA(cudaMemcpyAsync(c->d_ptr_out.get(), out.data(), out.size() * sizeof(void *), cudaMemcpyHostToDevice, c->stream));
   BFHE_CUDA(cudaStreamSynchronize(c->stream));
   prof_begin(c, 2);
-  int r2 = launch_eval_not(c->P, c->d_ptr_in, c->d_ptr_out, (int)in.size(), c->stream);
+  int r2 = launch_eval_not(c->P, c->d_ptr_in.get(), c->d_ptr_out.get(), (int)in.size(), c->stream);
   prof_end(c);
   if (r2) return cuda_fail((cudaError_t)r2, "eval_not launch");
   return BFHE_OK;
@@ -1086,11 +1045,8 @@ extern "C" int bfhe_eval_not_batch(bfhe_ctx *c, uint32_t *slab, const uint32_t *
   return not_ptr_batch(c, in, out);
 }
 
-static int eval_batch_locked(bfhe_ctx *c, uint32_t *slab, const bfhe_gate *gates, size_t count, u32 *acc_dbg_host) {
-  int rc = ensure_device_keys(c);
-  if (rc) return rc;
-  const size_t st = c->p.ct_stride;
-  size_t ncomp = 0;
+// every gate's op in range, and no gate reading the very same ciphertext twice
+static int check_gates(const bfhe_gate *gates, size_t count) {
   for (size_t i = 0; i < count; i++) {
     const u32 g = gates[i].op & 0xff;
     if (g > BFHE_BOOTSTRAP) { set_error("unknown gate type"); return BFHE_ERR_ARG; }
@@ -1100,11 +1056,20 @@ static int eval_batch_locked(bfhe_ctx *c, uint32_t *slab, const bfhe_gate *gates
       set_error("EvalBinGate: please only use independent ciphertexts as inputs (gate " + std::to_string(i) + ")");
       return BFHE_ERR_ALIAS;
     }
-    if (g == BFHE_XOR || g == BFHE_XNOR) ncomp++;
   }
-  if (acc_dbg_host && ncomp) { set_error("debug blind rotation does not take composite gates"); return BFHE_ERR_ARG; }
-  rc = ensure_tmp(c, 2 * ncomp);
+  return BFHE_OK;
+}
+
+static int eval_batch_locked(bfhe_ctx *c, uint32_t *slab, const bfhe_gate *gates, size_t count, u32 *acc_dbg_host) {
+  int rc = ensure_device_keys(c);
   if (rc) return rc;
+  if ((rc = check_gates(gates, count))) return rc;
+  const size_t st = c->p.ct_stride;
+  size_t ncomp = 0;
+  for (size_t i = 0; i < count; i++)
+    if ((gates[i].op & 0xff) == BFHE_XOR || (gates[i].op & 0xff) == BFHE_XNOR) ncomp++;
+  if (acc_dbg_host && ncomp) { set_error("debug blind rotation does not take composite gates"); return BFHE_ERR_ARG; }
+  BFHE_CUDA(c->d_tmp.reserve(2 * ncomp * st, c->stream));
   std::vector<DevGate> l1, l2;
   std::vector<const u32 *> not_in;
   std::vector<u32 *> not_out;
@@ -1118,7 +1083,7 @@ static int eval_batch_locked(bfhe_ctx *c, uint32_t *slab, const bfhe_gate *gates
     u32 *o = slab + (size_t)g.out * st;
     if (gate == BFHE_XOR || gate == BFHE_XNOR) { // OR(AND(a, !b), AND(!a, b)), operand order as src/gate.cpp:198-202
       const u32 f0 = g.op & BFHE_NEG0, f1 = g.op & BFHE_NEG1;
-      u32 *t1 = c->d_tmp + (2 * t) * st, *t2 = c->d_tmp + (2 * t + 1) * st;
+      u32 *t1 = c->d_tmp.get() + (2 * t) * st, *t2 = c->d_tmp.get() + (2 * t + 1) * st;
       t++;
       l1.push_back(DevGate{a, b, t1, BFHE_AND | f0 | (f1 ^ BFHE_NEG1), 0});
       l1.push_back(DevGate{a, b, t2, BFHE_AND | (f0 ^ BFHE_NEG0) | f1, 0});
@@ -1166,15 +1131,7 @@ static int check_host_call(const bfhe_gate *gates, size_t count, size_t in_rows,
       set_error("bfhe_eval_bingate_host: gate rows out of range");
       return BFHE_ERR_ARG;
     }
-  for (size_t i = 0; i < count; i++) {
-    const u32 g = gates[i].op & 0xff;
-    if (g > BFHE_BOOTSTRAP) { set_error("unknown gate type"); return BFHE_ERR_ARG; }
-    if (g != BFHE_BOOTSTRAP && gates[i].in0 == gates[i].in1 && (((gates[i].op & BFHE_NEG0) != 0) == ((gates[i].op & BFHE_NEG1) != 0))) {
-      set_error("EvalBinGate: please only use independent ciphertexts as inputs (gate " + std::to_string(i) + ")");
-      return BFHE_ERR_ALIAS;
-    }
-  }
-  return BFHE_OK;
+  return check_gates(gates, count);
 }
 
 // one batch.  Staging slab: every request's input rows, in queue order, then every request's output rows, in the same order (a lone call
@@ -1188,14 +1145,8 @@ static int run_host_batch(bfhe_ctx *c, const std::vector<HostGateReq *> &batch) 
   for (const HostGateReq *r : batch) { in_total += r->in_rows; out_total += r->out_rows; count += r->count; }
   const size_t rows = in_total + out_total;
   if (rows > 0xffffffffu) { set_error("bfhe_eval_bingate_host: combined batch exceeds 2^32 rows"); return BFHE_ERR_ARG; }
-  if (rows > c->e2e_rows) {
-    BFHE_CUDA(cudaStreamSynchronize(c->stream));
-    cudaFree(c->e2e_slab);
-    c->e2e_slab = nullptr;
-    c->e2e_rows = 0;
-    BFHE_CUDA(cudaMalloc(&c->e2e_slab, rows * st * 4));
-    c->e2e_rows = rows;
-  }
+  BFHE_CUDA(c->e2e_slab.reserve(rows * st, c->stream));
+  u32 *slab = c->e2e_slab.get();
   std::vector<bfhe_gate> all;
   const bfhe_gate *list = batch[0]->gates; // a lone call: the translation is the identity
   if (batch.size() > 1) {
@@ -1216,21 +1167,21 @@ static int run_host_batch(bfhe_ctx *c, const std::vector<HostGateReq *> &batch) 
   size_t ib = 0;
   for (const HostGateReq *r : batch) {
     if (r->in_rows) {
-      cudaError_t e = cudaMemcpyAsync(c->e2e_slab + ib * st, r->in_host, r->in_rows * st * 4, cudaMemcpyHostToDevice, c->stream);
+      cudaError_t e = cudaMemcpyAsync(slab + ib * st, r->in_host, r->in_rows * st * 4, cudaMemcpyHostToDevice, c->stream);
       if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMemcpyAsync (bfhe_eval_bingate_host inputs)"); break; }
     }
     ib += r->in_rows;
   }
   if (!rc && out_total) {
-    cudaError_t e = cudaMemsetAsync(c->e2e_slab + in_total * st, 0, out_total * st * 4, c->stream);
+    cudaError_t e = cudaMemsetAsync(slab + in_total * st, 0, out_total * st * 4, c->stream);
     if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemsetAsync (bfhe_eval_bingate_host outputs)");
   }
-  if (!rc) rc = eval_batch_locked(c, c->e2e_slab, list, count, nullptr);
+  if (!rc) rc = eval_batch_locked(c, slab, list, count, nullptr);
   size_t ob = in_total;
   for (const HostGateReq *r : batch) {
     if (rc) break;
     if (r->out_rows) {
-      cudaError_t e = cudaMemcpyAsync(r->out_host, c->e2e_slab + ob * st, r->out_rows * st * 4, cudaMemcpyDeviceToHost, c->stream);
+      cudaError_t e = cudaMemcpyAsync(r->out_host, slab + ob * st, r->out_rows * st * 4, cudaMemcpyDeviceToHost, c->stream);
       if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync (bfhe_eval_bingate_host outputs)");
     }
     ob += r->out_rows;
@@ -1335,25 +1286,22 @@ extern "C" int bfhe_profile_read(bfhe_ctx *c, int kernel, double *ms, uint64_t *
 extern "C" int bfhe_microbench_int(bfhe_ctx *c, int which, double *ginstr_per_s) {
   int rc = need_device(c);
   if (rc) return rc;
-  u32 *sink = nullptr;
-  BFHE_CUDA(cudaMalloc(&sink, 64));
-  BFHE_CUDA(cudaMemset(sink, 0x5a, 64));
-  cudaEvent_t a, b;
-  cudaEventCreate(&a);
-  cudaEventCreate(&b);
+  DevBuf<u32> sink;
+  BFHE_CUDA(sink.alloc(16));
+  BFHE_CUDA(cudaMemset(sink.get(), 0x5a, 64));
+  DevEvent a, b;
+  a.create();
+  b.create();
   int threads = 0, ops = 0;
   const int iters = 4096;
-  launch_microbench(which, sink, 64, &threads, &ops, c->stream); // warm-up
-  cudaEventRecord(a, c->stream);
-  int r2 = launch_microbench(which, sink, iters, &threads, &ops, c->stream);
-  cudaEventRecord(b, c->stream);
+  launch_microbench(which, sink.get(), 64, &threads, &ops, c->stream); // warm-up
+  cudaEventRecord(a.e, c->stream);
+  int r2 = launch_microbench(which, sink.get(), iters, &threads, &ops, c->stream);
+  cudaEventRecord(b.e, c->stream);
   if (r2) return cuda_fail((cudaError_t)r2, "microbench");
-  BFHE_CUDA(cudaEventSynchronize(b));
+  BFHE_CUDA(cudaEventSynchronize(b.e));
   float ms = 0;
-  cudaEventElapsedTime(&ms, a, b);
-  cudaEventDestroy(a);
-  cudaEventDestroy(b);
-  cudaFree(sink);
+  cudaEventElapsedTime(&ms, a.e, b.e);
   double per_iter = which == 4 ? 3.0 : 1.0; // the Shoup half-butterfly issues 3 multiply-class instructions
   if (ginstr_per_s) *ginstr_per_s = (double)threads * ops * iters * per_iter / (ms * 1e-3) / 1e9;
   return BFHE_OK;
@@ -1362,22 +1310,21 @@ extern "C" int bfhe_microbench_int(bfhe_ctx *c, int which, double *ginstr_per_s)
 extern "C" int bfhe_dbg_ntt_roundtrip(bfhe_ctx *c, const uint32_t *a, size_t npoly, uint32_t *rt, uint32_t *prod, const uint32_t *b) {
   int rc = need_device(c);
   if (rc) return rc;
-  const size_t bytes = npoly * c->p.N * 4;
-  u32 *da = nullptr, *db = nullptr, *drt = nullptr, *dpr = nullptr;
-  BFHE_CUDA(cudaMalloc(&da, bytes));
-  BFHE_CUDA(cudaMalloc(&drt, bytes));
-  BFHE_CUDA(cudaMemcpy(da, a, bytes, cudaMemcpyHostToDevice));
+  const size_t words = npoly * c->p.N, bytes = words * 4;
+  DevBuf<u32> da, db, drt, dpr;
+  BFHE_CUDA(da.alloc(words));
+  BFHE_CUDA(drt.alloc(words));
+  BFHE_CUDA(cudaMemcpy(da.get(), a, bytes, cudaMemcpyHostToDevice));
   if (b) {
-    BFHE_CUDA(cudaMalloc(&db, bytes));
-    BFHE_CUDA(cudaMalloc(&dpr, bytes));
-    BFHE_CUDA(cudaMemcpy(db, b, bytes, cudaMemcpyHostToDevice));
+    BFHE_CUDA(db.alloc(words));
+    BFHE_CUDA(dpr.alloc(words));
+    BFHE_CUDA(cudaMemcpy(db.get(), b, bytes, cudaMemcpyHostToDevice));
   }
-  int r2 = launch_dbg_ntt(c->P, da, db, drt, dpr, (int)npoly, c->d_twl, c->stream);
+  int r2 = launch_dbg_ntt(c->P, da.get(), db.get(), drt.get(), dpr.get(), (int)npoly, c->d_twl.get(), c->stream);
   if (r2) return cuda_fail((cudaError_t)r2, "dbg_ntt");
   BFHE_CUDA(cudaStreamSynchronize(c->stream));
-  BFHE_CUDA(cudaMemcpy(rt, drt, bytes, cudaMemcpyDeviceToHost));
-  if (b) BFHE_CUDA(cudaMemcpy(prod, dpr, bytes, cudaMemcpyDeviceToHost));
-  cudaFree(da); cudaFree(db); cudaFree(drt); cudaFree(dpr);
+  BFHE_CUDA(cudaMemcpy(rt, drt.get(), bytes, cudaMemcpyDeviceToHost));
+  if (b) BFHE_CUDA(cudaMemcpy(prod, dpr.get(), bytes, cudaMemcpyDeviceToHost));
   return BFHE_OK;
 }
 

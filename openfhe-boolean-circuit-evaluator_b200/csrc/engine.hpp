@@ -3,6 +3,7 @@
 #include "../../include/bfhe.h"
 #include "common.hpp"
 #include "hostmath.hpp"
+#include <algorithm>
 #include <condition_variable>
 #include <cuda_runtime.h>
 #include <deque>
@@ -19,6 +20,70 @@ int cuda_fail(cudaError_t e, const char *what);
     cudaError_t _e = (call);                                                                                           \
     if (_e != cudaSuccess) return ::bfhe::cuda_fail(_e, #call);                                                        \
   } while (0)
+
+// Owner of one device allocation (Pinned: page-locked host memory), released on destruction.  Allocate, reserve and release with the
+// owning context's device current.
+template <typename T, bool Pinned = false> class DevBuf {
+public:
+  DevBuf() = default;
+  DevBuf(const DevBuf &) = delete;
+  DevBuf &operator=(const DevBuf &) = delete;
+  DevBuf(DevBuf &&o) noexcept : p_(o.p_), n_(o.n_) { o.p_ = nullptr; o.n_ = 0; }
+  DevBuf &operator=(DevBuf &&o) noexcept {
+    if (this != &o) { reset(); p_ = o.p_; n_ = o.n_; o.p_ = nullptr; o.n_ = 0; }
+    return *this;
+  }
+  ~DevBuf() { reset(); }
+  // a fresh buffer of `count` elements; the old one is released first
+  cudaError_t alloc(size_t count) {
+    reset();
+    void *p = nullptr;
+    cudaError_t e = Pinned ? cudaMallocHost(&p, count * sizeof(T)) : cudaMalloc(&p, count * sizeof(T));
+    if (e != cudaSuccess) return e;
+    p_ = static_cast<T *>(p);
+    n_ = count;
+    return cudaSuccess;
+  }
+  // grow-only: a larger buffer once `stream` is done with the old one (work queued on it may still read or write it)
+  cudaError_t reserve(size_t count, cudaStream_t stream) {
+    if (count <= n_) return cudaSuccess;
+    cudaError_t e = cudaStreamSynchronize(stream);
+    return e != cudaSuccess ? e : alloc(count);
+  }
+  void reset() {
+    if (p_) Pinned ? cudaFreeHost(p_) : cudaFree(p_);
+    p_ = nullptr;
+    n_ = 0;
+  }
+  T *get() const { return p_; }
+  size_t size() const { return n_; }
+
+private:
+  T *p_ = nullptr;
+  size_t n_ = 0;
+};
+
+// dst := a device copy of src (at least one element, so that an empty list still has a valid address)
+template <typename T> cudaError_t upload(DevBuf<T> &dst, const std::vector<T> &src) {
+  cudaError_t e = dst.alloc(std::max<size_t>(src.size(), 1));
+  return e != cudaSuccess ? e : cudaMemcpy(dst.get(), src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice);
+}
+
+// owner of a local cudaEvent_t (timing enabled)
+struct DevEvent {
+  cudaEvent_t e = nullptr;
+  DevEvent() = default;
+  DevEvent(const DevEvent &) = delete;
+  DevEvent &operator=(const DevEvent &) = delete;
+  ~DevEvent() { if (e) cudaEventDestroy(e); }
+  cudaError_t create() { return cudaEventCreate(&e); }
+};
+
+// cost (ms) of one wave (blind rotation + key switch) in the kernel forms the circuit planner weighs: these B200 defaults, or measured once
+// per context on its device with its key set (host/circuit.cpp probe_costs)
+struct WaveCosts {
+  double cl4 = 1.05, cl2 = 1.55, lat = 2.36, thr = 5.85;
+};
 
 struct ProfSpan {
   cudaEvent_t a, b;
@@ -65,38 +130,33 @@ struct bfhe_ctx {
   bfhe::u32 ksk_elem_bytes = 4;
   bfhe::u64 bk_words = 0, ksk_elems = 0;
 
-  // device key material
-  bfhe::u32 *d_bk = nullptr, *d_twl = nullptr, *d_psiM = nullptr;
-  void *d_ksk = nullptr;
-  bfhe::u32 *d_bk4 = nullptr, *d_tw2 = nullptr, *d_F = nullptr; // 2-CTA cluster kernel (kernels_v2.cu)
-  bfhe::u32 *d_bkx = nullptr, *d_twx = nullptr; // slot-sliced cluster kernel (kernels_cl.cu)
-  bfhe::u32 *d_bkf = nullptr; // GINX throughput kernel at the STD128_OPT shape: top digit folded into the key (kernels.cu bk_fold_kernel)
-  bfhe::V2Bufs v2{};
+  // device key material: tables made by bfhe_create, key copies by upload_keys; handed to the kernels as keys()
+  bfhe::DevBuf<bfhe::u32> d_twl, d_psiM, d_tw2, d_F, d_twx;
+  bfhe::DevBuf<bfhe::u32> d_bk, d_bkf, d_bk4, d_bkx;
+  bfhe::DevBuf<bfhe::u8> d_ksk;
   bool dev_keys = false;
+  bfhe::DevKeys keys() const {
+    return {d_bk.get(), d_bkf.get(), d_bk4.get(), d_bkx.get(), d_twl.get(), d_psiM.get(), d_tw2.get(), d_F.get(), d_twx.get(), d_ksk.get(),
+            (int)ksk_elem_bytes};
+  }
 
   // per-call scratch
   static constexpr size_t CHUNK = 32768; // upper bound of gates per blind-rotation launch (buffer sizes)
   size_t chunk = CHUNK;                  // actual launch size: largest multiple of one full wave (4 gates x SM count) <= CHUNK
-  bfhe::DevGate *d_gates = nullptr;      // CHUNK entries (buffer 0)
-  bfhe::DevGate *d_gates_b = nullptr;    // buffer 1: key switch of chunk k overlaps blind rotation of chunk k+1
-  bfhe::u32 *d_ext_b = nullptr;
+  bfhe::DevBuf<bfhe::DevGate> d_gates;   // CHUNK entries (buffer 0)
+  bfhe::DevBuf<bfhe::DevGate> d_gates_b; // buffer 1: key switch of chunk k overlaps blind rotation of chunk k+1
+  bfhe::DevBuf<bfhe::u32> d_ext, d_ext_b; // CHUNK * (N+4) each
   cudaStream_t ks_stream = nullptr;
   cudaEvent_t ev_br[2] = {nullptr, nullptr}, ev_ks[2] = {nullptr, nullptr};
-  bfhe::DevGate *h_gates[2] = {nullptr, nullptr}; // pinned staging
+  bfhe::DevBuf<bfhe::DevGate, true> h_gates[2]; // pinned staging
   cudaEvent_t stage_ev[2] = {nullptr, nullptr};
   int stage_next = 0;
-  bfhe::u32 *d_ext = nullptr;            // CHUNK * (N+4)
-  bfhe::u32 *d_tmp = nullptr;            // composite-gate temporaries; the bodies of a compact ciphertext blob (expand_ct_rows)
-  size_t tmp_rows = 0;
-  const bfhe::u32 **d_ptr_in = nullptr;  // EvalNOT pointer lists
-  bfhe::u32 **d_ptr_out = nullptr;
-  size_t ptr_cap = 0;
-  bfhe::u32 *e2e_slab = nullptr;
-  size_t e2e_rows = 0;
-  int force_g = 0; // test hook: gates per CTA
-  // measured cost (ms) of one wave (blind rotation + key switch) in the 4-CTA / 2-CTA cluster, one-gate-per-SM and four-gates-per-SM
-  // forms on this device with this key set (host/circuit.cpp probe_costs)
-  double form_cost_ms[4] = {0, 0, 0, 0};
+  bfhe::DevBuf<bfhe::u32> d_tmp;         // composite-gate temporaries; the bodies of a compact ciphertext blob (expand_ct_rows)
+  bfhe::DevBuf<const bfhe::u32 *> d_ptr_in; // EvalNOT pointer lists
+  bfhe::DevBuf<bfhe::u32 *> d_ptr_out;
+  bfhe::DevBuf<bfhe::u32> e2e_slab;      // bfhe_eval_bingate_host staging
+  int force_g = 0; // test hook: the bfhe::Form every launch uses (AUTO: the launch's own choice)
+  bfhe::WaveCosts form_costs;
   bool form_cost_measured = false;
 
   bool profiling = false;

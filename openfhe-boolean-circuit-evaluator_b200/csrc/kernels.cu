@@ -952,21 +952,20 @@ blind_rotate_lat_kernel(const __grid_constant__ DevConst P, const DevGate *__res
 
 template <int LOGN, int DG, int LOGBG, bool AP>
 static int launch_lat_inst(const DevConst &P, const DevGate *d_gates, int count, const u32 *d_bk, const u32 *d_twl,
-                           const u32 *d_psiM, u32 *d_ext, u32 *d_acc, cudaStream_t st, LaunchInfo *info) {
+                           const u32 *d_psiM, u32 *d_ext, u32 *d_acc, cudaStream_t st) {
   using Cfg = LatCfg<LOGN, DG, LOGBG, AP>;
   auto kern = blind_rotate_lat_kernel<LOGN, DG, LOGBG, AP>;
   static bool attr_done[64];
   if (int rc = once_per_device(attr_done, [&] { return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::smem_bytes); }))
     return rc;
   if (count <= 0) return 0; // attribute warm-up only
-  if (info) { info->gates_per_cta = 1; info->ctas = count; info->smem_bytes = Cfg::smem_bytes; }
   kern<<<count, Cfg::THREADS, Cfg::smem_bytes, st>>>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc);
   return (int)cudaGetLastError();
 }
 
 template <int LOGN, int DG, int LOGBG, int G, bool AP>
 static int launch_br_inst(const DevConst &P, const DevGate *d_gates, int count, const u32 *d_bk, const u32 *d_twl,
-                          const u32 *d_psiM, u32 *d_ext, u32 *d_acc, cudaStream_t st, LaunchInfo *info) {
+                          const u32 *d_psiM, u32 *d_ext, u32 *d_acc, cudaStream_t st) {
   using Cfg = BrCfg<LOGN, DG, LOGBG, G, AP>;
   auto kern = blind_rotate_kernel<LOGN, DG, LOGBG, G, AP>;
   static bool attr_done[64];
@@ -974,19 +973,18 @@ static int launch_br_inst(const DevConst &P, const DevGate *d_gates, int count, 
     return rc;
   if (count <= 0) return 0; // attribute warm-up only
   const int ctas = (count + G - 1) / G;
-  if (info) { info->gates_per_cta = G; info->ctas = ctas; info->smem_bytes = Cfg::smem_bytes; }
   kern<<<ctas, Cfg::THREADS, Cfg::smem_bytes, st>>>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc);
   return (int)cudaGetLastError();
 }
 
 template <int LOGN, int DG, int LOGBG, bool AP>
 static int launch_br_g(int G, const DevConst &P, const DevGate *d_gates, int count, const u32 *d_bk, const u32 *d_twl,
-                       const u32 *d_psiM, u32 *d_ext, u32 *d_acc, cudaStream_t st, LaunchInfo *info) {
+                       const u32 *d_psiM, u32 *d_ext, u32 *d_acc, cudaStream_t st) {
   switch (G) {
-  case 1: return launch_br_inst<LOGN, DG, LOGBG, 1, AP>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc, st, info);
-  case 2: return launch_br_inst<LOGN, DG, LOGBG, 2, AP>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc, st, info);
+  case 1: return launch_br_inst<LOGN, DG, LOGBG, 1, AP>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc, st);
+  case 2: return launch_br_inst<LOGN, DG, LOGBG, 2, AP>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc, st);
   // (6 gates per CTA, 3 warps per scheduler with a register-lean product, measured 7 % slower than 4: DESIGN.md 5.4)
-  default: return launch_br_inst<LOGN, DG, LOGBG, 4, AP>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc, st, info);
+  default: return launch_br_inst<LOGN, DG, LOGBG, 4, AP>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc, st);
   }
 }
 
@@ -994,11 +992,11 @@ template <int LOGN, int DG, int LOGBG> static int br_attrs() {
   DevConst P{};
   int rc = 0;
   for (int G : {1, 2, 4}) {
-    rc |= launch_br_g<LOGN, DG, LOGBG, false>(G, P, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
-    rc |= launch_br_g<LOGN, DG, LOGBG, true>(G, P, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
+    rc |= launch_br_g<LOGN, DG, LOGBG, false>(G, P, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0);
+    rc |= launch_br_g<LOGN, DG, LOGBG, true>(G, P, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0);
   }
-  rc |= launch_lat_inst<LOGN, DG, LOGBG, false>(P, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
-  rc |= launch_lat_inst<LOGN, DG, LOGBG, true>(P, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr);
+  rc |= launch_lat_inst<LOGN, DG, LOGBG, false>(P, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0);
+  rc |= launch_lat_inst<LOGN, DG, LOGBG, true>(P, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0);
   return rc;
 }
 int blind_rotate_set_attrs() {
@@ -1009,47 +1007,56 @@ int blind_rotate_set_attrs() {
   return rc;
 }
 
-int launch_blind_rotate(const DevConst &P, int method_ap, const DevGate *d_gates, int count, const u32 *d_bk, const u32 *d_twl,
-                        const u32 *d_psiM, u32 *d_ext, u32 *d_acc_dbg, int force_g, void *stream, LaunchInfo *info, const V2Bufs *v2) {
+bool form_supported(const DevConst &P, int method_ap, Form f) {
+  const bool std_shape = P.N == 1024 && P.dG == 4 && P.logBG == 7, toy_shape = P.N == 512 && P.dG == 3 && P.logBG == 9;
+  switch (f) {
+  case Form::AUTO:
+  case Form::LAT: return std_shape || toy_shape;
+  case Form::THR1:
+  case Form::THR2:
+  case Form::THR4: return toy_shape || (std_shape && (method_ap || bk_fold_supported(P, method_ap))); // GINX at this shape reads bkf
+  case Form::CL2: return cl2_supported(P, method_ap);
+  case Form::CL4: return clx_supported(P, method_ap) && (method_ap || cl2_supported(P, method_ap)); // GINX reads the 2-CTA form's F table
+  }
+  return false;
+}
+
+int launch_blind_rotate(const DevConst &P, int method_ap, const DevGate *d_gates, int count, const DevKeys &k, u32 *d_ext, u32 *d_acc_dbg,
+                        Form form, void *stream) {
   if (count <= 0) return 0;
+  if (!form_supported(P, method_ap, form)) return (int)cudaErrorInvalidValue;
   cudaStream_t st = (cudaStream_t)stream;
-  const bool have_cl2 = v2 && v2->d_bk4 && v2->d_tw2 && v2->d_F && v2_supported(P, method_ap);
-  const bool have_clx = v2 && v2->d_bkx && v2->d_twx && (method_ap || v2->d_F) && clx_supported(P, method_ap);
-  if (force_g == 128) return have_clx ? launch_blind_rotate_clx(P, method_ap, d_gates, count, *v2, d_ext, d_acc_dbg, stream, info) : (int)cudaErrorInvalidValue;
-  if (force_g == 32) return have_cl2 ? launch_blind_rotate_cl2(P, d_gates, count, *v2, d_ext, d_acc_dbg, stream, info) : (int)cudaErrorInvalidValue;
-  if (force_g != 0 && force_g != 1 && force_g != 2 && force_g != 4 && force_g != 8) return (int)cudaErrorInvalidValue;
+  if (form == Form::CL4) return launch_blind_rotate_clx(P, method_ap, d_gates, count, k, d_ext, d_acc_dbg, stream);
+  if (form == Form::CL2) return launch_blind_rotate_cl2(P, d_gates, count, k, d_ext, d_acc_dbg, stream);
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   // Which variant?  Measured on B200, STD128_OPT GINX (profiles/): one gate on four SMs 0.98 ms per wave of up to 33 gates; one gate on two
   // SMs 1.48 ms up to 74; latency form (one gate per CTA) 2.22 ms per wave of `sms` gates; throughput form (4 gates per CTA share every
   // key word) 5.68 ms per wave of 4 * sms gates.  Narrow circuit levels go to the cluster forms, wide batches to the throughput form.
-  if (force_g == 0 && have_clx && count <= clx_fast_gates()) return launch_blind_rotate_clx(P, method_ap, d_gates, count, *v2, d_ext, d_acc_dbg, stream, info);
-  if (force_g == 0 && have_cl2 && count <= cl2_max_gates()) return launch_blind_rotate_cl2(P, d_gates, count, *v2, d_ext, d_acc_dbg, stream, info);
+  if (form == Form::AUTO && form_supported(P, method_ap, Form::CL4) && count <= clx_fast_gates())
+    return launch_blind_rotate_clx(P, method_ap, d_gates, count, k, d_ext, d_acc_dbg, stream);
+  if (form == Form::AUTO && form_supported(P, method_ap, Form::CL2) && count <= cl2_max_gates())
+    return launch_blind_rotate_cl2(P, d_gates, count, k, d_ext, d_acc_dbg, stream);
   const long lat_cost = (long)((count + sms - 1) / sms) * 222;           // 2.22 ms per wave of `sms` gates
   const long thr_cost = (long)((count + 4 * sms - 1) / (4 * sms)) * 568; // 5.68 ms per wave of 4 * sms gates
-  const bool lat = force_g == 8 || (force_g == 0 && lat_cost <= thr_cost);
+  const bool lat = form == Form::LAT || (form == Form::AUTO && lat_cost <= thr_cost);
+  const bool std_shape = P.N == 1024; // form_supported admits two shapes: (N 1024, dG 4, base 2^7) and (N 512, dG 3, base 2^9)
   if (lat) {
-    if (P.N == 1024 && P.dG == 4 && P.logBG == 7)
-      return method_ap ? launch_lat_inst<10, 4, 7, true>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info)
-                       : launch_lat_inst<10, 4, 7, false>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info);
-    if (P.N == 512 && P.dG == 3 && P.logBG == 9)
-      return method_ap ? launch_lat_inst<9, 3, 9, true>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info)
-                       : launch_lat_inst<9, 3, 9, false>(P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info);
-    return (int)cudaErrorInvalidValue;
+    if (std_shape)
+      return method_ap ? launch_lat_inst<10, 4, 7, true>(P, d_gates, count, k.bk, k.twl, k.psiM, d_ext, d_acc_dbg, st)
+                       : launch_lat_inst<10, 4, 7, false>(P, d_gates, count, k.bk, k.twl, k.psiM, d_ext, d_acc_dbg, st);
+    return method_ap ? launch_lat_inst<9, 3, 9, true>(P, d_gates, count, k.bk, k.twl, k.psiM, d_ext, d_acc_dbg, st)
+                     : launch_lat_inst<9, 3, 9, false>(P, d_gates, count, k.bk, k.twl, k.psiM, d_ext, d_acc_dbg, st);
   }
-  int G = force_g > 0 ? force_g : 4;
-  if (P.N == 1024 && P.dG == 4 && P.logBG == 7) {
-    if (method_ap) return launch_br_g<10, 4, 7, true>(G, P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info);
+  const int G = form == Form::AUTO ? 4 : (int)form;
+  if (std_shape) {
+    if (method_ap) return launch_br_g<10, 4, 7, true>(G, P, d_gates, count, k.bk, k.twl, k.psiM, d_ext, d_acc_dbg, st);
     static_assert(BrCfg<10, 4, 7, 4, false>::FOLD, "the GINX throughput kernel of this shape reads the folded key");
-    if (!v2 || !v2->d_bkf) return (int)cudaErrorInvalidValue;
-    return launch_br_g<10, 4, 7, false>(G, P, d_gates, count, v2->d_bkf, d_twl, d_psiM, d_ext, d_acc_dbg, st, info);
+    return launch_br_g<10, 4, 7, false>(G, P, d_gates, count, k.bkf, k.twl, k.psiM, d_ext, d_acc_dbg, st);
   }
-  if (P.N == 512 && P.dG == 3 && P.logBG == 9) {
-    return method_ap ? launch_br_g<9, 3, 9, true>(G, P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info)
-                     : launch_br_g<9, 3, 9, false>(G, P, d_gates, count, d_bk, d_twl, d_psiM, d_ext, d_acc_dbg, st, info);
-  }
-  return (int)cudaErrorInvalidValue;
+  return method_ap ? launch_br_g<9, 3, 9, true>(G, P, d_gates, count, k.bk, k.twl, k.psiM, d_ext, d_acc_dbg, st)
+                   : launch_br_g<9, 3, 9, false>(G, P, d_gates, count, k.bk, k.twl, k.psiM, d_ext, d_acc_dbg, st);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1255,13 +1262,14 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(COLS *RG) keyswitch_
   cluster_sync_all(); // peers stay until rank 0 has read
 }
 
-int launch_keyswitch(const DevConst &P, const u32 *d_ext, const DevGate *d_gates, int count, const void *d_ksk, int elem_bytes,
-                     void *stream, const PeerX *pxp) {
+int launch_keyswitch(const DevConst &P, const u32 *d_ext, const DevGate *d_gates, int count, const DevKeys &keys, void *stream,
+                     const PeerX *pxp) {
   if (count <= 0) return 0;
+  const void *d_ksk = keys.ksk;
   const PeerX px = pxp ? *pxp : PeerX();
   cudaStream_t st = (cudaStream_t)stream;
   const int nrows = P.N * P.dKS;
-  if (elem_bytes == 2) {
+  if (keys.ksk_elem_bytes == 2) {
     constexpr int COLS = 256, RG = 4;
     const int rowlen_words = 256; // 512 uint16 per row
     size_t smem = (size_t)((nrows + 1) & ~1) * 4 + (size_t)RG * COLS * 2 * 8; // STD128_OPT: 24 KB, within the default 48 KB limit

@@ -525,17 +525,16 @@ int launch_bk_slice_clx(const u32 *d_src, u32 *d_dst, size_t npoly, int method_a
   else clx::bk_slice_clx_kernel<<<148 * 8, 256, 0, (cudaStream_t)stream>>>(d_src, d_dst, npoly / clx::KEYPOLYS);
   return (int)cudaGetLastError();
 }
-int launch_blind_rotate_clx(const DevConst &P, int method_ap, const DevGate *d_gates, int count, const V2Bufs &vb, u32 *d_ext, u32 *d_acc_dbg,
-                            void *stream, LaunchInfo *info) {
+int launch_blind_rotate_clx(const DevConst &P, int method_ap, const DevGate *d_gates, int count, const DevKeys &k, u32 *d_ext, u32 *d_acc_dbg,
+                            void *stream) {
   if (count <= 0) return 0;
   if (int rc = clx_attrs_once()) return rc;
-  if (info) { info->gates_per_cta = 1; info->ctas = clx::R * count; info->smem_bytes = clx::Smem::bytes; }
   if (method_ap)
-    clx::blind_rotate_clx_kernel<true><<<clx::R * count, clx::THREADS, clx::Smem::bytes, (cudaStream_t)stream>>>(P, d_gates, count, vb.d_bkx, vb.d_twx,
-                                                                                                           vb.d_F, d_ext, d_acc_dbg);
+    clx::blind_rotate_clx_kernel<true><<<clx::R * count, clx::THREADS, clx::Smem::bytes, (cudaStream_t)stream>>>(P, d_gates, count, k.bkx, k.twx, k.F,
+                                                                                                           d_ext, d_acc_dbg);
   else
-    clx::blind_rotate_clx_kernel<false><<<clx::R * count, clx::THREADS, clx::Smem::bytes, (cudaStream_t)stream>>>(P, d_gates, count, vb.d_bkx, vb.d_twx,
-                                                                                                            vb.d_F, d_ext, d_acc_dbg);
+    clx::blind_rotate_clx_kernel<false><<<clx::R * count, clx::THREADS, clx::Smem::bytes, (cudaStream_t)stream>>>(P, d_gates, count, k.bkx, k.twx, k.F,
+                                                                                                            d_ext, d_acc_dbg);
   return (int)cudaGetLastError();
 }
 

@@ -575,7 +575,7 @@ __global__ void bk_permute_v2_kernel(const u32 *__restrict__ src, u32 *__restric
 
 } // namespace v2
 
-bool v2_supported(const DevConst &P, int method_ap) {
+bool cl2_supported(const DevConst &P, int method_ap) {
   return !method_ap && P.N == 1024 && P.dG == 4 && P.logBG == 7 && P.Q == SOLINAS_Q && P.n <= (u32)v2::NPAD;
 }
 int v2_set_attrs() {
@@ -602,13 +602,11 @@ int cl2_max_gates() {
   });
   return gates[d];
 }
-int launch_blind_rotate_cl2(const DevConst &P, const DevGate *d_gates, int count, const V2Bufs &vb, u32 *d_ext, u32 *d_acc_dbg, void *stream,
-                            LaunchInfo *info) {
+int launch_blind_rotate_cl2(const DevConst &P, const DevGate *d_gates, int count, const DevKeys &k, u32 *d_ext, u32 *d_acc_dbg, void *stream) {
   if (count <= 0) return 0;
   if (int rc = v2_attrs_once()) return rc;
-  if (info) { info->gates_per_cta = 1; info->ctas = 2 * count; info->smem_bytes = v2::Cl2Cfg::smem_bytes; }
-  v2::blind_rotate_cl2_kernel<<<2 * count, v2::Cl2Cfg::THREADS, v2::Cl2Cfg::smem_bytes, (cudaStream_t)stream>>>(P, d_gates, count, vb.d_bk4, vb.d_tw2,
-                                                                                                         vb.d_F, d_ext, d_acc_dbg);
+  v2::blind_rotate_cl2_kernel<<<2 * count, v2::Cl2Cfg::THREADS, v2::Cl2Cfg::smem_bytes, (cudaStream_t)stream>>>(P, d_gates, count, k.bk4, k.tw2, k.F,
+                                                                                                         d_ext, d_acc_dbg);
   return (int)cudaGetLastError();
 }
 int launch_bk_permute_v2(const u32 *d_src, u32 *d_dst, size_t npoly, void *stream) {

@@ -70,8 +70,8 @@ struct Level {
 // exchange: what a sharded level pays on top of its kernels -- the key switch's peer stores, one flag round trip over NVLink and one
 // tiny wait launch (~0.015 ms), or one ncclAllGather (~0.05 ms, BFHE_EXCHANGE=nccl).  The plan is made before the slabs exist, so the
 // peer-store figure is assumed unless NCCL was asked for; should the mapping fail later, the plan is merely a little optimistic.
-struct FormCosts {
-  double cl4 = 1.05, cl2 = 1.55, lat = 2.36, thr = 5.85, exchange = exchange_default();
+struct FormCosts : WaveCosts {
+  double exchange = exchange_default();
   bool measured = false;
   static double exchange_default() { const char *m = std::getenv("BFHE_EXCHANGE"); return m && std::strcmp(m, "nccl") == 0 ? 0.05 : 0.015; }
 };
@@ -127,15 +127,14 @@ struct bfhe_circuit {
   uint64_t clocks = 0;
 
   // device state
-  uint32_t *slab = nullptr;
-  DevGate *d_desc = nullptr;             // my slice of every level, concatenated
+  DevBuf<u32> slab;
+  DevBuf<DevGate> d_desc;                // my slice of every level, concatenated
   std::vector<size_t> desc_off;          // per level
   std::vector<uint32_t> my_count;        // per level
-  const u32 **d_not_in = nullptr;    // low bit of an input pointer set: plain copy instead of EvalNOT
-  u32 **d_not_out = nullptr;
+  DevBuf<const u32 *> d_not_in;      // low bit of an input pointer set: plain copy instead of EvalNOT
+  DevBuf<u32 *> d_not_out;
   std::vector<size_t> not_off;       // per level; the last two entries delimit the DFF update batches
-  u32 *d_ext = nullptr;
-  size_t ext_cap = 0;
+  DevBuf<u32> d_ext;                 // widest level * (N+4)
   bool dev_ready = false;
   cudaGraphExec_t graph = nullptr;
   bool use_graph = true;
@@ -143,8 +142,9 @@ struct bfhe_circuit {
   // cannot be mapped (no peer access) or BFHE_EXCHANGE=nccl
   bool peer_ok = false;
   std::vector<void *> peer_slab_map, peer_flag_map; // cudaIpcOpenMemHandle results (null for the own rank)
-  u32 **d_peer_slabs = nullptr, **d_peer_flags = nullptr;
-  u32 *x_flags = nullptr, *x_counter = nullptr, *x_epoch = nullptr, *x_err = nullptr; // one allocation: flags[32] | counter | epoch | err
+  DevBuf<u32 *> d_peer_slabs, d_peer_flags;
+  DevBuf<u32> x_buf; // flags[32] | counter | epoch | err
+  u32 *x_flags = nullptr, *x_counter = nullptr, *x_epoch = nullptr, *x_err = nullptr; // into x_buf
   uint32_t x_per_epoch = 1;
   std::vector<int> shard_index; // level -> index among the sharded levels (-1: not exchanged)
 
@@ -152,7 +152,7 @@ struct bfhe_circuit {
   std::vector<uint8_t> in_bits_set, plain_wire;
   bool has_input = false, done = false;
   bool ct_input = false;          // the input came as ciphertexts (bfhe_circuit_set_input_ct): there are no input bits
-  u32 *d_egress = nullptr;        // clock_ct into host memory: the output rows are staged here
+  DevBuf<u32> d_egress;           // clock_ct into host memory: the output rows are staged here
   double device_ms = 0, host_ms = 0;
   uint64_t verify_mismatches = 0, verify_checked = 0;
 };
@@ -164,15 +164,14 @@ static void free_device(bfhe_circuit *c) {
     if (c->graph) cudaGraphExecDestroy(c->graph);
     for (void *m : c->peer_slab_map) if (m) cudaIpcCloseMemHandle(m);
     for (void *m : c->peer_flag_map) if (m) cudaIpcCloseMemHandle(m);
-    cudaFree(c->d_peer_slabs); cudaFree(c->d_peer_flags); cudaFree(c->x_flags);
-    cudaFree(c->slab); cudaFree(c->d_desc); cudaFree(c->d_not_in); cudaFree(c->d_not_out); cudaFree(c->d_ext);
-    cudaFree(c->d_egress);
+    c->d_peer_slabs.reset(); c->d_peer_flags.reset(); c->x_buf.reset();
+    c->slab.reset(); c->d_desc.reset(); c->d_not_in.reset(); c->d_not_out.reset(); c->d_ext.reset();
+    c->d_egress.reset();
   }
   c->peer_slab_map.clear(); c->peer_flag_map.clear();
-  c->d_peer_slabs = nullptr; c->d_peer_flags = nullptr; c->x_flags = c->x_counter = c->x_epoch = c->x_err = nullptr;
+  c->x_flags = c->x_counter = c->x_epoch = c->x_err = nullptr;
   c->peer_ok = false;
-  c->graph = nullptr; c->slab = nullptr; c->d_desc = nullptr; c->d_not_in = nullptr; c->d_not_out = nullptr; c->d_ext = nullptr;
-  c->d_egress = nullptr;
+  c->graph = nullptr;
   c->dev_ready = false;
 }
 
@@ -180,8 +179,7 @@ static void free_device(bfhe_circuit *c) {
 // planning
 // ---------------------------------------------------------------------------------------------
 static int build_plan_cap(bfhe_circuit *c, uint32_t cap);
-static bool cluster_forms_available(const bfhe_ctx *x) { return x && x->v2.d_tw2 && x->p.method == BFHE_GINX; } // 2-CTA form (GINX)
-static bool clx_form_available(const bfhe_ctx *x) { return x && x->v2.d_twx; }                                   // 4-CTA form (GINX and AP)
+static bool has_form(const bfhe_ctx *x, Form f) { return form_supported(x->P, x->p.method == BFHE_AP, f); }
 
 struct FormCaps { int sms = 0, cl2 = 0, cl4 = 0; };
 // cost (ms) of one wave of n bootstraps on ONE GPU: 4-CTA cluster form up to `cl4` gates, 2-CTA cluster form up to `cl2`, else the
@@ -211,8 +209,8 @@ static FormCaps form_caps(const bfhe_circuit *c) {
   // device's cudaOccupancyMaxActiveClusters (which differs between GPUs of one box: 74 and 63 two-CTA clusters were both seen on
   // 148-SM B200s): 5/12 of the SMs for one gate on two SMs, 2/9 for one gate on four.  A wave that a particular GPU cannot keep
   // co-resident in the planned form simply runs in the next form there (launch_blind_rotate checks the real limit).
-  f.cl2 = cluster_forms_available(c->ctx) ? f.sms * 5 / 12 : 0;
-  f.cl4 = clx_form_available(c->ctx) ? f.sms * 2 / 9 : 0;
+  f.cl2 = has_form(c->ctx, Form::CL2) ? f.sms * 5 / 12 : 0;
+  f.cl4 = has_form(c->ctx, Form::CL4) ? f.sms * 2 / 9 : 0;
   return f;
 }
 static double plan_cost_ms(const bfhe_circuit *c, const FormCaps &f) {
@@ -591,57 +589,55 @@ static int probe_costs(bfhe_circuit *c) {
     const FormCaps f = form_caps(c);
     const size_t st = x->p.ct_stride, N = x->p.N;
     const int nmax = 4 * f.sms;
-    u32 *slab = nullptr, *ext = nullptr;
-    DevGate *dg = nullptr;
-    BFHE_CUDA(cudaMalloc(&slab, (size_t)(2 + nmax) * st * 4));
-    BFHE_CUDA(cudaMalloc(&ext, (size_t)nmax * (N + 4) * 4));
-    BFHE_CUDA(cudaMalloc(&dg, (size_t)nmax * sizeof(DevGate)));
+    DevBuf<u32> slab, ext;
+    DevBuf<DevGate> dg;
+    BFHE_CUDA(slab.alloc((size_t)(2 + nmax) * st));
+    BFHE_CUDA(ext.alloc((size_t)nmax * (N + 4)));
+    BFHE_CUDA(dg.alloc((size_t)nmax));
     std::vector<u32> rows(2 * st);
     u64 lcg = 0x9E3779B97F4A7C15ull; // any fixed non-trivial rows: the kernels' work does not depend on the values (zeros would let the
     for (auto &v : rows) { lcg = lcg * 6364136223846793005ull + 1442695040888963407ull; v = (u32)(lcg >> 40) % x->p.q; } // latency form skip steps)
     std::vector<DevGate> hg(nmax);
-    for (int i = 0; i < nmax; i++) hg[i] = DevGate{slab, slab + st, slab + (size_t)(2 + i) * st, BFHE_NAND, 0};
-    BFHE_CUDA(cudaMemcpy(slab, rows.data(), rows.size() * 4, cudaMemcpyHostToDevice));
-    BFHE_CUDA(cudaMemcpy(dg, hg.data(), hg.size() * sizeof(DevGate), cudaMemcpyHostToDevice));
-    cudaEvent_t e0, e1;
-    BFHE_CUDA(cudaEventCreate(&e0));
-    BFHE_CUDA(cudaEventCreate(&e1));
-    const int force[4] = {128, 32, 8, 4};
-    const int count[4] = {std::min(f.cl4, clx_fast_gates()), std::min(f.cl2, cl2_max_gates()), f.sms, 4 * f.sms};
-    const double dflt[4] = {FormCosts().cl4, FormCosts().cl2, FormCosts().lat, FormCosts().thr};
-    for (int k = 0; k < 4; k++) {
-      x->form_cost_ms[k] = dflt[k];
-      if (count[k] <= 0 || (k == 0 && !clx_form_available(x)) || (k == 1 && !cluster_forms_available(x))) continue;
+    for (int i = 0; i < nmax; i++) hg[i] = DevGate{slab.get(), slab.get() + st, slab.get() + (size_t)(2 + i) * st, BFHE_NAND, 0};
+    BFHE_CUDA(cudaMemcpy(slab.get(), rows.data(), rows.size() * 4, cudaMemcpyHostToDevice));
+    BFHE_CUDA(cudaMemcpy(dg.get(), hg.data(), hg.size() * sizeof(DevGate), cudaMemcpyHostToDevice));
+    DevEvent e0, e1;
+    BFHE_CUDA(e0.create());
+    BFHE_CUDA(e1.create());
+    struct Probe { Form form; int count; double WaveCosts::*ms; };
+    const Probe probes[] = {{Form::CL4, std::min(f.cl4, clx_fast_gates()), &WaveCosts::cl4}, {Form::CL2, std::min(f.cl2, cl2_max_gates()), &WaveCosts::cl2},
+                            {Form::LAT, f.sms, &WaveCosts::lat}, {Form::THR4, 4 * f.sms, &WaveCosts::thr}};
+    x->form_costs = WaveCosts(); // a form not measured keeps its default
+    for (const Probe &pr : probes) {
+      if (pr.count <= 0 || !has_form(x, pr.form)) continue;
       float best = 0;
       for (int rep = 0; rep < 3; rep++) { // first repetition warms the key into L2
-        BFHE_CUDA(cudaEventRecord(e0, x->stream));
-        int rc = launch_blind_rotate(x->P, x->p.method == BFHE_AP, dg, count[k], x->d_bk, x->d_twl, x->d_psiM, ext, nullptr, force[k], x->stream, nullptr, &x->v2);
+        BFHE_CUDA(cudaEventRecord(e0.e, x->stream));
+        int rc = launch_blind_rotate(x->P, x->p.method == BFHE_AP, dg.get(), pr.count, x->keys(), ext.get(), nullptr, pr.form, x->stream);
         if (rc) return cuda_fail((cudaError_t)rc, "probe: blind_rotate launch");
-        rc = launch_keyswitch(x->P, ext, dg, count[k], x->d_ksk, x->ksk_elem_bytes, x->stream);
+        rc = launch_keyswitch(x->P, ext.get(), dg.get(), pr.count, x->keys(), x->stream);
         if (rc) return cuda_fail((cudaError_t)rc, "probe: keyswitch launch");
-        BFHE_CUDA(cudaEventRecord(e1, x->stream));
-        BFHE_CUDA(cudaEventSynchronize(e1));
+        BFHE_CUDA(cudaEventRecord(e1.e, x->stream));
+        BFHE_CUDA(cudaEventSynchronize(e1.e));
         float ms = 0;
-        cudaEventElapsedTime(&ms, e0, e1);
+        cudaEventElapsedTime(&ms, e0.e, e1.e);
         if (rep == 1 || (rep == 2 && ms < best)) best = ms;
       }
-      x->form_cost_ms[k] = best;
+      x->form_costs.*pr.ms = best;
     }
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
-    cudaFree(slab); cudaFree(ext); cudaFree(dg);
     x->form_cost_measured = true;
   }
-  float v[4] = {(float)x->form_cost_ms[0], (float)x->form_cost_ms[1], (float)x->form_cost_ms[2], (float)x->form_cost_ms[3]};
+  const WaveCosts &m = x->form_costs;
+  float v[4] = {(float)m.cl4, (float)m.cl2, (float)m.lat, (float)m.thr};
   if (c->world > 1 && c->comm) { // every rank must plan with the same numbers: element-wise maximum over the ranks
-    float *d = nullptr;
-    BFHE_CUDA(cudaMalloc(&d, (size_t)c->world * 4 * sizeof(float)));
-    BFHE_CUDA(cudaMemcpyAsync(d + 4 * c->rank, v, sizeof v, cudaMemcpyHostToDevice, x->stream));
-    int nrc = g_nccl.AllGather(d + 4 * c->rank, d, 4, NCCL_FLOAT32, c->comm, x->stream);
-    if (nrc) { cudaFree(d); set_error("ncclAllGather (probe) failed"); return BFHE_ERR_NCCL; }
+    DevBuf<float> d;
+    BFHE_CUDA(d.alloc((size_t)c->world * 4));
+    BFHE_CUDA(cudaMemcpyAsync(d.get() + 4 * c->rank, v, sizeof v, cudaMemcpyHostToDevice, x->stream));
+    int nrc = g_nccl.AllGather(d.get() + 4 * c->rank, d.get(), 4, NCCL_FLOAT32, c->comm, x->stream);
+    if (nrc) { set_error("ncclAllGather (probe) failed"); return BFHE_ERR_NCCL; }
     std::vector<float> all((size_t)c->world * 4);
-    BFHE_CUDA(cudaMemcpyAsync(all.data(), d, all.size() * sizeof(float), cudaMemcpyDeviceToHost, x->stream));
+    BFHE_CUDA(cudaMemcpyAsync(all.data(), d.get(), all.size() * sizeof(float), cudaMemcpyDeviceToHost, x->stream));
     BFHE_CUDA(cudaStreamSynchronize(x->stream));
-    cudaFree(d);
     for (int r = 0; r < c->world; r++)
       for (int k = 0; k < 4; k++) v[k] = std::max(v[k], all[(size_t)r * 4 + k]);
   }
@@ -666,21 +662,23 @@ static int setup_peer_exchange(bfhe_circuit *c) {
   struct Rec { cudaIpcMemHandle_t slab, flags; uint32_t ok; uint32_t pad[3]; };
   static_assert(sizeof(Rec) % 16 == 0, "record size");
   Rec mine{};
-  BFHE_CUDA(cudaMalloc(&c->x_flags, 64 * sizeof(u32)));
+  BFHE_CUDA(c->x_buf.alloc(64));
+  c->x_flags = c->x_buf.get();
   c->x_counter = c->x_flags + 32; c->x_epoch = c->x_flags + 33; c->x_err = c->x_flags + 34;
   {
     std::vector<u32> init(64, 0);
     for (int r = 0; r < 32; r++) init[r] = c->x_per_epoch; // = value(epoch 0, end-of-Clock): the first Clock's opening wait passes
     BFHE_CUDA(cudaMemcpy(c->x_flags, init.data(), init.size() * sizeof(u32), cudaMemcpyHostToDevice));
   }
-  mine.ok = !(mode && std::strcmp(mode, "nccl") == 0) && cudaIpcGetMemHandle(&mine.slab, c->slab) == cudaSuccess &&
+  mine.ok = !(mode && std::strcmp(mode, "nccl") == 0) && cudaIpcGetMemHandle(&mine.slab, c->slab.get()) == cudaSuccess &&
             cudaIpcGetMemHandle(&mine.flags, c->x_flags) == cudaSuccess;
   cudaGetLastError();
-  Rec *d = nullptr;
-  BFHE_CUDA(cudaMalloc(&d, (size_t)W * sizeof(Rec)));
+  DevBuf<Rec> rec;
+  BFHE_CUDA(rec.alloc((size_t)W));
+  Rec *d = rec.get();
   BFHE_CUDA(cudaMemcpyAsync(d + c->rank, &mine, sizeof(Rec), cudaMemcpyHostToDevice, x->stream));
   int nrc = g_nccl.AllGather(d + c->rank, d, sizeof(Rec) / 4, NCCL_UINT32, c->comm, x->stream);
-  if (nrc) { cudaFree(d); set_error("ncclAllGather (IPC handles) failed"); return BFHE_ERR_NCCL; }
+  if (nrc) { set_error("ncclAllGather (IPC handles) failed"); return BFHE_ERR_NCCL; }
   std::vector<Rec> all(W);
   BFHE_CUDA(cudaMemcpyAsync(all.data(), d, (size_t)W * sizeof(Rec), cudaMemcpyDeviceToHost, x->stream));
   BFHE_CUDA(cudaStreamSynchronize(x->stream));
@@ -690,7 +688,7 @@ static int setup_peer_exchange(bfhe_circuit *c) {
   c->peer_slab_map.assign(W, nullptr); c->peer_flag_map.assign(W, nullptr);
   uint32_t opened = ok ? 1 : 0;
   for (int r = 0; r < W && opened; r++) {
-    if (r == c->rank) { slabs[r] = c->slab; flags[r] = c->x_flags; continue; }
+    if (r == c->rank) { slabs[r] = c->slab.get(); flags[r] = c->x_flags; continue; }
     if (cudaIpcOpenMemHandle(&c->peer_slab_map[r], all[r].slab, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess ||
         cudaIpcOpenMemHandle(&c->peer_flag_map[r], all[r].flags, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) { cudaGetLastError(); opened = 0; break; }
     slabs[r] = (u32 *)c->peer_slab_map[r]; flags[r] = (u32 *)c->peer_flag_map[r];
@@ -699,23 +697,20 @@ static int setup_peer_exchange(bfhe_circuit *c) {
   uint32_t *dflag = reinterpret_cast<uint32_t *>(d);
   BFHE_CUDA(cudaMemcpyAsync(dflag + c->rank, &opened, sizeof(uint32_t), cudaMemcpyHostToDevice, x->stream));
   nrc = g_nccl.AllGather(dflag + c->rank, dflag, 1, NCCL_UINT32, c->comm, x->stream);
-  if (nrc) { cudaFree(d); set_error("ncclAllGather (IPC status) failed"); return BFHE_ERR_NCCL; }
+  if (nrc) { set_error("ncclAllGather (IPC status) failed"); return BFHE_ERR_NCCL; }
   std::vector<uint32_t> st(W);
   BFHE_CUDA(cudaMemcpyAsync(st.data(), dflag, (size_t)W * sizeof(uint32_t), cudaMemcpyDeviceToHost, x->stream));
   BFHE_CUDA(cudaStreamSynchronize(x->stream));
-  cudaFree(d);
   for (int r = 0; r < W; r++) ok = ok && st[r];
   if (!ok) return BFHE_OK; // ncclAllGather path
-  BFHE_CUDA(cudaMalloc(&c->d_peer_slabs, (size_t)W * sizeof(u32 *)));
-  BFHE_CUDA(cudaMalloc(&c->d_peer_flags, (size_t)W * sizeof(u32 *)));
-  BFHE_CUDA(cudaMemcpy(c->d_peer_slabs, slabs.data(), (size_t)W * sizeof(u32 *), cudaMemcpyHostToDevice));
-  BFHE_CUDA(cudaMemcpy(c->d_peer_flags, flags.data(), (size_t)W * sizeof(u32 *), cudaMemcpyHostToDevice));
+  BFHE_CUDA(upload(c->d_peer_slabs, slabs));
+  BFHE_CUDA(upload(c->d_peer_flags, flags));
   c->peer_ok = true;
   return BFHE_OK;
 }
 static PeerX peer_x(const bfhe_circuit *c, uint32_t index) {
   PeerX px;
-  px.slabs = c->d_peer_slabs; px.local_base = c->slab; px.flags = c->d_peer_flags; px.counter = c->x_counter; px.epoch = c->x_epoch;
+  px.slabs = c->d_peer_slabs.get(); px.local_base = c->slab.get(); px.flags = c->d_peer_flags.get(); px.counter = c->x_counter; px.epoch = c->x_epoch;
   px.world = (u32)c->world; px.rank = (u32)c->rank; px.index = index; px.per_epoch = c->x_per_epoch;
   return px;
 }
@@ -738,15 +733,15 @@ static int upload_plan(bfhe_circuit *c) {
   }
   const size_t st = x->p.ct_stride;
   // one row past the plan holds the status word of a ciphertext SetInput, next to the fresh rows so that one broadcast carries both
-  BFHE_CUDA(cudaMalloc(&c->slab, (size_t)(c->total_rows + 1) * st * 4));
-  BFHE_CUDA(cudaMemset(c->slab, 0, (size_t)(c->total_rows + 1) * st * 4));
+  BFHE_CUDA(c->slab.alloc((size_t)(c->total_rows + 1) * st));
+  BFHE_CUDA(cudaMemset(c->slab.get(), 0, (size_t)(c->total_rows + 1) * st * 4));
   std::vector<DevGate> desc;
   std::vector<const u32 *> nin;
   std::vector<u32 *> nout;
   c->desc_off.clear(); c->my_count.clear(); c->not_off.clear();
   auto push_not = [&](const NotOp &o) { // the copy flag travels in the low bit of the (16-byte aligned) input pointer
-    nin.push_back(reinterpret_cast<const u32 *>(reinterpret_cast<uintptr_t>(c->slab + (size_t)o.in_row * st) | (o.copy ? 1u : 0u)));
-    nout.push_back(c->slab + (size_t)o.out_row * st);
+    nin.push_back(reinterpret_cast<const u32 *>(reinterpret_cast<uintptr_t>(c->slab.get() + (size_t)o.in_row * st) | (o.copy ? 1u : 0u)));
+    nout.push_back(c->slab.get() + (size_t)o.out_row * st);
   };
   uint32_t widest = std::max(1u, c->n_dff);
   for (uint32_t L = 0; L < c->levels.size(); L++) {
@@ -757,7 +752,7 @@ static int upload_plan(bfhe_circuit *c) {
     widest = std::max(widest, n);
     for (uint32_t i = b; i < b + n; i++) {
       const bfhe_gate &g = c->levels[L].gates[i];
-      desc.push_back(DevGate{c->slab + (size_t)g.in0 * st, c->slab + (size_t)g.in1 * st, c->slab + (size_t)g.out * st, g.op, 0});
+      desc.push_back(DevGate{c->slab.get() + (size_t)g.in0 * st, c->slab.get() + (size_t)g.in1 * st, c->slab.get() + (size_t)g.out * st, g.op, 0});
     }
     c->not_off.push_back(nin.size());
     for (const NotOp &o : c->levels[L].nots) push_not(o);
@@ -767,14 +762,10 @@ static int upload_plan(bfhe_circuit *c) {
   c->not_off.push_back(nin.size());
   for (uint32_t i = 0; i < c->n_dff; i++) push_not(c->dff_ops[c->n_dff + i]); // batch 2: state[i] = tmp[i]
   c->not_off.push_back(nin.size());
-  BFHE_CUDA(cudaMalloc(&c->d_desc, std::max<size_t>(desc.size(), 1) * sizeof(DevGate)));
-  BFHE_CUDA(cudaMemcpy(c->d_desc, desc.data(), desc.size() * sizeof(DevGate), cudaMemcpyHostToDevice));
-  BFHE_CUDA(cudaMalloc(&c->d_not_in, std::max<size_t>(nin.size(), 1) * sizeof(void *)));
-  BFHE_CUDA(cudaMalloc(&c->d_not_out, std::max<size_t>(nin.size(), 1) * sizeof(void *)));
-  BFHE_CUDA(cudaMemcpy(c->d_not_in, nin.data(), nin.size() * sizeof(void *), cudaMemcpyHostToDevice));
-  BFHE_CUDA(cudaMemcpy(c->d_not_out, nout.data(), nout.size() * sizeof(void *), cudaMemcpyHostToDevice));
-  c->ext_cap = widest;
-  BFHE_CUDA(cudaMalloc(&c->d_ext, (size_t)widest * (x->p.N + 4) * 4));
+  BFHE_CUDA(upload(c->d_desc, desc));
+  BFHE_CUDA(upload(c->d_not_in, nin));
+  BFHE_CUDA(upload(c->d_not_out, nout));
+  BFHE_CUDA(c->d_ext.alloc((size_t)widest * (x->p.N + 4)));
   rc = setup_peer_exchange(c);
   if (rc) return rc;
   c->dev_ready = true;
@@ -793,18 +784,18 @@ static int enqueue_levels(bfhe_circuit *c) {
     if (rc) return cuda_fail((cudaError_t)rc, "peer exchange launch");
   }
   if (c->n_dff) { // clocked circuits: the state rows take the values latched at the end of the previous clock (or the power-up values)
-    int rc = launch_eval_not(x->P, c->d_not_in + c->not_off[NLv + 1], c->d_not_out + c->not_off[NLv + 1], (int)c->n_dff, x->stream);
+    int rc = launch_eval_not(x->P, c->d_not_in.get() + c->not_off[NLv + 1], c->d_not_out.get() + c->not_off[NLv + 1], (int)c->n_dff, x->stream);
     if (rc) return cuda_fail((cudaError_t)rc, "DFF state launch");
   }
   for (uint32_t L = 0; L < c->levels.size(); L++) {
     const uint32_t n = c->my_count[L];
     if (n) {
-      int rc = launch_blind_rotate(x->P, x->p.method == BFHE_AP, c->d_desc + c->desc_off[L], (int)n, x->d_bk, x->d_twl, x->d_psiM,
-                                   c->d_ext, nullptr, x->force_g, x->stream, nullptr, &x->v2);
+      int rc = launch_blind_rotate(x->P, x->p.method == BFHE_AP, c->d_desc.get() + c->desc_off[L], (int)n, x->keys(), c->d_ext.get(), nullptr,
+                                   (Form)x->force_g, x->stream);
       if (rc) return cuda_fail((cudaError_t)rc, "blind_rotate launch");
       const bool xl = px_on && c->shard_index[L] >= 0;
       const PeerX px = xl ? peer_x(c, (uint32_t)c->shard_index[L]) : PeerX();
-      rc = launch_keyswitch(x->P, c->d_ext, c->d_desc + c->desc_off[L], (int)n, x->d_ksk, x->ksk_elem_bytes, x->stream, xl ? &px : nullptr);
+      rc = launch_keyswitch(x->P, c->d_ext.get(), c->d_desc.get() + c->desc_off[L], (int)n, x->keys(), x->stream, xl ? &px : nullptr);
       if (rc) return cuda_fail((cudaError_t)rc, "keyswitch launch");
     }
     if (px_on && c->shard_index[L] >= 0) { // outputs were stored into every slab by the key switch: wait for the peers' flags of this level
@@ -813,20 +804,20 @@ static int enqueue_levels(bfhe_circuit *c) {
       if (!rc) rc = launch_peer_wait(c->x_flags, c->x_epoch, (u32)c->world, (u32)c->rank, c->shard_index[L], c->x_per_epoch, c->x_err, x->stream);
       if (rc) return cuda_fail((cudaError_t)rc, "peer exchange launch");
     } else if (c->world > 1 && c->level_rpr[L] && c->levels[L].sharded) {
-      u32 *base = c->slab + (size_t)c->levels[L].first_row * st;
+      u32 *base = c->slab.get() + (size_t)c->levels[L].first_row * st;
       const size_t cnt = (size_t)c->level_rpr[L] * st;
       int nrc = g_nccl.AllGather(base + (size_t)c->rank * cnt, base, cnt, NCCL_UINT32, c->comm, x->stream);
       if (nrc) { set_error(std::string("ncclAllGather: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(nrc) : "?")); return BFHE_ERR_NCCL; }
     }
     const size_t nn = c->not_off[L + 1] - c->not_off[L];
     if (nn) {
-      int rc = launch_eval_not(x->P, c->d_not_in + c->not_off[L], c->d_not_out + c->not_off[L], (int)nn, x->stream);
+      int rc = launch_eval_not(x->P, c->d_not_in.get() + c->not_off[L], c->d_not_out.get() + c->not_off[L], (int)nn, x->stream);
       if (rc) return cuda_fail((cudaError_t)rc, "eval_not launch");
     }
   }
   if (c->n_dff) { // latch: scratch[i] = D_i (the state rows keep this clock's Q until the next clock starts, so outputs and verify
                   // mode read consistent values, and a D that is another flip-flop's Q sees the old state)
-    int rc = launch_eval_not(x->P, c->d_not_in + c->not_off[NLv], c->d_not_out + c->not_off[NLv], (int)c->n_dff, x->stream);
+    int rc = launch_eval_not(x->P, c->d_not_in.get() + c->not_off[NLv], c->d_not_out.get() + c->not_off[NLv], (int)c->n_dff, x->stream);
     if (rc) return cuda_fail((cudaError_t)rc, "DFF latch launch");
   }
   if (px_on) { // end-of-Clock signal: this rank no longer reads its slab, the peers may start storing the next Clock's rows
@@ -1179,22 +1170,22 @@ static int commit_input(bfhe_circuit *c, bool init_state, size_t bcast_words, bo
   bfhe_ctx *x = c->ctx;
   const size_t st = x->p.ct_stride;
   if (bcast_words) {
-    u32 *fresh = c->slab + (size_t)c->fresh_base * st;
+    u32 *fresh = c->slab.get() + (size_t)c->fresh_base * st;
     int nrc = g_nccl.Broadcast(fresh, fresh, bcast_words, NCCL_UINT32, 0, c->comm, x->stream);
     if (nrc) { set_error(ct ? "ncclBroadcast of the input ciphertexts failed" : "ncclBroadcast of the fresh input encryptions failed"); return BFHE_ERR_NCCL; }
   }
   if (init_state) {
     std::vector<DevGate> init(c->n_dff);
     for (uint32_t i = 0; i < c->n_dff; i++) {
-      const u32 *src = c->slab + (size_t)(c->dff_fresh_base + i) * st;
-      init[i] = DevGate{src, src, c->slab + (size_t)(c->dff_tmp_base + i) * st, BFHE_BOOTSTRAP, 0}; // latched; the clock moves it into the state row
+      const u32 *src = c->slab.get() + (size_t)(c->dff_fresh_base + i) * st;
+      init[i] = DevGate{src, src, c->slab.get() + (size_t)(c->dff_tmp_base + i) * st, BFHE_BOOTSTRAP, 0}; // latched; the clock moves it into the state row
     }
     int rc = run_gate_list(x, init.data(), init.size(), nullptr);
     if (rc) return rc;
     c->state_init_pending = false;
   }
   u32 bad_row = INGEST_OK;
-  if (ct) BFHE_CUDA(cudaMemcpyAsync(&bad_row, c->slab + (size_t)c->total_rows * st, sizeof bad_row, cudaMemcpyDeviceToHost, x->stream));
+  if (ct) BFHE_CUDA(cudaMemcpyAsync(&bad_row, c->slab.get() + (size_t)c->total_rows * st, sizeof bad_row, cudaMemcpyDeviceToHost, x->stream));
   BFHE_CUDA(cudaStreamSynchronize(x->stream));
   if (bad_row != INGEST_OK && bad_row >= INGEST_REJECTED) {
     set_error(reject_msg.empty() ? "SetInput: rank 0 rejected its compact input blob" : reject_msg);
@@ -1246,7 +1237,7 @@ extern "C" int bfhe_circuit_set_input(bfhe_circuit *c, const uint8_t *bits, size
       }
     }
     // fresh_base .. fresh_base + n_in and dff_fresh_base .. are adjacent rows (build_plan_cap)
-    BFHE_CUDA(cudaMemcpyAsync(c->slab + (size_t)c->fresh_base * st, fresh.data(), fresh.size() * 4, cudaMemcpyHostToDevice, x->stream));
+    BFHE_CUDA(cudaMemcpyAsync(c->slab.get() + (size_t)c->fresh_base * st, fresh.data(), fresh.size() * 4, cudaMemcpyHostToDevice, x->stream));
     return commit_input(c, init_state, c->world > 1 && seed == 0 ? fresh.size() : 0, false);
   }
   c->has_input = true;
@@ -1299,7 +1290,7 @@ static int set_input_ciphertexts(bfhe_circuit *c, size_t nbits, const uint32_t *
   if (source) {
     if (!reject && !blob && on_device && nbits)
       if (int rc = check_device_buffer(x, cts, "SetInput: the ciphertext buffer")) return rc;
-    u32 *fresh = c->slab + (size_t)c->fresh_base * st, *status = c->slab + (size_t)c->total_rows * st;
+    u32 *fresh = c->slab.get() + (size_t)c->fresh_base * st, *status = c->slab.get() + (size_t)c->total_rows * st;
     if (reject) {
       status_word = INGEST_REJECTED | (u32)-reject;
     } else if (blob) {
@@ -1315,7 +1306,7 @@ static int set_input_ciphertexts(bfhe_circuit *c, size_t nbits, const uint32_t *
     if (reject || blob) BFHE_CUDA(cudaMemcpyAsync(status, &status_word, sizeof status_word, cudaMemcpyHostToDevice, x->stream));
     // no secret key, no Encrypt(0): flip-flops power up from the trivial encryption of 0.  The rows may still hold a bit-path
     // SetInput's Encrypt(0).
-    if (init_state) BFHE_CUDA(cudaMemsetAsync(c->slab + (size_t)c->dff_fresh_base * st, 0, (size_t)c->n_dff * st * 4, x->stream));
+    if (init_state) BFHE_CUDA(cudaMemsetAsync(c->slab.get() + (size_t)c->dff_fresh_base * st, 0, (size_t)c->n_dff * st * 4, x->stream));
   }
   // sharded: the input rows, the flip-flops' fresh rows and the status word are adjacent (build_plan_cap, upload_plan)
   const size_t bcast = c->world > 1 ? ((size_t)c->n_in + c->n_dff) * st + 1 : 0;
@@ -1347,7 +1338,7 @@ static int clock_run(bfhe_circuit *c, uint8_t *out_bits, size_t cap, uint8_t *pl
   if (!c->has_input) { set_error("Clock before SetInput (or after a change of flags / schedule / sharding: call SetInput again)"); return BFHE_ERR_STATE; }
   // a combinational circuit is done after one clock (src/circuit.cpp:538-541); one with flip-flops is clocked again and again
   if (c->done && c->n_dff == 0) { set_error("done ckt clocked! should reset"); return BFHE_ERR_STATE; }
-  if (c->encrypted && (!c->dev_ready || !c->slab)) { set_error("Clock: encrypted mode was switched on after SetInput; call SetInput again"); return BFHE_ERR_STATE; }
+  if (c->encrypted && (!c->dev_ready || !c->slab.get())) { set_error("Clock: encrypted mode was switched on after SetInput; call SetInput again"); return BFHE_ERR_STATE; }
   if (c->encrypted && c->world > 1 && !c->comm) { set_error("Clock: sharded evaluation without an NCCL communicator"); return BFHE_ERR_STATE; }
   if (c->verify != c->planned_verify) { set_error("Clock: verify mode changed after SetInput; call SetInput again"); return BFHE_ERR_STATE; }
   if (c->plaintext && c->ct_input) { set_error("Clock: plaintext mode needs input bits; the input was set as ciphertexts"); return BFHE_ERR_STATE; }
@@ -1375,13 +1366,13 @@ static int clock_run(bfhe_circuit *c, uint8_t *out_bits, size_t cap, uint8_t *pl
         return BFHE_ERR_ARG;
       }
     }
-    cudaEvent_t e0, e1;
-    BFHE_CUDA(cudaEventCreate(&e0));
-    BFHE_CUDA(cudaEventCreate(&e1));
+    DevEvent e0, e1;
+    BFHE_CUDA(e0.create());
+    BFHE_CUDA(e1.create());
     int rc = BFHE_OK;
     if (c->use_graph && !c->graph) { // one CUDA graph per circuit, sharded or not (NCCL collectives are capturable)
       if (c->world > 1 && !c->peer_ok) { // NCCL's lazy set-up (channels, buffers) must happen outside the capture: one eager exchange first
-        int nrc = g_nccl.AllGather(c->slab + (size_t)c->rank * st, c->slab, st, NCCL_UINT32, c->comm, x->stream);
+        int nrc = g_nccl.AllGather(c->slab.get() + (size_t)c->rank * st, c->slab.get(), st, NCCL_UINT32, c->comm, x->stream);
         if (nrc) { set_error("ncclAllGather warm-up failed"); return BFHE_ERR_NCCL; }
         BFHE_CUDA(cudaStreamSynchronize(x->stream));
         // rows 0 .. world-1 (level-0 outputs) were overwritten with copies of themselves per rank: level 0 rewrites them
@@ -1396,19 +1387,17 @@ static int clock_run(bfhe_circuit *c, uint8_t *out_bits, size_t cap, uint8_t *pl
       cudaGraphDestroy(g);
       if (ce != cudaSuccess) return cuda_fail(ce, "cudaGraphInstantiate");
     }
-    BFHE_CUDA(cudaEventRecord(e0, x->stream));
+    BFHE_CUDA(cudaEventRecord(e0.e, x->stream));
     if (c->use_graph) {
       BFHE_CUDA(cudaGraphLaunch(c->graph, x->stream));
     } else {
       rc = enqueue_levels(c);
       if (rc) return rc;
     }
-    BFHE_CUDA(cudaEventRecord(e1, x->stream));
-    BFHE_CUDA(cudaEventSynchronize(e1));
+    BFHE_CUDA(cudaEventRecord(e1.e, x->stream));
+    BFHE_CUDA(cudaEventSynchronize(e1.e));
     float ms = 0;
-    cudaEventElapsedTime(&ms, e0, e1);
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
+    cudaEventElapsedTime(&ms, e0.e, e1.e);
     c->device_ms += ms;
     if (c->world > 1 && c->peer_ok) { // a wait for a peer's flag timed out (the kernels do not hang: they record which peer and go on)
       u32 xe = 0;
@@ -1418,15 +1407,15 @@ static int clock_run(bfhe_circuit *c, uint8_t *out_bits, size_t cap, uint8_t *pl
     if (out_cts) { // outputs stay encrypted: one launch copies every output row, through EvalNOT where the output reads its row negated
       u32 *dst = out_cts;
       if (!on_device) {
-        if (!c->d_egress) BFHE_CUDA(cudaMalloc(&c->d_egress, std::max<size_t>(nout, 1) * st * 4));
-        dst = c->d_egress;
+        BFHE_CUDA(c->d_egress.reserve(std::max<size_t>(nout, 1) * st, x->stream));
+        dst = c->d_egress.get();
       }
       BFHE_CUDA(cudaMemsetAsync(dst, 0, (size_t)nout * st * 4, x->stream)); // the kernel writes the ct_words, not the padding
       std::vector<const u32 *> in(nout);
       std::vector<u32 *> out(nout);
       for (uint32_t b = 0; b < nout; b++) {
         const uint32_t w = c->out_wire[b];
-        in[b] = reinterpret_cast<const u32 *>(reinterpret_cast<uintptr_t>(c->slab + (size_t)c->wire_row[w] * st) | (c->wire_neg[w] ? 0u : 1u));
+        in[b] = reinterpret_cast<const u32 *>(reinterpret_cast<uintptr_t>(c->slab.get() + (size_t)c->wire_row[w] * st) | (c->wire_neg[w] ? 0u : 1u));
         out[b] = dst + (size_t)b * st;
       }
       rc = not_ptr_batch(x, in, out);
@@ -1435,7 +1424,7 @@ static int clock_run(bfhe_circuit *c, uint8_t *out_bits, size_t cap, uint8_t *pl
       BFHE_CUDA(cudaStreamSynchronize(x->stream));
     } else if (c->verify) { // OUTPUT gates: decrypt on the host (src/circuit.cpp:796-801)
       std::vector<u32> rows((size_t)c->total_rows * st);
-      BFHE_CUDA(cudaMemcpy(rows.data(), c->slab, rows.size() * 4, cudaMemcpyDeviceToHost));
+      BFHE_CUDA(cudaMemcpy(rows.data(), c->slab.get(), rows.size() * 4, cudaMemcpyDeviceToHost));
       std::vector<uint8_t> dec(c->total_rows);
       rc = bfhe_decrypt(x, rows.data(), c->total_rows, dec.data());
       if (rc) return rc;
@@ -1451,7 +1440,7 @@ static int clock_run(bfhe_circuit *c, uint8_t *out_bits, size_t cap, uint8_t *pl
     } else {
       std::vector<u32> orow((size_t)nout * st);
       for (uint32_t b = 0; b < nout; b++)
-        BFHE_CUDA(cudaMemcpyAsync(orow.data() + (size_t)b * st, c->slab + (size_t)c->wire_row[c->out_wire[b]] * st, st * 4,
+        BFHE_CUDA(cudaMemcpyAsync(orow.data() + (size_t)b * st, c->slab.get() + (size_t)c->wire_row[c->out_wire[b]] * st, st * 4,
                                   cudaMemcpyDeviceToHost, x->stream));
       BFHE_CUDA(cudaStreamSynchronize(x->stream));
       std::vector<uint8_t> dec(nout);
@@ -1491,6 +1480,6 @@ extern "C" int bfhe_circuit_download_slab(bfhe_circuit *c, uint32_t *host, size_
   if (!c || !c->dev_ready) return BFHE_ERR_STATE;
   if (rows_cap < c->total_rows) return BFHE_ERR_ARG;
   BFHE_CUDA(cudaSetDevice(c->ctx->device));
-  BFHE_CUDA(cudaMemcpy(host, c->slab, (size_t)c->total_rows * c->ctx->p.ct_stride * 4, cudaMemcpyDeviceToHost));
+  BFHE_CUDA(cudaMemcpy(host, c->slab.get(), (size_t)c->total_rows * c->ctx->p.ct_stride * 4, cudaMemcpyDeviceToHost));
   return BFHE_OK;
 }
